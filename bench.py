@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- post-head path throughput (Detect decode + per-task NMS) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic raw head tensors: BASELINE.json config 3 (3 task heads
 20/19/12 classes, 640x640 -> 8400 anchors, B=64 images per GPU, fp16, val settings conf 0.001 / iou 0.6 / multi_label /
@@ -14,6 +14,10 @@ entry and the decode launch carries the programmatic-serialization attribute); a
 steps are exactly K decode launches + K NMS launches.  32 of the K steps (16 when K < 128) are "instrumented" replays of the
 same two kernels in serial order with timing events recorded by the graph itself around each kernel: that is where
 `roofline` (the decode kernel alone on the GPU) comes from; they cost ~13 us more than an overlapped step each.
+
+`--dump-outputs DIR` writes what the last timed step delivered (rank 0) as DIR/detections.npy (float32 [tasks, images,
+max_det, 6], rows past each count zeroed) and DIR/counts.npy (float32 [tasks, images]); the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 
 Prints ONE JSON line (rank 0).  `value` = device-resident throughput; `e2e` = the host-buffer public API (pinned H2D
 of the raw heads + D2H of the detections inside the timed region); `roofline` = decode kernel vs the measured HBM peak;
@@ -35,6 +39,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from untouched (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -425,6 +430,19 @@ def head_tail_line(dev, reps=10):
             "roofline": {"bound": "hbm", "achieved": gbps, "peak": peak, "unit": "GB/s", "frac": gbps / peak, "peak_source": peak_src}}
 
 
+def dump_outputs(out_dir, result):
+    """``result`` = (dets [T, B, max_det, 6] float32, counts [T, B] int32) as a caller of the pipeline receives them.
+    Rows past each count are padding the kernel leaves unwritten, so they are zeroed to make two runs comparable."""
+    import numpy as np
+
+    dets, counts = (x.cpu() for x in result)
+    dets = dets.clone()
+    dets[torch.arange(dets.shape[2]).view(1, 1, -1) >= counts.unsqueeze(-1)] = 0.0
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "detections.npy"), dets.numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "counts.npy"), counts.numpy().astype(np.float32))
+
+
 # ------------------------------------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
@@ -435,7 +453,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the surface / eager-reference / planted / serial / config-5 lines")
     ap.add_argument("--serial", action="store_true", help="decode -> NMS of the same batch back to back (no overlap) in the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the detections and counts of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -544,6 +565,11 @@ def main():
         t_end.record()
         barrier()
     elapsed_ms = t_start.elapsed_time(t_end)
+    if args.dump_outputs and rank == 0:  # the last batch sits in outs slot (steps - 1) & 1, as in the check above
+        # barrier() above ended in torch.cuda.synchronize(), which waits for every stream of the device, so the
+        # pipeline's last NMS (and, N > 1, the delivery's collect) has finished writing this slot
+        last = (steps - 1) & 1
+        dump_outputs(args.dump_outputs, delivery.result(last) if delivery is not None else pipe.outs[last])
     samples = [pipe.timed_ms(i) for i in range(len(timed_at))]
     nms_ms, dec_ms = [s[0] for s in samples], [s[1] for s in samples]
     per_rank = None

@@ -5,6 +5,7 @@
 # Translation units compile in parallel (make -j); objects are cached per flag set under csrc/build/.
 set -e
 HERE=$(cd "$(dirname "$0")" && pwd)
+command -v nvcc >/dev/null 2>&1 || PATH="${CUDA_HOME:-/usr/local/cuda}/bin:$PATH"
 OUT="${CERB_OUT:-$HERE/../libcerb_post.so}"
 EXTRA="$*"
 TAG=default

@@ -3,21 +3,62 @@ oracle/gen_golden.py produced by executing the unmodified reference."""
 import numpy as np
 import pytest
 import torch
+import torch.nn.functional as F
 
 from conftest import golden_manifest, golden_names, load_golden, split_rows
 from cerberusdet_b200.synth import STRIDES
 from oracle import ref_port as rp
 
 
+ROUNDINGS = 4
+
+
+def assert_matches_golden(got, want, terms, sum_dtype=None):
+    """``got`` equals the golden ``want`` bit for bit, or every element lies within ROUNDINGS roundings of its own value
+    in the output dtype plus ROUNDINGS roundings in ``sum_dtype`` (default: the output dtype) of ``terms``, the magnitude
+    of what that element is summed from.  CPU convolution, matrix-product and reduction kernels (ATen, MKL, oneDNN)
+    choose their summation order by instruction set, CPU vendor and thread count, so on a host other than the one that
+    produced the vectors the last bits may differ; the bound is per element, so an error of the port itself (a shifted
+    box, a changed logit, a missing bias) does not fit in it (test_golden_bounds_reject_port_errors)."""
+    got = got.detach()
+    assert got.dtype == want.dtype and got.shape == want.shape
+    if torch.equal(got, want):
+        return
+    eps, sum_eps = torch.finfo(want.dtype).eps, torch.finfo(sum_dtype or want.dtype).eps
+    bound = ROUNDINGS * (eps * want.double().abs() + sum_eps * terms.double())
+    bad = (got.double() - want.double()).abs() > bound
+    assert not bad.any(), (f"{int(bad.sum())} of {bad.numel()} elements differ by more than {ROUNDINGS} roundings of their "
+                           f"value and terms, the first at {tuple(bad.nonzero()[0].tolist())}")
+
+
+def decode_terms(y):
+    """Per-element magnitude of the terms of a decoded ``y [B, 4+nc, A]``: the corners (c -+ size/2) that centre and size
+    are computed from, |c| + |size|/2, and the sigmoid scores themselves."""
+    y = y.double().abs()
+    t = y.clone()
+    t[:, 0] = t[:, 2] = y[:, 0] + y[:, 2] / 2
+    t[:, 1] = t[:, 3] = y[:, 1] + y[:, 3] / 2
+    return t
+
+
+def head_tail_case(g):
+    """The inputs of the two convolutions of every level, and per level the magnitude of the terms of each raw output:
+    the same convolutions on absolute values.  (CPU convolutions of half tensors sum in float32.)"""
+    t = lambda k: torch.from_numpy(g[k])  # noqa: E731
+    args = [[t(f"{k}{i}") for i in range(3)] for k in ("box_feat", "cls_feat", "box_w", "box_b", "cls_w", "cls_b")]
+    a = lambda x: x.double().abs()  # noqa: E731
+    terms = [torch.cat((F.conv2d(a(bf), a(bw), a(bb)), F.conv2d(a(cf), a(cw), a(cb))), 1) for bf, cf, bw, bb, cw, cb in zip(*args)]
+    return args, terms
+
+
 @pytest.mark.parametrize("name", golden_names("decode"))
-def test_decode_port_bit_exact(name):
+def test_decode_port_matches_golden(name):
     g = load_golden(name)
     nc = golden_manifest()[name]["nc"]
     levels = [torch.from_numpy(g[f"level{i}"]) for i in range(3)]
     y = rp.decode_port(levels, nc, STRIDES)
-    ref = torch.from_numpy(g["y"])
-    assert y.dtype == ref.dtype and y.shape == ref.shape
-    assert torch.equal(y, ref)  # same ATen kernels -> bit exact on CPU
+    want = torch.from_numpy(g["y"])
+    assert_matches_golden(y, want, decode_terms(want))
 
 
 @pytest.mark.parametrize("greedy", ["torchvision", "c"])
@@ -77,9 +118,9 @@ def test_real_model_config1_vectors(name):
     g = load_golden(name)
     meta = golden_manifest()[name]
     levels = [torch.from_numpy(g[f"level{i}"]) for i in range(3)]
-    y = rp.decode_port(levels, meta["nc"], STRIDES)
-    assert torch.equal(y, torch.from_numpy(g["y"]))
-    for greedy in ("torchvision", "c"):
+    y = torch.from_numpy(g["y"])
+    assert_matches_golden(rp.decode_port(levels, meta["nc"], STRIDES), y, decode_terms(y))
+    for greedy in ("torchvision", "c"):  # selection on the reference's own decoded tensor: bit for bit
         got = rp.nms_port(y, greedy=greedy, **meta["kwargs"])
         want = split_rows(g["rows"], g["counts"])
         assert len(got) == 1 and torch.equal(got[0], want[0])
@@ -87,35 +128,41 @@ def test_real_model_config1_vectors(name):
 
 # ------------------------------------------------------------------ training-time sibling decode (SURVEY 8f-4)
 @pytest.mark.parametrize("name", golden_names("train_bbox"))
-def test_bbox_decode_port_bit_exact(name):
+def test_bbox_decode_port_matches_golden(name):
     """The oracle restatement of Loss.bbox_decode (utils/loss.py:126-131) against vectors the unmodified reference
-    produced (oracle/gen_golden_train.py): forward and the autograd gradient, bit for bit (same ATen kernels)."""
+    produced (oracle/gen_golden_train.py): forward and the autograd gradient (assert_matches_golden)."""
     from oracle import ref_port as rp
 
     g = load_golden(name)
     pred = torch.from_numpy(g["pred"]).requires_grad_(True)
-    out = rp.bbox_decode_port(torch.from_numpy(g["anchor_points"]), pred)
-    assert torch.equal(out.detach(), torch.from_numpy(g["out"]))
-    (grad_in,) = torch.autograd.grad(out, pred, torch.from_numpy(g["grad_out"]))
-    assert torch.equal(grad_in, torch.from_numpy(g["grad_in"]))
+    anchors = torch.from_numpy(g["anchor_points"])
+    out = rp.bbox_decode_port(anchors, pred)
+    want, grad_out = torch.from_numpy(g["out"]), torch.from_numpy(g["grad_out"])
+    corner_anchor = anchors.double().repeat(1, 2)  # (x, y, x, y) of every anchor
+    assert_matches_golden(out, want, corner_anchor.abs() + (want.double() - corner_anchor).abs())  # anchor -+ distance
+    (grad_in,) = torch.autograd.grad(out, pred, grad_out)
+    # d/dlogit_j of sum_k p_k k: p_j (j - E) per side, E <= REG_MAX - 1
+    assert_matches_golden(grad_in, torch.from_numpy(g["grad_in"]), (rp.REG_MAX - 1) * grad_out.abs().repeat_interleave(rp.REG_MAX, -1))
 
 
 # ------------------------------------------------------------------ head tail (SURVEY 8f-3): the checker, ahead of the kernel
 @pytest.mark.parametrize("name", golden_names("headtail"))
-def test_head_tail_port_bit_exact(name):
+def test_head_tail_port_matches_golden(name):
     """Last 1x1 convs of both towers + concat + decode, restated in the oracle, against what the unmodified reference
     Detect module (real conv towers, eval mode) returned for the captured inputs of those convs
     (oracle/gen_golden_headtail.py)."""
     from oracle import ref_port as rp
 
     g = load_golden(name)
-    t = lambda k: torch.from_numpy(g[k])  # noqa: E731
-    y, raw = rp.head_tail_port([t(f"box_feat{i}") for i in range(3)], [t(f"cls_feat{i}") for i in range(3)],
-                               [t(f"box_w{i}") for i in range(3)], [t(f"box_b{i}") for i in range(3)],
-                               [t(f"cls_w{i}") for i in range(3)], [t(f"cls_b{i}") for i in range(3)], (8.0, 16.0, 32.0))
+    args, terms = head_tail_case(g)
+    y, raw = rp.head_tail_port(*args, (8.0, 16.0, 32.0))
+    golden_raw = [torch.from_numpy(g[f"raw{i}"]) for i in range(3)]
     for i in range(3):
-        assert torch.equal(raw[i], t(f"raw{i}")), f"raw level {i}"
-    assert torch.equal(y, t("y"))
+        assert_matches_golden(raw[i], golden_raw[i], terms[i], torch.float32)
+    if not all(torch.equal(a, b) for a, b in zip(raw, golden_raw)):  # the DFL softmax amplifies a rounding of the raw
+        y = rp.decode_port(golden_raw, int(args[4][0].shape[0]), (8.0, 16.0, 32.0))  # levels: decode the reference's own
+    want = torch.from_numpy(g["y"])
+    assert_matches_golden(y, want, decode_terms(want))
 
 
 def _tal_case_of(name):
@@ -127,15 +174,43 @@ def _tal_case_of(name):
 
 
 @pytest.mark.parametrize("name", golden_names("tal"))
-def test_tal_assign_port_bit_exact(name):
+def test_tal_assign_port_matches_golden(name):
     """oracle/ref_port.tal_assign_port against what the unmodified TaskAlignedAssigner.forward returned on the same seeded
-    inputs (oracle/gen_golden_tal.py): all five tensors, bit for bit."""
+    inputs (oracle/gen_golden_tal.py): all five tensors, bit for bit except the normalised scores (assert_matches_golden:
+    products and quotients of overlaps, each score is its own scale)."""
     g = load_golden(name)
     c, meta = _tal_case_of(name)
     labels, bboxes, scores, fg, gidx, ambiguous = rp.tal_assign_port(**c, num_classes=meta["nc"])
     assert torch.equal(labels, torch.from_numpy(g["target_labels"]))
     assert torch.equal(bboxes, torch.from_numpy(g["target_bboxes"]))
-    assert torch.equal(scores, torch.from_numpy(g["target_scores"]))
+    want = torch.from_numpy(g["target_scores"])
+    assert_matches_golden(scores, want, want.abs())
     assert torch.equal(fg, torch.from_numpy(g["fg_mask"]))
     assert torch.equal(gidx, torch.from_numpy(g["target_gt_idx"]))
     assert fg.any() and (fg.sum(1) > 0).all()
+
+
+def test_golden_bounds_reject_port_errors():
+    """The per-element bounds of assert_matches_golden do not admit small errors of a port: classes off by one, score
+    logits +0.05, centres +4 px on the stride-8 level, sizes +1 px, a missing class-convolution bias."""
+    for name in golden_names("decode") + golden_names("model"):
+        want = torch.from_numpy(load_golden(name)["y"])
+        a0 = (int(golden_manifest()[name]["imgsz"][0]) // 8) * (int(golden_manifest()[name]["imgsz"][1]) // 8)
+        rolled = torch.cat((want[:, :4], want[:, 4:].roll(1, 1)), 1)
+        wrong = [] if torch.equal(rolled, want) else [rolled]  # (nc = 1, or every class scored alike as in model_cfg1)
+        logit = torch.cat((want[:, :4], torch.sigmoid(torch.logit(want[:, 4:].double()) + 0.05).to(want.dtype)), 1)
+        centre, size = want.clone(), want.clone()
+        centre[:, 0, :a0] += 4
+        size[:, 2:4] += 1
+        for got in wrong + [logit, centre, size]:
+            with pytest.raises(AssertionError):
+                assert_matches_golden(got, want, decode_terms(want))
+    for name in golden_names("headtail"):
+        g = load_golden(name)
+        args, terms = head_tail_case(g)
+        for i in range(3):
+            raw = torch.from_numpy(g[f"raw{i}"])
+            no_bias = raw.clone()
+            no_bias[:, 64:] -= args[5][i].view(1, -1, 1, 1)
+            with pytest.raises(AssertionError):
+                assert_matches_golden(no_bias, raw, terms[i], torch.float32)
