@@ -36,6 +36,9 @@ EXPORTS = (
     "cerb_bbox_decode_bwd",
     "cerb_tal_workspace_bytes",
     "cerb_tal_assign",
+    "cerb_bbox_loss_workspace_bytes",
+    "cerb_bbox_loss_fwd",
+    "cerb_bbox_loss_bwd",
     "cerb_debug_set",
     "cerb_debug_reset",
     "cerb_debug_set_chunking",
@@ -119,6 +122,13 @@ def load() -> ctypes.CDLL:
         lib.cerb_tal_workspace_bytes.argtypes = [i, i, i, i]
         lib.cerb_tal_assign.restype = i
         lib.cerb_tal_assign.argtypes = [vp] * 6 + [i] * 5 + [d, d, d, i] + [vp] * 6 + [sz, vp]
+    if hasattr(lib, "cerb_bbox_loss_fwd") or "CERB_LIB" not in os.environ:
+        lib.cerb_bbox_loss_workspace_bytes.restype = sz
+        lib.cerb_bbox_loss_workspace_bytes.argtypes = [i, i]
+        lib.cerb_bbox_loss_fwd.restype = i
+        lib.cerb_bbox_loss_fwd.argtypes = [vp] * 7 + [d] + [i] * 5 + [vp] * 4 + [sz, vp]
+        lib.cerb_bbox_loss_bwd.restype = i
+        lib.cerb_bbox_loss_bwd.argtypes = [vp] * 7 + [d] + [i] * 5 + [vp] * 5
     if hasattr(lib, "cerb_debug_set") or "CERB_LIB" not in os.environ:  # (tools/ A/B runs may load an older build)
         lib.cerb_debug_set.restype = i
         lib.cerb_debug_set.argtypes = [ctypes.c_char_p, i]

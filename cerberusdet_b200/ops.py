@@ -736,3 +736,100 @@ def tal_assign(pd_scores: torch.Tensor, pd_bboxes: torch.Tensor, anc_points: tor
     for t in (sc, pb, an, gl, gb, mg, ws):
         t.record_stream(torch.cuda.current_stream(dev))
     return labels, bboxes, scores, fg, gidx
+
+
+# ----------------------------------------------------------------------------- box-regression loss term (SURVEY 8f-4)
+def _dense32(x: torch.Tensor) -> torch.Tensor:
+    """Contiguous and 32-byte aligned (the 256-bit row accesses of the training kernels)."""
+    x = x.contiguous()
+    return x if x.data_ptr() % 32 == 0 else x.clone(memory_format=torch.contiguous_format)
+
+
+class _BboxLoss(torch.autograd.Function):
+    """``BboxLoss.forward`` (reference utils/loss.py:12-44) as one CUDA kernel per direction; differentiable in
+    ``pred_dist`` and ``pred_bboxes``."""
+
+    @staticmethod
+    def forward(ctx, pred_dist, pred_bboxes, anchor_points, target_bboxes, target_scores, target_scores_sum, fg_mask, per_anchor):
+        lib = _lib.load()
+        _require_cuda(pred_dist, "pred_dist")
+        dev = pred_dist.device
+        if pred_dist.dim() != 3 or pred_dist.shape[2] != 64:
+            raise ValueError(f"pred_dist must be [B, A, 64] (16 bins per side), got {tuple(pred_dist.shape)}")
+        B, A, _ = (int(v) for v in pred_dist.shape)
+        C = int(target_scores.shape[-1]) if target_scores.dim() == 3 else -1
+        for name, t, shape in (("pred_bboxes", pred_bboxes, (B, A, 4)), ("anchor_points", anchor_points, (A, 2)),
+                               ("target_bboxes", target_bboxes, (B, A, 4)), ("target_scores", target_scores, (B, A, C)),
+                               ("fg_mask", fg_mask, (B, A))):
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{name} must be {list(shape)}, got {tuple(t.shape)}")
+            if t.device != dev:
+                raise TypeError(f"{name} must be on {dev}, got {t.device}")
+        code = _dtype_code(pred_dist)
+        if pred_bboxes.dtype != pred_dist.dtype or anchor_points.dtype != pred_dist.dtype:
+            raise TypeError("pred_dist, pred_bboxes and anchor_points must share one dtype")
+        if target_bboxes.dtype != torch.float32 or target_scores.dtype != torch.float32 or fg_mask.dtype != torch.bool:
+            raise TypeError("target_bboxes and target_scores must be float32 and fg_mask bool")
+        tss_dev, tss_host = None, 1.0
+        if torch.is_tensor(target_scores_sum):
+            if target_scores_sum.numel() != 1:
+                raise ValueError("target_scores_sum must hold one value")
+            if target_scores_sum.is_cuda:
+                if target_scores_sum.device != dev:
+                    raise TypeError(f"target_scores_sum must be on {dev}, got {target_scores_sum.device}")
+                tss_dev = target_scores_sum.detach().reshape(()).float()
+            else:
+                tss_host = float(target_scores_sum)  # a CPU value: no device round trip
+        else:
+            tss_host = float(target_scores_sum)
+        x, pb, ap = _dense32(pred_dist.detach()), pred_bboxes.detach().contiguous(), anchor_points.detach().contiguous()
+        tb, ts, fg = target_bboxes.contiguous(), target_scores.contiguous(), fg_mask.contiguous()
+        loss_iou = torch.empty((), dtype=torch.float32, device=dev)
+        loss_dfl = torch.empty((), dtype=torch.float32, device=dev)
+        ws_bytes = int(lib.cerb_bbox_loss_workspace_bytes(B, A))
+        ws = torch.zeros((ws_bytes,), dtype=torch.uint8, device=dev)
+        if per_anchor is not None and (tuple(per_anchor.shape) != (B, A, 2) or per_anchor.dtype != torch.float32
+                                       or not per_anchor.is_contiguous() or per_anchor.device != dev):
+            raise ValueError(f"per_anchor must be a contiguous float32 [{B}, {A}, 2] tensor on {dev}")
+        tss_ptr = tss_dev.data_ptr() if tss_dev is not None else None
+        with torch.cuda.device(dev):
+            rc = lib.cerb_bbox_loss_fwd(x.data_ptr(), pb.data_ptr(), ap.data_ptr(), tb.data_ptr(), ts.data_ptr(), fg.data_ptr(),
+                                        tss_ptr, tss_host, B, A, C, 16, code, loss_iou.data_ptr(), loss_dfl.data_ptr(),
+                                        per_anchor.data_ptr() if per_anchor is not None else None, ws.data_ptr(), ws_bytes,
+                                        _stream_ptr(dev))
+        _lib.check(rc)
+        ctx.save_for_backward(x, pb, ap, tb, ts, fg, tss_dev)
+        ctx.meta = (B, A, C, code, tss_dev is not None, tss_host)
+        return loss_iou, loss_dfl
+
+    @staticmethod
+    def backward(ctx, g_iou, g_dfl):
+        x, pb, ap, tb, ts, fg, tss = ctx.saved_tensors
+        B, A, C, code, has_tss, tss_host = ctx.meta
+        lib = _lib.load()
+        dev = x.device
+        g_iou = torch.zeros((), dtype=torch.float32, device=dev) if g_iou is None else g_iou.detach().reshape(()).float()
+        g_dfl = torch.zeros((), dtype=torch.float32, device=dev) if g_dfl is None else g_dfl.detach().reshape(()).float()
+        grad_dist = torch.empty_like(x)
+        grad_boxes = torch.empty_like(pb)
+        with torch.cuda.device(dev):
+            rc = lib.cerb_bbox_loss_bwd(x.data_ptr(), pb.data_ptr(), ap.data_ptr(), tb.data_ptr(), ts.data_ptr(), fg.data_ptr(),
+                                        tss.data_ptr() if has_tss else None, tss_host, B, A, C, 16, code, g_iou.data_ptr(),
+                                        g_dfl.data_ptr(), grad_dist.data_ptr(), grad_boxes.data_ptr(), _stream_ptr(dev))
+        _lib.check(rc)
+        return grad_dist, grad_boxes, None, None, None, None, None, None
+
+
+def bbox_loss(pred_dist: torch.Tensor, pred_bboxes: torch.Tensor, anchor_points: torch.Tensor, target_bboxes: torch.Tensor,
+              target_scores: torch.Tensor, target_scores_sum, fg_mask: torch.Tensor,
+              per_anchor: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Drop-in for the reference's ``BboxLoss(reg_max=15, use_dfl=True).forward`` (utils/loss.py:12-44):
+    ``(loss_iou, loss_dfl)`` as 0-d float32 tensors, differentiable in ``pred_dist [B, A, 64]`` and
+    ``pred_bboxes [B, A, 4]``.  No host synchronisation: the foreground mask is read by the kernels, and
+    ``target_scores_sum`` (a 0-d CUDA tensor, or a number such as the call site's ``1``) is read on the device.
+
+    Two dtype combinations: everything float32; or the trainer's fp16-autocast case -- ``pred_dist``, ``pred_bboxes`` and
+    ``anchor_points`` float16, ``target_bboxes`` / ``target_scores`` float32 -- with the reference's half roundings.
+    ``per_anchor`` (float32 ``[B, A, 2]``, optional) receives the per-anchor terms ``(1 - CIoU) * weight`` and
+    ``DFL * weight`` (zero at background anchors)."""
+    return _BboxLoss.apply(pred_dist, pred_bboxes, anchor_points, target_bboxes, target_scores, target_scores_sum, fg_mask, per_anchor)

@@ -15,6 +15,12 @@ What gets rebound (and restored by ``uninstall()``):
   ``dist2bbox`` stays in fp16 -- exactly the half path of the kernels (probabilities rounded to half, one rounding of
   the expectation, one per corner), so fp16 ``pred_dist`` + fp16 anchors under autocast go to the kernels; any other
   dtype mix (fp32 under autocast, anchors of another dtype) keeps the reference's own code;
+* with ``loss=True`` ``cerberusdet.utils.loss.BboxLoss.forward`` -> ``ops.bbox_loss`` (the box-regression term the loss
+  computes right after the assigner, reference utils/loss.py:12-44: CIoU + DFL in one forward and one backward kernel, no
+  host synchronisation).  On the path: ``use_dfl`` with 16 bins, CUDA tensors, and either everything fp32 without
+  autocast or the trainer's fp16 autocast case (fp16 ``pred_dist`` / ``pred_bboxes`` / ``anchor_points``, fp32 targets);
+  anything else (CPU tensors, ``use_dfl=False``, another ``reg_max``, other dtype mixes, bf16 autocast) keeps the
+  reference's own code;
 * with ``val=True`` the validation loop's per-image matching (val.py:32-54 ``process_batch``) -> ``ops.match_batch``.
 
 CUDA fp16/fp32 tensors go to the kernels; anything else (CPU tensors, training mode, masks/labels
@@ -40,14 +46,14 @@ def installed() -> bool:
     return bool(_saved)
 
 
-def install(import_all: bool = False, train: bool = False, val: bool = False) -> Dict[str, List[str]]:
+def install(import_all: bool = False, train: bool = False, val: bool = False, loss: bool = False) -> Dict[str, List[str]]:
     """Patch the reference modules that are importable.  ``import_all`` also imports ``val`` /
     ``detect`` / ``cerberusdet_inference`` (they pull in the whole data pipeline); by default only
     modules already imported, plus ``models.yolo`` and ``utils.general``, are touched.  ``train`` also rebinds
     ``Loss.bbox_decode``, ``TaskAlignedAssigner.forward`` and the loss module's ``make_anchors`` (imports
-    ``cerberusdet.utils.loss``), ``val`` the validation matching (imports
-    ``cerberusdet.val``).  Calling it again adds whatever is not patched yet (e.g. ``install()`` then
-    ``install(train=True)``)."""
+    ``cerberusdet.utils.loss``), ``loss`` the box-regression term ``BboxLoss.forward`` (imports
+    ``cerberusdet.utils.loss``), ``val`` the validation matching (imports ``cerberusdet.val``).  Calling it again adds
+    whatever is not patched yet (e.g. ``install()`` then ``install(train=True)``, then ``install(loss=True)``)."""
     import torch
 
     from . import detect as _detect
@@ -161,6 +167,33 @@ def install(import_all: bool = False, train: bool = False, val: bool = False) ->
 
             make_anchors._cerb_reference = reference_make_anchors
             patch_once(loss_mod, "make_anchors", make_anchors, "cerberusdet.utils.loss.make_anchors")
+    if loss:
+        from . import ops as _ops
+
+        loss_mod = importlib.import_module("cerberusdet.utils.loss")
+        if not hasattr(loss_mod.BboxLoss.forward, "_cerb_reference"):
+            reference_bbox_loss = loss_mod.BboxLoss.forward
+
+            def bbox_loss_forward(self, pred_dist, pred_bboxes, anchor_points, target_bboxes, target_scores, target_scores_sum,
+                                  fg_mask):
+                tensors = (pred_dist, pred_bboxes, anchor_points, target_bboxes, target_scores, fg_mask)
+                on_path = (self.use_dfl and self.reg_max == 15 and all(t.is_cuda for t in tensors) and pred_dist.dim() == 3
+                           and pred_dist.shape[-1] == 64 and fg_mask.dtype == torch.bool
+                           and target_bboxes.dtype == torch.float32 and target_scores.dtype == torch.float32
+                           and pred_bboxes.dtype == pred_dist.dtype and anchor_points.dtype == pred_dist.dtype)
+                if on_path and torch.is_autocast_enabled("cuda"):
+                    # fp16 autocast: half predictions, fp32 targets -- the kernels' half mode
+                    on_path = pred_dist.dtype == torch.float16 and torch.get_autocast_dtype("cuda") == torch.float16
+                elif on_path:
+                    on_path = pred_dist.dtype == torch.float32
+                if not on_path:  # CPU tensors, use_dfl=False, reg_max != 15, other dtype mixes: the reference's own code
+                    return reference_bbox_loss(self, pred_dist, pred_bboxes, anchor_points, target_bboxes, target_scores,
+                                               target_scores_sum, fg_mask)
+                return _ops.bbox_loss(pred_dist, pred_bboxes, anchor_points, target_bboxes, target_scores, target_scores_sum,
+                                      fg_mask)
+
+            bbox_loss_forward._cerb_reference = reference_bbox_loss
+            patch_once(loss_mod.BboxLoss, "forward", bbox_loss_forward, "cerberusdet.utils.loss.BboxLoss.forward")
     if val:
         from . import val_stats as _val_stats
 

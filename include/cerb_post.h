@@ -294,6 +294,45 @@ int cerb_tal_assign(const void* pd_scores, const float* pd_bboxes, const float* 
                     size_t workspace_bytes, void* stream);
 
 /*
+ * The box-regression term of the training loss (SURVEY 8f row 4, the step after the assigner): BboxLoss.forward
+ * (cerberusdet/utils/loss.py:12-44) with use_dfl and 16 bins, i.e. the CIoU loss (bbox_iou(xywh=False, CIoU=True),
+ * utils/metrics.py:373-408) and the distribution focal loss against bbox2dist(anchor_points, target_bboxes, 15)
+ * (utils/tal.py:208-211), both summed over the foreground anchors, weighted by the target-score row sums and divided by
+ * target_scores_sum.  One launch; no host synchronisation (the reference's boolean-mask indexing costs five).
+ *
+ *   pred_dist      [B, A, 4 * reg_max] (bins of a side contiguous), dtype, 32-byte aligned
+ *   pred_bboxes    [B, A, 4] xyxy grid units, dtype        anchor_points [A, 2] grid units, dtype
+ *   target_bboxes  [B, A, 4] xyxy grid units, fp32        target_scores [B, A, C] fp32      fg_mask [B, A] bool bytes
+ *   target_scores_sum   device fp32 scalar, or NULL: target_scores_sum_host is used
+ *   dtype          CERB_F32: every tensor above fp32.  CERB_F16: the trainer's fp16 autocast case -- half predictions and
+ *                  anchors, fp32 targets; the reference's half roundings (w1, h1, w1*h1, w1/h1, atan(w1/h1), the
+ *                  cross-entropy's log-probabilities) are kept
+ *   loss_iou, loss_dfl   out: device fp32 scalars
+ *   per_anchor     optional out [B, A, 2] fp32: (1 - CIoU) * weight and DFL * weight per anchor (0 at background), or NULL
+ *   workspace      cerb_bbox_loss_workspace_bytes(B, A) bytes, 16-byte aligned, ZEROED before its first use (the
+ *                  kernel leaves it reusable: it resets its counter, so CUDA-graph replays need nothing else)
+ * Sums are reduced in a fixed order: equal inputs give equal bits.  reg_max must be 16; CERB_EINVAL for another value,
+ * an unknown dtype, misaligned rows or B*A beyond 2^31 - 1.
+ */
+size_t cerb_bbox_loss_workspace_bytes(int B, int A);
+int cerb_bbox_loss_fwd(const void* pred_dist, const void* pred_bboxes, const void* anchor_points, const float* target_bboxes,
+                       const float* target_scores, const unsigned char* fg_mask, const float* target_scores_sum,
+                       double target_scores_sum_host, int B, int A, int C, int reg_max, int dtype, float* loss_iou,
+                       float* loss_dfl, float* per_anchor, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * Its backward (loss.py:12-44, tal.py:208-211, metrics.py:373-408), recomputed from the same inputs: grad_iou and
+ * grad_dfl are the device fp32 gradients of the two scalars; out grad_pred_dist [B, A, 64] (dense: zeros at background
+ * anchors, 32-byte aligned) and grad_pred_bboxes [B, A, 4], both in dtype.  Autograd's conventions: CIoU's alpha is a
+ * constant, minimum / maximum split the gradient in half on exact ties, clamp(0) passes it at exactly 0, and the
+ * cross-entropy gradient is softmax - onehot in fp32, rounded once to dtype.
+ */
+int cerb_bbox_loss_bwd(const void* pred_dist, const void* pred_bboxes, const void* anchor_points, const float* target_bboxes,
+                       const float* target_scores, const unsigned char* fg_mask, const float* target_scores_sum,
+                       double target_scores_sum_host, int B, int A, int C, int reg_max, int dtype, const float* grad_iou,
+                       const float* grad_dfl, void* grad_pred_dist, void* grad_pred_bboxes, void* stream);
+
+/*
  * Test / tools hooks.  cerb_debug_set(name, value) overrides one internal choice FOR THE CALLING THREAD (so the
  * library stays re-entrant); cerb_debug_reset() drops every override of the calling thread.  Results never depend
  * on a knob: the parity tests run the alternatives against each other.  Knobs: "decode_pipe" (0 = register-resident
