@@ -245,7 +245,7 @@ def bbox_decode_port(anchor_points: torch.Tensor, pred_dist: torch.Tensor) -> to
     (utils/tal.py:196-205): ``pred_dist [B, A, 64]`` (bins of a side contiguous) and ``anchor_points [A, 2]`` ->
     ``[B, A, 4]`` = (x1, y1, x2, y2) in grid units.  Differentiable (the test compares autograd gradients too)."""
     b, a, c = pred_dist.shape
-    proj = torch.arange(REG_MAX, dtype=torch.float)
+    proj = torch.arange(REG_MAX, dtype=torch.float, device=pred_dist.device)
     dist = pred_dist.view(b, a, 4, c // 4).softmax(3).matmul(proj.type(pred_dist.dtype))
     lt, rb = torch.split(dist, 2, -1)
     return torch.cat((anchor_points - lt, anchor_points + rb), -1)
@@ -290,7 +290,7 @@ def ciou_port(box1: torch.Tensor, box2: torch.Tensor, eps: float = 1e-7) -> torc
 
 def tal_assign_port(pd_scores: torch.Tensor, pd_bboxes: torch.Tensor, anc_points: torch.Tensor, gt_labels: torch.Tensor,
                     gt_bboxes: torch.Tensor, mask_gt: torch.Tensor, topk: int = 10, num_classes: int = 80, alpha: float = 0.5,
-                    beta: float = 6.0, eps: float = 1e-9):
+                    beta: float = 6.0, eps: float = 1e-9, claims: bool = False):
     """``TaskAlignedAssigner.forward`` (utils/tal.py:56-178, with ``select_candidates_in_gts`` :13-28 and
     ``select_highest_overlaps`` :31-53) restated stage by stage.  One thing is made canonical: the reference's
     ``torch.topk`` (:140) leaves the order of EQUAL metrics unspecified; here ties go to the lower anchor index.  That
@@ -299,7 +299,8 @@ def tal_assign_port(pd_scores: torch.Tensor, pd_bboxes: torch.Tensor, anc_points
     ``ambiguous [B, G]`` (last return value) flags those boxes so that tests compare the others.
 
     Returns ``(target_labels [B, A] int64, target_bboxes [B, A, 4], target_scores [B, A, C], fg_mask [B, A] bool,
-    target_gt_idx [B, A] int64, ambiguous [B, G] bool)``."""
+    target_gt_idx [B, A] int64, ambiguous [B, G] bool)``; with ``claims=True`` also ``[B, A]`` int64, the number of boxes
+    whose top-k claims each anchor before ``select_highest_overlaps`` resolves anchors claimed by several."""
     bs, n_max = pd_scores.size(0), gt_bboxes.size(1)
     A = pd_scores.size(1)
     if n_max == 0:
@@ -329,6 +330,7 @@ def tal_assign_port(pd_scores: torch.Tensor, pd_bboxes: torch.Tensor, anc_points
     ambiguous = (n_positive < topk) & (n_zero_inside > 0) & (mask_gt.squeeze(-1) > 0)
     # select_highest_overlaps (:31-53)
     fg_mask = mask_pos.sum(-2)
+    n_claims = fg_mask.long()
     if fg_mask.max() > 1:
         mask_multi = (fg_mask.unsqueeze(1) > 1).repeat([1, n_max, 1])
         is_max = F.one_hot(overlaps.argmax(1), n_max).permute(0, 2, 1).to(overlaps.dtype)
@@ -346,7 +348,8 @@ def tal_assign_port(pd_scores: torch.Tensor, pd_bboxes: torch.Tensor, anc_points
     pos_align = align_metric.amax(-1, keepdim=True)
     pos_ov = (overlaps * mask_pos).amax(-1, keepdim=True)
     norm = (align_metric * pos_ov / (pos_align + eps)).amax(-2).unsqueeze(-1)
-    return target_labels, target_bboxes, target_scores * norm, fg_mask.bool(), target_gt_idx, ambiguous
+    out = (target_labels, target_bboxes, target_scores * norm, fg_mask.bool(), target_gt_idx, ambiguous)
+    return out + (n_claims,) if claims else out
 
 
 def tal_case(seed: int, bs: int, level_hw, strides, nc: int, n_gt: int, noise: float = 4.0, score_dtype=torch.float32):

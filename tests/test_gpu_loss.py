@@ -37,7 +37,8 @@ def ops():
 
 
 def _grads_close(got, want, rtol, group, half):
-    """``|got - want| <= rtol * (|want| + S) (+ one half ulp of S)``, S = max |want| over groups of ``group`` values."""
+    """``|got - want| <= rtol * (|want| + S) (+ one half ulp of S)``, S = max |want| over groups of ``group`` values.
+    Returns the worst ``|got - want| / bound``."""
     g, w = got.float().cpu(), want.float().cpu()
     S = w.abs().reshape(-1, group).amax(-1, keepdim=True).expand(-1, group).reshape(w.shape)
     bound = rtol * (w.abs() + S) + 1e-30
@@ -47,6 +48,7 @@ def _grads_close(got, want, rtol, group, half):
     assert torch.isfinite(g).all()
     ok = d <= bound
     assert ok.all(), f"worst excess {(d - bound).max().item():.3e} of {int((~ok).sum())} values"
+    return float((d / bound).max())
 
 
 def _case(ops, kind, dtype=torch.float32):
