@@ -39,6 +39,8 @@ EXPORTS = (
     "cerb_bbox_loss_workspace_bytes",
     "cerb_bbox_loss_fwd",
     "cerb_bbox_loss_bwd",
+    "cerb_ap_workspace_bytes",
+    "cerb_ap_per_class",
     "cerb_debug_set",
     "cerb_debug_reset",
     "cerb_debug_set_chunking",
@@ -129,6 +131,11 @@ def load() -> ctypes.CDLL:
         lib.cerb_bbox_loss_fwd.argtypes = [vp] * 7 + [d] + [i] * 5 + [vp] * 4 + [sz, vp]
         lib.cerb_bbox_loss_bwd.restype = i
         lib.cerb_bbox_loss_bwd.argtypes = [vp] * 7 + [d] + [i] * 5 + [vp] * 5
+    if hasattr(lib, "cerb_ap_per_class") or "CERB_LIB" not in os.environ:
+        lib.cerb_ap_workspace_bytes.restype = sz
+        lib.cerb_ap_workspace_bytes.argtypes = [lg, i, i]
+        lib.cerb_ap_per_class.restype = i
+        lib.cerb_ap_per_class.argtypes = [vp, i, vp, vp, lg, vp, vp, i, d, vp, vp, vp, vp, sz, vp]
     if hasattr(lib, "cerb_debug_set") or "CERB_LIB" not in os.environ:  # (tools/ A/B runs may load an older build)
         lib.cerb_debug_set.restype = i
         lib.cerb_debug_set.argtypes = [ctypes.c_char_p, i]

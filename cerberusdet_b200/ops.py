@@ -833,3 +833,51 @@ def bbox_loss(pred_dist: torch.Tensor, pred_bboxes: torch.Tensor, anchor_points:
     ``per_anchor`` (float32 ``[B, A, 2]``, optional) receives the per-anchor terms ``(1 - CIoU) * weight`` and
     ``DFL * weight`` (zero at background anchors)."""
     return _BboxLoss.apply(pred_dist, pred_bboxes, anchor_points, target_bboxes, target_scores, target_scores_sum, fg_mask, per_anchor)
+
+
+# ----------------------------------------------------------------------------- validation mAP statistics
+def ap_per_class(tp: torch.Tensor, conf: torch.Tensor, pred_cls: torch.Tensor, target_cls: torch.Tensor, eps: float = 1e-16):
+    """The GPU part of the reference's ``ap_per_class`` (utils/metrics.py:56-120, with ``compute_ap``) in one
+    ``cerb_ap_per_class`` call: ``tp [N, K]`` bool (K <= 32 IoU thresholds), ``conf`` / ``pred_cls [N]`` and
+    ``target_cls [M]`` float16 | float32, all CUDA tensors.  Returns device tensors ``(ap [nc, K], p [nc, 1000],
+    r [nc, 1000])`` float64 and ``(unique_classes [nc] float32, nt [nc] int64)`` as ``np.unique(target_cls,
+    return_counts=True)`` gives them.  Equal confidences are ordered by row index (``np.argsort(-conf, kind="stable")``).
+
+    For callers that hold the statistics on the device (``val_stats.validation_batch_statistics``): concatenate them there
+    and call this, with no host round trip for the ``[N, K]`` rows; only ``nc`` class values come to the host.  NaN in
+    ``conf`` or ``target_cls`` raises ``ValueError``."""
+    lib = _lib.load()
+    for t, what in ((tp, "tp"), (conf, "conf"), (pred_cls, "pred_cls"), (target_cls, "target_cls")):
+        _require_cuda(t, what)
+        if t is not tp and t.dtype not in (torch.float16, torch.float32):
+            raise TypeError(f"{what} must be float16 or float32, got {t.dtype}")
+    if tp.dtype != torch.bool or tp.dim() != 2:
+        raise TypeError(f"tp must be a [N, K] bool tensor, got {tp.dtype} {tuple(tp.shape)}")
+    n, K = (int(v) for v in tp.shape)
+    if not 1 <= K <= 32:
+        raise ValueError(f"tp has {K} IoU thresholds, 1..32 supported")
+    if tuple(conf.shape) != (n,) or tuple(pred_cls.shape) != (n,):
+        raise ValueError(f"conf and pred_cls must be [{n}], got {tuple(conf.shape)} and {tuple(pred_cls.shape)}")
+    dev = tp.device
+    conf32, cls32 = conf.to(dev, torch.float32).contiguous(), pred_cls.to(dev, torch.float32).contiguous()
+    target = target_cls.to(dev, torch.float32).reshape(-1)
+    nan_target, nan_conf = torch.stack((target.isnan().any(), conf32.isnan().any())).tolist()
+    if nan_target or nan_conf:
+        raise ValueError("target_cls contains NaN" if nan_target else "conf contains NaN")
+    classes, nt = torch.unique(target, sorted=True, return_counts=True)
+    classes_h, nt_h = classes.cpu(), nt.cpu()
+    nc = int(classes.numel())
+    tpc = tp.contiguous()
+    ap = torch.empty((nc, K), dtype=torch.float64, device=dev)
+    p = torch.empty((nc, 1000), dtype=torch.float64, device=dev)
+    r = torch.empty((nc, 1000), dtype=torch.float64, device=dev)
+    ws_bytes = int(lib.cerb_ap_workspace_bytes(n, K, nc))
+    ws = torch.empty((max(ws_bytes, 1),), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        rc = lib.cerb_ap_per_class(tpc.data_ptr(), K, conf32.data_ptr(), cls32.data_ptr(), n, classes_h.data_ptr(),
+                                   nt_h.data_ptr(), nc, float(eps), ap.data_ptr(), p.data_ptr(), r.data_ptr(), ws.data_ptr(),
+                                   ws_bytes, _stream_ptr(dev))
+    _lib.check(rc)
+    for t in (tpc, conf32, cls32, ws):
+        t.record_stream(torch.cuda.current_stream(dev))
+    return ap, p, r, classes, nt

@@ -21,7 +21,12 @@ What gets rebound (and restored by ``uninstall()``):
   autocast or the trainer's fp16 autocast case (fp16 ``pred_dist`` / ``pred_bboxes`` / ``anchor_points``, fp32 targets);
   anything else (CPU tensors, ``use_dfl=False``, another ``reg_max``, other dtype mixes, bf16 autocast) keeps the
   reference's own code;
-* with ``val=True`` the validation loop's per-image matching (val.py:32-54 ``process_batch``) -> ``ops.match_batch``.
+* with ``val=True`` the validation loop's per-image matching (val.py:32-54 ``process_batch``) -> ``ops.match_batch``;
+* with ``metrics=True`` ``ap_per_class`` (utils/metrics.py:56-120), which ``DetMetrics.process`` reads as a module global,
+  -> ``val_stats.ap_per_class`` (``ops.ap_per_class`` for the per-class curves and APs, the host tail in numpy), in
+  ``cerberusdet.utils.metrics`` and in every imported ``cerberusdet.*`` module that imported the name.  ``plot=True``,
+  no CUDA device, non-bool ``tp``, more than 32 IoU columns, float64 inputs or NaN scores / classes keep the reference's
+  own function.
 
 CUDA fp16/fp32 tensors go to the kernels; anything else (CPU tensors, training mode, masks/labels
 arguments) is handed to the reference's own, saved implementation -- the patch never changes what a
@@ -46,13 +51,15 @@ def installed() -> bool:
     return bool(_saved)
 
 
-def install(import_all: bool = False, train: bool = False, val: bool = False, loss: bool = False) -> Dict[str, List[str]]:
+def install(import_all: bool = False, train: bool = False, val: bool = False, loss: bool = False,
+            metrics: bool = False) -> Dict[str, List[str]]:
     """Patch the reference modules that are importable.  ``import_all`` also imports ``val`` /
     ``detect`` / ``cerberusdet_inference`` (they pull in the whole data pipeline); by default only
     modules already imported, plus ``models.yolo`` and ``utils.general``, are touched.  ``train`` also rebinds
     ``Loss.bbox_decode``, ``TaskAlignedAssigner.forward`` and the loss module's ``make_anchors`` (imports
     ``cerberusdet.utils.loss``), ``loss`` the box-regression term ``BboxLoss.forward`` (imports
-    ``cerberusdet.utils.loss``), ``val`` the validation matching (imports ``cerberusdet.val``).  Calling it again adds
+    ``cerberusdet.utils.loss``), ``val`` the validation matching (imports ``cerberusdet.val``), ``metrics`` the mAP
+    statistics ``ap_per_class`` (imports ``cerberusdet.utils.metrics``).  Calling it again adds
     whatever is not patched yet (e.g. ``install()`` then ``install(train=True)``, then ``install(loss=True)``)."""
     import torch
 
@@ -201,6 +208,16 @@ def install(import_all: bool = False, train: bool = False, val: bool = False, lo
         if not hasattr(val_mod.process_batch, "_cerb_reference"):
             patch_once(val_mod, "process_batch", _val_stats.make_process_batch(val_mod.process_batch),
                        "cerberusdet.val.process_batch")
+    if metrics:
+        from . import val_stats as _val_stats
+
+        metrics_mod = importlib.import_module("cerberusdet.utils.metrics")
+        cur = metrics_mod.ap_per_class
+        ap_per_class = cur if hasattr(cur, "_cerb_reference") else _val_stats.make_ap_per_class(cur)
+        for modname, mod in list(sys.modules.items()):
+            if (modname == "cerberusdet" or modname.startswith("cerberusdet.")) and hasattr(mod, "ap_per_class") \
+                    and mod.ap_per_class is ap_per_class._cerb_reference:
+                patch_once(mod, "ap_per_class", ap_per_class, f"{modname}.ap_per_class")
     if not done["patched"]:
         return {"already": ["installed"]}
     return done

@@ -7,9 +7,16 @@ descending; every detection keeps its first pair (its best label), the survivors
 are de-duplicated per label keeping the first, i.e. the lowest detection index (val.py:48-51).  The reference sorts with
 numpy's unstable default, so exactly equal IoUs have no defined order there; the canonical rule here (and in the CUDA
 kernel) is "IoU descending, then label index ascending".
+
+After the loop: ``ap_per_class`` (cerberusdet/utils/metrics.py:56-120), the drop-in whose per-class curves and APs come
+from ``ops.ap_per_class`` and whose O(nc * 1000) tail runs here in numpy, and ``make_ap_per_class``, its guarded form for
+``patch.install(metrics=True)``.
 """
 from __future__ import annotations
 
+from pathlib import Path
+
+import numpy as np
 import torch
 
 from .cross_task import pairwise_iou
@@ -169,3 +176,73 @@ def validation_batch_statistics(dets: torch.Tensor, counts: torch.Tensor, batch:
             continue
         stats.append((correct[i, :n], pred[i, :n, 4], pred[i, :n, 5], tcls))
     return stats
+
+
+# ------------------------------------------------------------------------------------ mAP statistics (after the loop)
+def _smooth(y, f=0.05):
+    """Box filter of fraction ``f`` (utils/metrics.py ``smooth``)."""
+    nf = round(len(y) * f * 2) // 2 + 1
+    p = np.ones(nf // 2)
+    yp = np.concatenate((p * y[0], y, p * y[-1]), 0)
+    return np.convolve(yp, np.ones(nf) / nf, mode="valid")
+
+
+def _on_device(x, device):
+    return x.to(device) if torch.is_tensor(x) else torch.from_numpy(np.ascontiguousarray(x)).to(device)
+
+
+def ap_per_class(tp, conf, pred_cls, target_cls, plot=False, save_dir=Path(), names=(), eps=1e-16, prefix=""):
+    """Drop-in for the reference's ``ap_per_class`` (utils/metrics.py:56-120) with its signature and 7-tuple of numpy
+    arrays ``(tp, fp, p, r, f1, ap, unique_classes)``.  Inputs are numpy arrays (copied to the device) or CUDA tensors.
+    ``ap`` and the ``p`` / ``r`` curves come from ``ops.ap_per_class``; the O(nc * 1000) tail (f1, ``smooth``, argmax, the
+    rounded tp / fp) runs here in numpy, as in the reference.  Equal confidences are ordered by row index, which is
+    ``np.argsort(-conf, kind="stable")``; the reference's unstable argsort leaves their order undefined.  Plots are not
+    drawn: ``plot=True`` raises (``make_ap_per_class`` sends it to the reference)."""
+    from . import ops
+
+    if plot:
+        raise ValueError("ap_per_class: plot=True is the reference's (it draws the curves with matplotlib)")
+    device = next((x.device for x in (tp, conf, pred_cls, target_cls) if torch.is_tensor(x) and x.is_cuda), torch.device("cuda"))
+    tp, conf, pred_cls, target_cls = (_on_device(x, device) for x in (tp, conf, pred_cls, target_cls))
+    ap, p, r, unique_classes, nt = (t.cpu().numpy() for t in ops.ap_per_class(tp, conf.reshape(-1), pred_cls.reshape(-1),
+                                                                              target_cls.reshape(-1), eps=eps))
+    f1 = 2 * p * r / (p + r + eps)
+    names = [v for k, v in names.items() if k in unique_classes]  # (used by the reference's plots only)
+    names = dict(enumerate(names))
+    i = _smooth(f1.mean(0), 0.1).argmax()  # max F1 index
+    p, r, f1 = p[:, i], r[:, i], f1[:, i]
+    tp = (r * nt).round()  # true positives
+    fp = (tp / (p + eps) - tp).round()  # false positives
+    return tp, fp, p, r, f1, ap, unique_classes.astype(int)
+
+
+def _ap_on_path(tp, conf, pred_cls, target_cls, kwargs) -> bool:
+    if kwargs.get("plot") or set(kwargs) - {"plot", "save_dir", "names", "eps", "prefix"} or not torch.cuda.is_available():
+        return False
+    arrays = (tp, conf, pred_cls, target_cls)
+    if not all(isinstance(x, np.ndarray) or (torch.is_tensor(x) and x.is_cuda) for x in arrays):
+        return False
+    if tp.dtype not in (np.bool_, torch.bool) or tp.ndim != 2 or not 1 <= tp.shape[1] <= 32:
+        return False
+    if any(x.dtype not in (np.float16, np.float32, torch.float16, torch.float32) for x in arrays[1:]):
+        return False
+    if conf.shape != (tp.shape[0],) or pred_cls.shape != (tp.shape[0],):
+        return False
+    nan = lambda x: bool(torch.isnan(x).any()) if torch.is_tensor(x) else bool(np.isnan(x).any())  # noqa: E731
+    return not (nan(conf) or nan(target_cls))
+
+
+def make_ap_per_class(reference_ap_per_class):
+    """``ap_per_class`` for ``cerberusdet.utils.metrics`` (``patch.install(metrics=True)``): ``DetMetrics.process`` calls
+    it once per task at the end of validation (utils/metrics.py:241-246).  Anything off the kernels' path runs the
+    reference's own function: ``plot=True`` (the curves are drawn with matplotlib), no CUDA device, ``tp`` not bool or
+    with more than 32 IoU columns, float64 scores or classes, NaN in ``conf`` or ``target_cls``, CPU tensors."""
+
+    def ap_per_class_(tp, conf, pred_cls, target_cls, **kwargs):
+        if not _ap_on_path(tp, conf, pred_cls, target_cls, kwargs):
+            return reference_ap_per_class(tp, conf, pred_cls, target_cls, **kwargs)
+        return ap_per_class(tp, conf, pred_cls, target_cls, **kwargs)
+
+    ap_per_class_.__doc__ = ap_per_class.__doc__
+    ap_per_class_._cerb_reference = reference_ap_per_class
+    return ap_per_class_

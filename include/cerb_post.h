@@ -333,6 +333,31 @@ int cerb_bbox_loss_bwd(const void* pred_dist, const void* pred_bboxes, const voi
                        const float* grad_dfl, void* grad_pred_dist, void* grad_pred_bboxes, void* stream);
 
 /*
+ * Per-class average precision of the validation statistics: ap_per_class (cerberusdet/utils/metrics.py:56-120) with
+ * compute_ap (np.interp of the precision envelope at np.linspace(0, 1, 101), np.trapz), up to the per-class arrays; the
+ * caller does the O(nc * 1000) tail (f1, smooth, argmax, rounded tp / fp).  Detections are ordered by conf descending,
+ * ties by row index ascending: np.argsort(-conf, kind="stable"), with -0.0 == 0.0 (the reference's unstable argsort has
+ * no defined order on ties).  Every float64 value is the reference's own IEEE operation, so the outputs equal numpy's
+ * bit for bit.
+ *
+ *   tp        [n, K] bytes, nonzero = true positive at IoU threshold j     conf, pred_cls   [n] fp32
+ *   classes   HOST [nc] fp32, strictly ascending (np.unique of the target classes); a detection whose class is not
+ *             among them (or NaN) is ignored, as `pred_cls == c` ignores it
+ *   n_labels  HOST [nc] labels per class (np.unique's counts)                eps              the reference's 1e-16
+ *   ap        out [nc, K] fp64      p, r   out [nc, 1000] fp64: precision / recall at px = np.linspace(0, 1, 1000) of
+ *             column 0, np.interp(-px, -conf, ., left=1 | 0).  A class with no detection or no label keeps zero rows.
+ *   workspace cerb_ap_workspace_bytes(n, K, nc) bytes, 256-byte aligned (0 returned: the size cannot be computed,
+ *             e.g. without a CUDA device)
+ * Requires what process_batch guarantees: per class and column, at most n_labels true positives (recall <= 1).
+ * CERB_EINVAL for n outside 0..2^31-1, K outside 1..32, nc < 0, classes not strictly ascending or NaN, negative
+ * n_labels; CERB_ENOSPC for a workspace that is too small.  n == 0 or nc == 0 is valid (zero outputs).
+ */
+size_t cerb_ap_workspace_bytes(long n, int K, int nc);
+int cerb_ap_per_class(const unsigned char* tp, int K, const float* conf, const float* pred_cls, long n, const float* classes,
+                      const long long* n_labels, int nc, double eps, double* ap, double* p, double* r, void* workspace,
+                      size_t workspace_bytes, void* stream);
+
+/*
  * Test / tools hooks.  cerb_debug_set(name, value) overrides one internal choice FOR THE CALLING THREAD (so the
  * library stays re-entrant); cerb_debug_reset() drops every override of the calling thread.  Results never depend
  * on a knob: the parity tests run the alternatives against each other.  Knobs: "decode_pipe" (0 = register-resident
