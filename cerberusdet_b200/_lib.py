@@ -14,39 +14,6 @@ LIB_PATH = os.environ.get("CERB_LIB") or os.path.join(_HERE, "libcerb_post.so") 
 CERB_F16, CERB_F32 = 0, 1
 CERB_EINVAL, CERB_ECUDA, CERB_ENOSPC = -1, -2, -3
 
-EXPORTS = (
-    "cerb_version",
-    "cerb_last_error",
-    "cerb_decode",
-    "cerb_decode_split",
-    "cerb_head_tail",
-    "cerb_summary_row_len",
-    "cerb_nms_workspace_bytes",
-    "cerb_nms",
-    "cerb_nms_stats",
-    "cerb_nms_deliver",
-    "cerb_deliver_collect",
-    "cerb_deliver_push",
-    "cerb_decode_nms",
-    "cerb_cross_task",
-    "cerb_cross_task_workspace_bytes",
-    "cerb_cross_task_ws",
-    "cerb_val_match",
-    "cerb_bbox_decode_fwd",
-    "cerb_bbox_decode_bwd",
-    "cerb_tal_workspace_bytes",
-    "cerb_tal_assign",
-    "cerb_bbox_loss_workspace_bytes",
-    "cerb_bbox_loss_fwd",
-    "cerb_bbox_loss_bwd",
-    "cerb_ap_workspace_bytes",
-    "cerb_ap_per_class",
-    "cerb_debug_set",
-    "cerb_debug_reset",
-    "cerb_debug_set_chunking",
-    "cerb_debug_set_hist_sample",
-)
-
 _lib = None
 
 
@@ -57,6 +24,46 @@ class Delivery(ctypes.Structure):
                 ("flag_remote", ctypes.c_void_p), ("ack_local", ctypes.c_void_p), ("seq_local", ctypes.c_void_p),
                 ("done_local", ctypes.c_void_p), ("collect_flags", ctypes.c_void_p), ("collect_ack", ctypes.c_void_p * 16),
                 ("collect_count", ctypes.c_void_p), ("world", ctypes.c_int), ("dst", ctypes.c_int)]
+
+
+_vp, _ip, _i, _d, _sz, _lg = ctypes.c_void_p, ctypes.POINTER(ctypes.c_int), ctypes.c_int, ctypes.c_double, ctypes.c_size_t, ctypes.c_long
+_vpp, _fp = ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_float)
+_NMS = [_vpp, _ip, _i, _i, _i, _i, _d, _d, _ip, _i, _i, _i, _i, _i, _d, _vpp, _vp, _vp, _vp, _sz]  # shared head of the cerb_nms* calls
+
+# {name: (restype, argtypes)} of every entry point of include/cerb_post.h
+PROTOTYPES = {
+    "cerb_version": (_i, []),
+    "cerb_last_error": (ctypes.c_char_p, []),
+    "cerb_decode": (_i, [_vpp, _ip, _i, _i, _i, _ip, _ip, _fp, _i, _vpp, _vpp, _ip, _vp]),
+    "cerb_decode_split": (_i, [_vpp, _vpp, _ip, _i, _i, _i, _ip, _ip, _fp, _i, _vpp, _vpp, _ip, _vp]),
+    "cerb_head_tail": (_i, [_vpp] * 6 + [_ip, _ip, _ip, _i, _i, _i, _ip, _ip, _fp, _i, _vpp, _vpp, _ip, _vp]),
+    "cerb_summary_row_len": (_sz, [_i, _i]),
+    "cerb_nms_workspace_bytes": (_sz, [_i, _i, _i]),
+    "cerb_nms": (_i, _NMS + [_vp]),
+    "cerb_nms_stats": (_i, _NMS + [_vp, _vp]),
+    "cerb_nms_deliver": (_i, _NMS + [ctypes.POINTER(Delivery), _vp]),
+    "cerb_deliver_collect": (_i, [_vp, _vpp, _vp, _i, _i, _vp]),
+    "cerb_deliver_push": (_i, [_vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp]),
+    "cerb_decode_nms": (_i, [_vpp, _ip, _i, _i, _i, _ip, _ip, _fp, _i, _vpp, _vpp, _d, _d, _ip, _i, _i, _i, _i, _i, _d, _vp, _vp, _vp, _sz, _vp]),
+    "cerb_cross_task": (_i, [_vp, _vp, _i, _i, _i, _ip, _d, _vp, _vp, _vp, _vp]),
+    "cerb_cross_task_workspace_bytes": (_sz, [_i, _i, _i]),
+    "cerb_cross_task_ws": (_i, [_vp, _vp, _i, _i, _i, _ip, _d, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "cerb_val_match": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _fp, _i, _vp, _vp]),
+    "cerb_bbox_decode_fwd": (_i, [_vp, _vp, _lg, _i, _i, _i, _vp, _vp]),
+    "cerb_bbox_decode_bwd": (_i, [_vp, _vp, _lg, _i, _i, _vp, _vp]),
+    "cerb_tal_workspace_bytes": (_sz, [_i, _i, _i, _i]),
+    "cerb_tal_assign": (_i, [_vp] * 6 + [_i] * 5 + [_d, _d, _d, _i] + [_vp] * 6 + [_sz, _vp]),
+    "cerb_bbox_loss_workspace_bytes": (_sz, [_i, _i]),
+    "cerb_bbox_loss_fwd": (_i, [_vp] * 7 + [_d] + [_i] * 5 + [_vp] * 4 + [_sz, _vp]),
+    "cerb_bbox_loss_bwd": (_i, [_vp] * 7 + [_d] + [_i] * 5 + [_vp] * 5),
+    "cerb_ap_workspace_bytes": (_sz, [_lg, _i, _i]),
+    "cerb_ap_per_class": (_i, [_vp, _i, _vp, _vp, _lg, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "cerb_debug_set": (_i, [ctypes.c_char_p, _i]),
+    "cerb_debug_reset": (_i, []),
+    "cerb_debug_set_chunking": (_i, [_i, _i]),
+    "cerb_debug_set_hist_sample": (_i, [_i]),
+}
+EXPORTS = tuple(PROTOTYPES)
 
 
 class CerbLibraryError(RuntimeError):
@@ -73,78 +80,11 @@ def load() -> ctypes.CDLL:
             "(or __graft_entry__.build()).  cerberusdet_b200 has no CPU fallback."
         )
     lib = ctypes.CDLL(LIB_PATH)
-    vp, ip, i, d, sz = ctypes.c_void_p, ctypes.POINTER(ctypes.c_int), ctypes.c_int, ctypes.c_double, ctypes.c_size_t
-    vpp = ctypes.POINTER(ctypes.c_void_p)
-    fp = ctypes.POINTER(ctypes.c_float)
-    lib.cerb_version.restype = i
-    lib.cerb_version.argtypes = []
-    lib.cerb_last_error.restype = ctypes.c_char_p
-    lib.cerb_last_error.argtypes = []
-    lib.cerb_decode.restype = i
-    lib.cerb_decode.argtypes = [vpp, ip, i, i, i, ip, ip, fp, i, vpp, vpp, ip, vp]
-    lib.cerb_decode_split.restype = i
-    lib.cerb_decode_split.argtypes = [vpp, vpp, ip, i, i, i, ip, ip, fp, i, vpp, vpp, ip, vp]
-    if hasattr(lib, "cerb_head_tail") or "CERB_LIB" not in os.environ:
-        lib.cerb_head_tail.restype = i
-        lib.cerb_head_tail.argtypes = [vpp] * 6 + [ip, ip, ip, i, i, i, ip, ip, fp, i, vpp, vpp, ip, vp]
-    lib.cerb_summary_row_len.restype = sz
-    lib.cerb_summary_row_len.argtypes = [i, i]
-    lib.cerb_nms_workspace_bytes.restype = sz
-    lib.cerb_nms_workspace_bytes.argtypes = [i, i, i]
-    lib.cerb_nms.restype = i
-    lib.cerb_nms.argtypes = [vpp, ip, i, i, i, i, d, d, ip, i, i, i, i, i, d, vpp, vp, vp, vp, sz, vp]
-    if hasattr(lib, "cerb_nms_stats") or "CERB_LIB" not in os.environ:
-        lib.cerb_nms_stats.restype = i
-        lib.cerb_nms_stats.argtypes = [vpp, ip, i, i, i, i, d, d, ip, i, i, i, i, i, d, vpp, vp, vp, vp, sz, vp, vp]
-    if hasattr(lib, "cerb_nms_deliver") or "CERB_LIB" not in os.environ:
-        lib.cerb_nms_deliver.restype = i
-        lib.cerb_nms_deliver.argtypes = [vpp, ip, i, i, i, i, d, d, ip, i, i, i, i, i, d, vpp, vp, vp, vp, sz, ctypes.POINTER(Delivery), vp]
-        lib.cerb_deliver_collect.restype = i
-        lib.cerb_deliver_collect.argtypes = [vp, vpp, vp, i, i, vp]
-        lib.cerb_deliver_push.restype = i
-        lib.cerb_deliver_push.argtypes = [vp, vp, sz, vp, vp, vp, vp, vp]
-    lib.cerb_decode_nms.restype = i
-    lib.cerb_decode_nms.argtypes = [vpp, ip, i, i, i, ip, ip, fp, i, vpp, vpp, d, d, ip, i, i, i, i, i, d, vp, vp, vp, sz, vp]
-    lib.cerb_cross_task.restype = i
-    lib.cerb_cross_task.argtypes = [vp, vp, i, i, i, ip, d, vp, vp, vp, vp]
-    if hasattr(lib, "cerb_cross_task_ws") or "CERB_LIB" not in os.environ:
-        lib.cerb_cross_task_workspace_bytes.restype = sz
-        lib.cerb_cross_task_workspace_bytes.argtypes = [i, i, i]
-        lib.cerb_cross_task_ws.restype = i
-        lib.cerb_cross_task_ws.argtypes = [vp, vp, i, i, i, ip, d, vp, vp, vp, vp, sz, vp]
-    lib.cerb_val_match.restype = i
-    lib.cerb_val_match.argtypes = [vp, vp, i, i, vp, vp, i, fp, i, vp, vp]
-    lg = ctypes.c_long
-    lib.cerb_bbox_decode_fwd.restype = i
-    lib.cerb_bbox_decode_fwd.argtypes = [vp, vp, lg, i, i, i, vp, vp]
-    lib.cerb_bbox_decode_bwd.restype = i
-    lib.cerb_bbox_decode_bwd.argtypes = [vp, vp, lg, i, i, vp, vp]
-    if hasattr(lib, "cerb_tal_assign") or "CERB_LIB" not in os.environ:
-        lib.cerb_tal_workspace_bytes.restype = sz
-        lib.cerb_tal_workspace_bytes.argtypes = [i, i, i, i]
-        lib.cerb_tal_assign.restype = i
-        lib.cerb_tal_assign.argtypes = [vp] * 6 + [i] * 5 + [d, d, d, i] + [vp] * 6 + [sz, vp]
-    if hasattr(lib, "cerb_bbox_loss_fwd") or "CERB_LIB" not in os.environ:
-        lib.cerb_bbox_loss_workspace_bytes.restype = sz
-        lib.cerb_bbox_loss_workspace_bytes.argtypes = [i, i]
-        lib.cerb_bbox_loss_fwd.restype = i
-        lib.cerb_bbox_loss_fwd.argtypes = [vp] * 7 + [d] + [i] * 5 + [vp] * 4 + [sz, vp]
-        lib.cerb_bbox_loss_bwd.restype = i
-        lib.cerb_bbox_loss_bwd.argtypes = [vp] * 7 + [d] + [i] * 5 + [vp] * 5
-    if hasattr(lib, "cerb_ap_per_class") or "CERB_LIB" not in os.environ:
-        lib.cerb_ap_workspace_bytes.restype = sz
-        lib.cerb_ap_workspace_bytes.argtypes = [lg, i, i]
-        lib.cerb_ap_per_class.restype = i
-        lib.cerb_ap_per_class.argtypes = [vp, i, vp, vp, lg, vp, vp, i, d, vp, vp, vp, vp, sz, vp]
-    if hasattr(lib, "cerb_debug_set") or "CERB_LIB" not in os.environ:  # (tools/ A/B runs may load an older build)
-        lib.cerb_debug_set.restype = i
-        lib.cerb_debug_set.argtypes = [ctypes.c_char_p, i]
-        lib.cerb_debug_reset.restype = i
-        lib.cerb_debug_reset.argtypes = []
-    lib.cerb_debug_set_chunking.restype = i
-    lib.cerb_debug_set_chunking.argtypes = [i, i]
-    lib.cerb_debug_set_hist_sample.restype = i
-    lib.cerb_debug_set_hist_sample.argtypes = [i]
+    for name, (restype, argtypes) in PROTOTYPES.items():
+        if "CERB_LIB" in os.environ and not hasattr(lib, name):
+            continue  # an older build (tools/ A/B runs): a call to the missing entry point fails where it is made
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = lib
     return lib
 

@@ -401,14 +401,6 @@ bool ap_layout(long n, int K, int nc, ApLayout& L) {
     return true;
 }
 
-#define AP_REQUIRE(cond, ...)            \
-    do {                                 \
-        if (!(cond)) {                   \
-            cerb_set_error(__VA_ARGS__); \
-            return CERB_EINVAL;          \
-        }                                \
-    } while (0)
-
 #define AP_CUDA(call)                                                                        \
     do {                                                                                     \
         const cudaError_t e_ = (call);                                                       \
@@ -429,16 +421,16 @@ extern "C" size_t cerb_ap_workspace_bytes(long n, int K, int nc) {
 extern "C" int cerb_ap_per_class(const unsigned char* tp, int K, const float* conf, const float* pred_cls, long n,
                                  const float* classes, const long long* n_labels, int nc, double eps, double* ap, double* p,
                                  double* r, void* workspace, size_t workspace_bytes, void* stream) {
-    cerb_set_error("%s", "");
-    AP_REQUIRE(n >= 0 && n <= 0x7fffffffL, "cerb_ap_per_class: n=%ld detections, 0 <= n < 2^31 required", n);
-    AP_REQUIRE(K >= 1 && K <= 32, "cerb_ap_per_class: K=%d IoU thresholds, 1..32 supported", K);
-    AP_REQUIRE(nc >= 0, "cerb_ap_per_class: nc=%d", nc);
-    AP_REQUIRE(n == 0 || (tp && conf && pred_cls), "cerb_ap_per_class: null argument (tp, conf, pred_cls)");
-    AP_REQUIRE(nc == 0 || (classes && n_labels && ap && p && r), "cerb_ap_per_class: null argument (classes, n_labels, ap, p, r)");
+    cerb_clear_error();
+    CERB_REQUIRE(n >= 0 && n <= 0x7fffffffL, "cerb_ap_per_class: n=%ld detections, 0 <= n < 2^31 required", n);
+    CERB_REQUIRE(K >= 1 && K <= 32, "cerb_ap_per_class: K=%d IoU thresholds, 1..32 supported", K);
+    CERB_REQUIRE(nc >= 0, "cerb_ap_per_class: nc=%d", nc);
+    CERB_REQUIRE(n == 0 || (tp && conf && pred_cls), "cerb_ap_per_class: null argument (tp, conf, pred_cls)");
+    CERB_REQUIRE(nc == 0 || (classes && n_labels && ap && p && r), "cerb_ap_per_class: null argument (classes, n_labels, ap, p, r)");
     for (int c = 0; c < nc; ++c) {
-        AP_REQUIRE(c == 0 || classes[c - 1] < classes[c], "cerb_ap_per_class: classes must be strictly ascending (and not NaN) at %d", c);
-        AP_REQUIRE(classes[c] == classes[c], "cerb_ap_per_class: classes[%d] is NaN", c);
-        AP_REQUIRE(n_labels[c] >= 0, "cerb_ap_per_class: n_labels[%d] < 0", c);
+        CERB_REQUIRE(c == 0 || classes[c - 1] < classes[c], "cerb_ap_per_class: classes must be strictly ascending (and not NaN) at %d", c);
+        CERB_REQUIRE(classes[c] == classes[c], "cerb_ap_per_class: classes[%d] is NaN", c);
+        CERB_REQUIRE(n_labels[c] >= 0, "cerb_ap_per_class: n_labels[%d] < 0", c);
     }
     if (nc == 0) return 0;
     cudaStream_t s = (cudaStream_t)stream;
@@ -453,11 +445,8 @@ extern "C" int cerb_ap_per_class(const unsigned char* tp, int K, const float* co
         cerb_set_error("cerb_ap_per_class: cannot size the radix sort (no CUDA device?)");
         return CERB_ECUDA;
     }
-    if (workspace == nullptr || workspace_bytes < L.total) {
-        cerb_set_error("cerb_ap_per_class: workspace of %zu bytes required, got %zu", L.total, workspace_bytes);
-        return CERB_ENOSPC;
-    }
-    AP_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "cerb_ap_per_class: workspace must be 256-byte aligned");
+    if (const int rc = cerb_require_workspace("cerb_ap_per_class", workspace, workspace_bytes, L.total)) return rc;
+    CERB_REQUIRE(cerb_aligned(workspace, 256), "cerb_ap_per_class: workspace must be 256-byte aligned");
     char* ws = (char*)workspace;
     float* classes_d = (float*)(ws + L.classes);
     long long* n_labels_d = (long long*)(ws + L.n_labels);

@@ -77,21 +77,25 @@ void cerb_set_error(const char* fmt, ...) {
     va_end(ap);
 }
 
-#define REQUIRE(cond, ...)            \
-    do {                              \
-        if (!(cond)) {                \
-            cerb_set_error(__VA_ARGS__); \
-            return CERB_EINVAL;       \
-        }                             \
-    } while (0)
+void cerb_clear_error() { g_err[0] = 0; }
 
-static bool aligned_to(const void* p, size_t a) { return (reinterpret_cast<uintptr_t>(p) % a) == 0; }
+int cerb_launch_status(const char* fn, cudaError_t e) {
+    if (e == cudaSuccess) return 0;
+    cerb_set_error("%s: launch failed: %s", fn, cudaGetErrorString(e));
+    return CERB_ECUDA;
+}
+
+int cerb_require_workspace(const char* fn, const void* ws, size_t have, size_t need) {
+    if (need == 0 || (ws != nullptr && have >= need)) return 0;
+    cerb_set_error("%s: workspace of %zu bytes required, got %zu", fn, need, have);
+    return CERB_ENOSPC;
+}
 
 extern "C" int cerb_version(void) { return 100; }
 extern "C" const char* cerb_last_error(void) { return g_err; }
 
 extern "C" int cerb_debug_set(const char* name, int value) {
-    REQUIRE(name != nullptr, "cerb_debug_set: null knob name");
+    CERB_REQUIRE(name != nullptr, "cerb_debug_set: null knob name");
     for (int i = 0; i < K_COUNT; ++i)
         if (strcmp(name, kKnobName[i]) == 0) {
             g_knobs.v[i] = value;
@@ -108,15 +112,15 @@ extern "C" int cerb_debug_reset(void) {
 
 extern "C" int cerb_debug_set_chunking(int chunk_cap, int chunk_first) {
     if (chunk_cap == 0 && chunk_first == 0) { g_knobs.set[K_CHUNK_CAP] = g_knobs.set[K_CHUNK_FIRST] = false; return 0; }
-    REQUIRE(chunk_cap >= 16 && chunk_cap <= 4096, "chunk_cap must be in [16, 4096], got %d", chunk_cap);
-    REQUIRE(chunk_first >= 1, "chunk_first must be >= 1, got %d", chunk_first);
+    CERB_REQUIRE(chunk_cap >= 16 && chunk_cap <= 4096, "chunk_cap must be in [16, 4096], got %d", chunk_cap);
+    CERB_REQUIRE(chunk_first >= 1, "chunk_first must be >= 1, got %d", chunk_first);
     g_knobs.v[K_CHUNK_CAP] = chunk_cap; g_knobs.set[K_CHUNK_CAP] = true;
     g_knobs.v[K_CHUNK_FIRST] = chunk_first; g_knobs.set[K_CHUNK_FIRST] = true;
     return 0;
 }
 
 extern "C" int cerb_debug_set_hist_sample(int stride) {
-    REQUIRE(stride >= 0 && stride <= 64, "hist sample stride must be in [0, 64], got %d", stride);
+    CERB_REQUIRE(stride >= 0 && stride <= 64, "hist sample stride must be in [0, 64], got %d", stride);
     g_knobs.v[K_HIST_SAMPLE] = stride;
     g_knobs.set[K_HIST_SAMPLE] = stride != 0;
     return 0;
@@ -131,12 +135,12 @@ extern "C" size_t cerb_summary_row_len(int A, int dtype) {
 static int decode_common(const void* const* lvl, const void* const* cls_lvl, const int* nc, int T, int L, int B,
                          const int* H, const int* W, const float* strides, int dtype, void* const* y, void* const* smax,
                          int* summary_written, void* stream) {
-    g_err[0] = 0;
-    REQUIRE(lvl && nc && H && W && strides && y, "cerb_decode: null argument");
-    REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_decode: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
-    REQUIRE(L >= 1 && L <= CERB_MAX_LEVELS, "cerb_decode: L=%d outside [1, %d]", L, CERB_MAX_LEVELS);
-    REQUIRE(B >= 0, "cerb_decode: negative batch");
-    REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_decode: unsupported dtype %d", dtype);
+    cerb_clear_error();
+    CERB_REQUIRE(lvl && nc && H && W && strides && y, "cerb_decode: null argument");
+    CERB_REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_decode: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
+    CERB_REQUIRE(L >= 1 && L <= CERB_MAX_LEVELS, "cerb_decode: L=%d outside [1, %d]", L, CERB_MAX_LEVELS);
+    CERB_REQUIRE(B >= 0, "cerb_decode: negative batch");
+    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_decode: unsupported dtype %d", dtype);
     DecodeParams P;
     memset(&P, 0, sizeof(P));
     P.T = T; P.L = L; P.B = B; P.nrows = T * L;
@@ -147,31 +151,31 @@ static int decode_common(const void* const* lvl, const void* const* cls_lvl, con
     long A = 0;
     if (summary_written) *summary_written = 0;
     for (int l = 0; l < L; ++l) {
-        REQUIRE(H[l] > 0 && W[l] > 0, "cerb_decode: level %d has empty shape %dx%d", l, H[l], W[l]);
+        CERB_REQUIRE(H[l] > 0 && W[l] > 0, "cerb_decode: level %d has empty shape %dx%d", l, H[l], W[l]);
         const long hw = (long)H[l] * W[l];
-        REQUIRE(hw < (1l << 30), "cerb_decode: level %d too large", l);
+        CERB_REQUIRE(hw < (1l << 30), "cerb_decode: level %d too large", l);
         P.hw[l] = (int)hw; P.w[l] = W[l]; P.aoff[l] = (int)A; P.stride[l] = strides[l];
         A += hw;
         while (vec > 1 && hw % vec) vec >>= 1;
     }
-    REQUIRE(A < (1l << 30), "cerb_decode: too many anchors");
+    CERB_REQUIRE(A < (1l << 30), "cerb_decode: too many anchors");
     P.A = (int)A;
     for (int t = 0; t < T; ++t) {
-        REQUIRE(nc[t] >= 1, "cerb_decode: task %d has nc=%d", t, nc[t]);
+        CERB_REQUIRE(nc[t] >= 1, "cerb_decode: task %d has nc=%d", t, nc[t]);
         P.nc[t] = nc[t];
-        REQUIRE(y[t] != nullptr || B == 0, "cerb_decode: y[%d] is null", t);
+        CERB_REQUIRE(y[t] != nullptr || B == 0, "cerb_decode: y[%d] is null", t);
         P.y[t] = y[t];
-        while (vec > 1 && !aligned_to(y[t], vec * elt)) vec >>= 1;
+        while (vec > 1 && !cerb_aligned(y[t], vec * elt)) vec >>= 1;
         for (int l = 0; l < L; ++l) {
             const void* p = lvl[t * L + l];
-            REQUIRE(p != nullptr || B == 0, "cerb_decode: lvl[%d][%d] is null", t, l);
+            CERB_REQUIRE(p != nullptr || B == 0, "cerb_decode: lvl[%d][%d] is null", t, l);
             P.lvl[t][l] = p;
-            while (vec > 1 && !aligned_to(p, vec * elt)) vec >>= 1;
+            while (vec > 1 && !cerb_aligned(p, vec * elt)) vec >>= 1;
             if (cls_lvl != nullptr) {
                 const void* c = cls_lvl[t * L + l];
-                REQUIRE(c != nullptr || B == 0, "cerb_decode_split: cls_lvl[%d][%d] is null", t, l);
+                CERB_REQUIRE(c != nullptr || B == 0, "cerb_decode_split: cls_lvl[%d][%d] is null", t, l);
                 P.cls[t][l] = c;
-                while (vec > 1 && !aligned_to(c, vec * elt)) vec >>= 1;
+                while (vec > 1 && !cerb_aligned(c, vec * elt)) vec >>= 1;
             }
         }
     }
@@ -180,7 +184,7 @@ static int decode_common(const void* const* lvl, const void* const* cls_lvl, con
     // the score summary (one maximum per 16-byte score vector) needs the full 128-bit path
     if (smax != nullptr && vec == (int)(16 / elt)) {
         bool all = true;
-        for (int t = 0; t < T; ++t) all = all && smax[t] != nullptr && aligned_to(smax[t], 16);
+        for (int t = 0; t < T; ++t) all = all && smax[t] != nullptr && cerb_aligned(smax[t], 16);
         if (all) {
             for (int t = 0; t < T; ++t) P.smax[t] = smax[t];
             if (summary_written) *summary_written = 1;
@@ -212,11 +216,7 @@ static int decode_common(const void* const* lvl, const void* const* cls_lvl, con
         (void)cudaGetLastError();
         e = cerb_launch_decode(P, dtype, vec, (cudaStream_t)stream);
     }
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_decode: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    return cerb_launch_status("cerb_decode", e);
 }
 
 extern "C" int cerb_decode(const void* const* lvl, const int* nc, int T, int L, int B, const int* H, const int* W,
@@ -228,10 +228,7 @@ extern "C" int cerb_decode(const void* const* lvl, const int* nc, int T, int L, 
 extern "C" int cerb_decode_split(const void* const* box_lvl, const void* const* cls_lvl, const int* nc, int T, int L, int B,
                                  const int* H, const int* W, const float* strides, int dtype, void* const* y,
                                  void* const* smax, int* summary_written, void* stream) {
-    if (cls_lvl == nullptr) {
-        cerb_set_error("cerb_decode_split: null argument");
-        return CERB_EINVAL;
-    }
+    CERB_REQUIRE(cls_lvl != nullptr, "cerb_decode_split: null argument");
     return decode_common(box_lvl, cls_lvl, nc, T, L, B, H, W, strides, dtype, y, smax, summary_written, stream);
 }
 
@@ -279,22 +276,22 @@ extern "C" int cerb_nms_deliver(const void* const* pred, const int* nc, int T, i
                                 double iou_thres, const int* classes, int n_classes, int agnostic, int multi_label,
                                 int max_det, int max_nms, double max_wh, const void* const* smax, float* dets, int* counts,
                                 void* workspace, size_t workspace_bytes, const cerb_delivery* dv, void* stream) {
-    REQUIRE(dv != nullptr, "cerb_nms_deliver: null delivery");
+    CERB_REQUIRE(dv != nullptr, "cerb_nms_deliver: null delivery");
     if (dv->flag_remote != nullptr) {
-        REQUIRE(dv->ack_local && dv->seq_local && dv->done_local, "cerb_nms_deliver: null protocol word");
-        REQUIRE(aligned_to(dv->flag_remote, 4) && aligned_to(dv->ack_local, 4) && aligned_to(dv->seq_local, 4) && aligned_to(dv->done_local, 4),
-                "cerb_nms_deliver: protocol words must be 4-byte aligned");
+        CERB_REQUIRE(dv->ack_local && dv->seq_local && dv->done_local, "cerb_nms_deliver: null protocol word");
+        CERB_REQUIRE(cerb_aligned(dv->flag_remote, 4) && cerb_aligned(dv->ack_local, 4) && cerb_aligned(dv->seq_local, 4) && cerb_aligned(dv->done_local, 4),
+                     "cerb_nms_deliver: protocol words must be 4-byte aligned");
     }
     if (dv->push_src != nullptr) {
-        REQUIRE(dv->flag_remote != nullptr && dv->push_dst != nullptr, "cerb_nms_deliver: push_src needs push_dst and the protocol words");
-        REQUIRE(aligned_to(dv->push_src, 16) && aligned_to(dv->push_dst, 16) && dv->push_words % 4 == 0 && dv->push_words < (1ull << 32),
-                "cerb_nms_deliver: push buffers must be 16-byte aligned and hold a multiple of 4 words");
+        CERB_REQUIRE(dv->flag_remote != nullptr && dv->push_dst != nullptr, "cerb_nms_deliver: push_src needs push_dst and the protocol words");
+        CERB_REQUIRE(cerb_aligned(dv->push_src, 16) && cerb_aligned(dv->push_dst, 16) && dv->push_words % 4 == 0 && dv->push_words < (1ull << 32),
+                     "cerb_nms_deliver: push buffers must be 16-byte aligned and hold a multiple of 4 words");
     }
     if (dv->collect_flags != nullptr) {
-        REQUIRE(dv->collect_count != nullptr && dv->world >= 1 && dv->world <= 16 && dv->dst >= 0 && dv->dst < dv->world,
-                "cerb_nms_deliver: bad collect side (world=%d dst=%d)", dv->world, dv->dst);
+        CERB_REQUIRE(dv->collect_count != nullptr && dv->world >= 1 && dv->world <= 16 && dv->dst >= 0 && dv->dst < dv->world,
+                     "cerb_nms_deliver: bad collect side (world=%d dst=%d)", dv->world, dv->dst);
         for (int r = 0; r < dv->world; ++r)
-            REQUIRE(r == dv->dst || dv->collect_ack[r] != nullptr, "cerb_nms_deliver: collect_ack[%d] is null", r);
+            CERB_REQUIRE(r == dv->dst || dv->collect_ack[r] != nullptr, "cerb_nms_deliver: collect_ack[%d] is null", r);
     }
     return nms_impl(pred, nc, T, B, A, dtype, conf_thres, iou_thres, classes, n_classes, agnostic, multi_label, max_det, max_nms,
                     max_wh, smax, dets, counts, workspace, workspace_bytes, nullptr, dv, stream);
@@ -302,10 +299,10 @@ extern "C" int cerb_nms_deliver(const void* const* pred, const int* nc, int T, i
 
 extern "C" int cerb_deliver_push(const void* src_local, void* dst_remote, size_t n_words, void* flag_remote, const void* ack_local,
                                  void* seq_local, void* done_local, void* stream) {
-    g_err[0] = 0;
-    REQUIRE(src_local && dst_remote && flag_remote && ack_local && seq_local && done_local, "cerb_deliver_push: null argument");
-    REQUIRE(aligned_to(src_local, 16) && aligned_to(dst_remote, 16) && n_words % 4 == 0,
-            "cerb_deliver_push: buffers must be 16-byte aligned and hold a multiple of 4 words");
+    cerb_clear_error();
+    CERB_REQUIRE(src_local && dst_remote && flag_remote && ack_local && seq_local && done_local, "cerb_deliver_push: null argument");
+    CERB_REQUIRE(cerb_aligned(src_local, 16) && cerb_aligned(dst_remote, 16) && n_words % 4 == 0,
+                 "cerb_deliver_push: buffers must be 16-byte aligned and hold a multiple of 4 words");
     PushParams P;
     P.src = (const float*)src_local;
     P.dst = (float*)dst_remote;
@@ -322,19 +319,14 @@ extern "C" int cerb_deliver_push(const void* src_local, void* dst_remote, size_t
     int kv = 0;
     if (knob(K_PUSH_CTAS, &kv) && kv >= 1 && kv <= 1024) ctas = (size_t)kv;
     P.mode = knob(K_PUSH_MODE, &kv) ? kv : 0;
-    cudaError_t e = cerb_launch_deliver_push(P, (int)ctas, (cudaStream_t)stream);
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_deliver_push: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    return cerb_launch_status("cerb_deliver_push", cerb_launch_deliver_push(P, (int)ctas, (cudaStream_t)stream));
 }
 
 extern "C" int cerb_deliver_collect(const void* flags_local, void* const* ack_remote, void* collected_local, int world, int dst,
                                     void* stream) {
-    g_err[0] = 0;
-    REQUIRE(flags_local && ack_remote && collected_local, "cerb_deliver_collect: null argument");
-    REQUIRE(world >= 1 && world <= CERB_MAX_RANKS && dst >= 0 && dst < world, "cerb_deliver_collect: world=%d dst=%d (at most %d ranks)", world, dst, CERB_MAX_RANKS);
+    cerb_clear_error();
+    CERB_REQUIRE(flags_local && ack_remote && collected_local, "cerb_deliver_collect: null argument");
+    CERB_REQUIRE(world >= 1 && world <= CERB_MAX_RANKS && dst >= 0 && dst < world, "cerb_deliver_collect: world=%d dst=%d (at most %d ranks)", world, dst, CERB_MAX_RANKS);
     CollectParams P;
     memset(&P, 0, sizeof(P));
     P.flags = (const unsigned*)flags_local;
@@ -342,39 +334,34 @@ extern "C" int cerb_deliver_collect(const void* flags_local, void* const* ack_re
     P.world = world;
     P.dst = dst;
     for (int r = 0; r < world; ++r) {
-        REQUIRE(r == dst || ack_remote[r] != nullptr, "cerb_deliver_collect: ack_remote[%d] is null", r);
+        CERB_REQUIRE(r == dst || ack_remote[r] != nullptr, "cerb_deliver_collect: ack_remote[%d] is null", r);
         P.ack[r] = (unsigned*)ack_remote[r];
     }
-    cudaError_t e = cerb_launch_deliver_collect(P, (cudaStream_t)stream);
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_deliver_collect: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    return cerb_launch_status("cerb_deliver_collect", cerb_launch_deliver_collect(P, (cudaStream_t)stream));
 }
 
 static int nms_impl(const void* const* pred, const int* nc, int T, int B, int A, int dtype, double conf_thres, double iou_thres,
                     const int* classes, int n_classes, int agnostic, int multi_label, int max_det, int max_nms, double max_wh,
                     const void* const* smax, float* dets, int* counts, void* workspace, size_t workspace_bytes,
                     unsigned long long* stats, const cerb_delivery* dv, void* stream) {
-    g_err[0] = 0;
-    REQUIRE(pred && nc, "cerb_nms: null argument");
-    REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_nms: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
-    REQUIRE(B >= 0 && A >= 0, "cerb_nms: negative size");
-    REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_nms: unsupported dtype %d", dtype);
-    REQUIRE(conf_thres >= 0.0 && conf_thres <= 1.0, "Invalid Confidence threshold %g, valid values are between 0.0 and 1.0", conf_thres);
-    REQUIRE(iou_thres >= 0.0 && iou_thres <= 1.0, "Invalid IoU %g, valid values are between 0.0 and 1.0", iou_thres);
-    REQUIRE(max_det >= 0 && max_nms >= 0, "cerb_nms: negative max_det/max_nms");
+    cerb_clear_error();
+    CERB_REQUIRE(pred && nc, "cerb_nms: null argument");
+    CERB_REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_nms: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
+    CERB_REQUIRE(B >= 0 && A >= 0, "cerb_nms: negative size");
+    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_nms: unsupported dtype %d", dtype);
+    CERB_REQUIRE(conf_thres >= 0.0 && conf_thres <= 1.0, "Invalid Confidence threshold %g, valid values are between 0.0 and 1.0", conf_thres);
+    CERB_REQUIRE(iou_thres >= 0.0 && iou_thres <= 1.0, "Invalid IoU %g, valid values are between 0.0 and 1.0", iou_thres);
+    CERB_REQUIRE(max_det >= 0 && max_nms >= 0, "cerb_nms: negative max_det/max_nms");
     if (B == 0) return 0;
-    REQUIRE(counts != nullptr, "cerb_nms: counts is null");
-    REQUIRE(dets != nullptr || max_det == 0, "cerb_nms: dets is null");
+    CERB_REQUIRE(counts != nullptr, "cerb_nms: counts is null");
+    CERB_REQUIRE(dets != nullptr || max_det == 0, "cerb_nms: dets is null");
     NmsParams P;
     memset(&P, 0, sizeof(P));
     P.T = T; P.B = B; P.A = A;
     for (int t = 0; t < T; ++t) {
-        REQUIRE(nc[t] >= 1, "cerb_nms: task %d has nc=%d", t, nc[t]);
-        REQUIRE((double)A * nc[t] < 4294967295.0, "cerb_nms: A*nc overflows the 32-bit candidate index");
-        REQUIRE(pred[t] != nullptr || A == 0, "cerb_nms: pred[%d] is null", t);
+        CERB_REQUIRE(nc[t] >= 1, "cerb_nms: task %d has nc=%d", t, nc[t]);
+        CERB_REQUIRE((double)A * nc[t] < 4294967295.0, "cerb_nms: A*nc overflows the 32-bit candidate index");
+        CERB_REQUIRE(pred[t] != nullptr || A == 0, "cerb_nms: pred[%d] is null", t);
         P.pred[t] = pred[t];
         P.nc[t] = nc[t];
     }
@@ -386,14 +373,14 @@ static int nms_impl(const void* const* pred, const int* nc, int T, int B, int A,
             P.class_mask[c >> 5] |= 1u << (c & 31);
         }
         for (int t = 0; t < T; ++t)
-            REQUIRE(nc[t] <= 32 * CERB_MAX_CLASS_WORDS, "cerb_nms: class filter supports nc <= %d", 32 * CERB_MAX_CLASS_WORDS);
+            CERB_REQUIRE(nc[t] <= 32 * CERB_MAX_CLASS_WORDS, "cerb_nms: class filter supports nc <= %d", 32 * CERB_MAX_CLASS_WORDS);
     }
     if (smax != nullptr) {
         const int V = dtype == CERB_F16 ? 8 : 4;
-        REQUIRE(A % V == 0, "cerb_nms: a score summary needs A (%d) to be a multiple of %d", A, V);
+        CERB_REQUIRE(A % V == 0, "cerb_nms: a score summary needs A (%d) to be a multiple of %d", A, V);
         for (int t = 0; t < T; ++t) {
-            REQUIRE(smax[t] != nullptr && aligned_to(smax[t], 16), "cerb_nms: smax[%d] is null or misaligned", t);
-            REQUIRE(aligned_to(pred[t], 16), "cerb_nms: summary path needs 16-byte aligned predictions");
+            CERB_REQUIRE(smax[t] != nullptr && cerb_aligned(smax[t], 16), "cerb_nms: smax[%d] is null or misaligned", t);
+            CERB_REQUIRE(cerb_aligned(pred[t], 16), "cerb_nms: summary path needs 16-byte aligned predictions");
             P.smax[t] = smax[t];
         }
     }
@@ -429,12 +416,9 @@ static int nms_impl(const void* const* pred, const int* nc, int T, int B, int A,
         }
     }
     const size_t need = cerb_nms_kept_ws_bytes(T, B, max_det);
+    if (const int rc = cerb_require_workspace("cerb_nms", workspace, workspace_bytes, need)) return rc;
     if (need) {
-        if (workspace == nullptr || workspace_bytes < need) {
-            cerb_set_error("cerb_nms: workspace of %zu bytes required, got %zu", need, workspace_bytes);
-            return CERB_ENOSPC;
-        }
-        REQUIRE(aligned_to(workspace, 16), "cerb_nms: workspace must be 16-byte aligned");
+        CERB_REQUIRE(cerb_aligned(workspace, 16), "cerb_nms: workspace must be 16-byte aligned");
         P.kept_ws = (float*)workspace;
     }
     P.chunk_cap = 4096;
@@ -464,12 +448,7 @@ static int nms_impl(const void* const* pred, const int* nc, int T, int B, int A,
             P.tame_hi = (float)(lo + gap);
         }
     }
-    cudaError_t e = cerb_launch_nms(P, dtype, (cudaStream_t)stream);
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_nms: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    return cerb_launch_status("cerb_nms", cerb_launch_nms(P, dtype, (cudaStream_t)stream));
 }
 
 extern "C" size_t cerb_cross_task_workspace_bytes(int T, int B, int max_det) {
@@ -480,19 +459,19 @@ extern "C" size_t cerb_cross_task_workspace_bytes(int T, int B, int max_det) {
 extern "C" int cerb_cross_task_ws(const float* dets, const int* counts, int T, int B, int max_det, const int* class_offset,
                                   double iou_thres, const float* scale, float* out, int* out_counts, void* workspace,
                                   size_t workspace_bytes, void* stream) {
-    g_err[0] = 0;
-    REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_cross_task: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
-    REQUIRE(B >= 0 && max_det >= 0, "cerb_cross_task: negative size");
-    REQUIRE(max_det <= 65535, "cerb_cross_task: max_det=%d exceeds 65535", max_det);
+    cerb_clear_error();
+    CERB_REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_cross_task: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
+    CERB_REQUIRE(B >= 0 && max_det >= 0, "cerb_cross_task: negative size");
+    CERB_REQUIRE(max_det <= 65535, "cerb_cross_task: max_det=%d exceeds 65535", max_det);
     if (B == 0) return 0;
-    REQUIRE(counts && class_offset && out_counts && (dets || max_det == 0) && (out || max_det == 0), "cerb_cross_task: null argument");
+    CERB_REQUIRE(counts && class_offset && out_counts && (dets || max_det == 0) && (out || max_det == 0), "cerb_cross_task: null argument");
     const size_t need = cerb_cross_task_ws_bytes(T, B, max_det);
     if (need && (workspace == nullptr || workspace_bytes < need)) {
         cerb_set_error("cerb_cross_task: T*max_det=%ld rows per image need a workspace of %zu bytes, got %zu", (long)T * max_det, need,
                        workspace ? workspace_bytes : (size_t)0);
         return CERB_ENOSPC;
     }
-    REQUIRE(!need || aligned_to(workspace, 16), "cerb_cross_task: workspace must be 16-byte aligned");
+    CERB_REQUIRE(!need || cerb_aligned(workspace, 16), "cerb_cross_task: workspace must be 16-byte aligned");
     CrossTaskParams P;
     memset(&P, 0, sizeof(P));
     P.dets = dets; P.counts = counts; P.T = T; P.B = B; P.max_det = max_det;
@@ -500,12 +479,7 @@ extern "C" int cerb_cross_task_ws(const float* dets, const int* counts, int T, i
     P.iou_thr = (float)iou_thres;
     P.scale = scale; P.out = out; P.out_counts = out_counts;
     P.workspace = need ? (unsigned char*)workspace : nullptr;
-    cudaError_t e = cerb_launch_cross_task(P, (cudaStream_t)stream);
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_cross_task: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    return cerb_launch_status("cerb_cross_task", cerb_launch_cross_task(P, (cudaStream_t)stream));
 }
 
 extern "C" int cerb_cross_task(const float* dets, const int* counts, int T, int B, int max_det, const int* class_offset,
@@ -531,55 +505,42 @@ extern "C" int cerb_decode_nms(const void* const* lvl, const int* nc, int T, int
 extern "C" int cerb_val_match(const float* dets, const int* counts, int B, int max_det, const float* labels,
                               const int* label_offsets, int max_labels_per_image, const float* iouv, int K,
                               unsigned char* correct, void* stream) {
-    g_err[0] = 0;
-    REQUIRE(B >= 0 && max_det >= 0, "cerb_val_match: negative size");
-    REQUIRE(K >= 1 && K <= 16, "cerb_val_match: K=%d thresholds outside [1, 16]", K);
-    REQUIRE(max_labels_per_image >= 0 && max_labels_per_image <= 1024, "cerb_val_match: more than 1024 labels per image (%d)", max_labels_per_image);
+    cerb_clear_error();
+    CERB_REQUIRE(B >= 0 && max_det >= 0, "cerb_val_match: negative size");
+    CERB_REQUIRE(K >= 1 && K <= 16, "cerb_val_match: K=%d thresholds outside [1, 16]", K);
+    CERB_REQUIRE(max_labels_per_image >= 0 && max_labels_per_image <= 1024, "cerb_val_match: more than 1024 labels per image (%d)", max_labels_per_image);
     if (B == 0 || max_det == 0) return 0;
-    REQUIRE(dets && counts && label_offsets && iouv && correct, "cerb_val_match: null argument");
+    CERB_REQUIRE(dets && counts && label_offsets && iouv && correct, "cerb_val_match: null argument");
     ValMatchParams P;
     memset(&P, 0, sizeof(P));
     P.dets = dets; P.counts = counts; P.labels = labels; P.label_offsets = label_offsets;
     P.B = B; P.max_det = max_det; P.K = K; P.correct = correct;
     for (int i = 0; i < K; ++i) P.iouv[i] = iouv[i];
-    cudaError_t e = cerb_launch_val_match(P, max_labels_per_image, (cudaStream_t)stream);
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_val_match: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    return cerb_launch_status("cerb_val_match", cerb_launch_val_match(P, max_labels_per_image, (cudaStream_t)stream));
 }
 
 // ------------------------------------------------------------------ training-time sibling decode (SURVEY 8f-4)
 extern "C" int cerb_bbox_decode_fwd(const void* pred_dist, const void* anchor_points, long n_rows, int A, int reg_max,
                                     int dtype, void* out, void* stream) {
-    g_err[0] = 0;
-    REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_bbox_decode_fwd: unsupported dtype %d", dtype);
-    REQUIRE(reg_max == CERB_REG_MAX, "cerb_bbox_decode_fwd: reg_max=%d, only %d is supported (models/yolo.py:75)", reg_max, CERB_REG_MAX);
-    REQUIRE(n_rows >= 0 && n_rows < (1l << 40) && A >= 0, "cerb_bbox_decode_fwd: bad sizes n_rows=%ld A=%d", n_rows, A);
+    cerb_clear_error();
+    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_bbox_decode_fwd: unsupported dtype %d", dtype);
+    CERB_REQUIRE(reg_max == CERB_REG_MAX, "cerb_bbox_decode_fwd: reg_max=%d, only %d is supported (models/yolo.py:75)", reg_max, CERB_REG_MAX);
+    CERB_REQUIRE(n_rows >= 0 && n_rows < (1l << 40) && A >= 0, "cerb_bbox_decode_fwd: bad sizes n_rows=%ld A=%d", n_rows, A);
     if (n_rows == 0) return 0;
-    REQUIRE(A >= 1 && n_rows % A == 0, "cerb_bbox_decode_fwd: n_rows=%ld is not a multiple of A=%d", n_rows, A);
-    REQUIRE(pred_dist && anchor_points && out, "cerb_bbox_decode_fwd: null argument");
-    cudaError_t e = cerb_launch_bbox_decode_fwd(pred_dist, anchor_points, n_rows, A, dtype, out, (cudaStream_t)stream);
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_bbox_decode_fwd: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    CERB_REQUIRE(A >= 1 && n_rows % A == 0, "cerb_bbox_decode_fwd: n_rows=%ld is not a multiple of A=%d", n_rows, A);
+    CERB_REQUIRE(pred_dist && anchor_points && out, "cerb_bbox_decode_fwd: null argument");
+    return cerb_launch_status("cerb_bbox_decode_fwd",
+                              cerb_launch_bbox_decode_fwd(pred_dist, anchor_points, n_rows, A, dtype, out, (cudaStream_t)stream));
 }
 
 extern "C" int cerb_bbox_decode_bwd(const void* pred_dist, const void* grad_out, long n_rows, int reg_max, int dtype,
                                     void* grad_pred_dist, void* stream) {
-    g_err[0] = 0;
-    REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_bbox_decode_bwd: unsupported dtype %d", dtype);
-    REQUIRE(reg_max == CERB_REG_MAX, "cerb_bbox_decode_bwd: reg_max=%d, only %d is supported (models/yolo.py:75)", reg_max, CERB_REG_MAX);
-    REQUIRE(n_rows >= 0 && n_rows < (1l << 40), "cerb_bbox_decode_bwd: bad n_rows=%ld", n_rows);
+    cerb_clear_error();
+    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_bbox_decode_bwd: unsupported dtype %d", dtype);
+    CERB_REQUIRE(reg_max == CERB_REG_MAX, "cerb_bbox_decode_bwd: reg_max=%d, only %d is supported (models/yolo.py:75)", reg_max, CERB_REG_MAX);
+    CERB_REQUIRE(n_rows >= 0 && n_rows < (1l << 40), "cerb_bbox_decode_bwd: bad n_rows=%ld", n_rows);
     if (n_rows == 0) return 0;
-    REQUIRE(pred_dist && grad_out && grad_pred_dist, "cerb_bbox_decode_bwd: null argument");
-    cudaError_t e = cerb_launch_bbox_decode_bwd(pred_dist, grad_out, n_rows, dtype, grad_pred_dist, (cudaStream_t)stream);
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_bbox_decode_bwd: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    CERB_REQUIRE(pred_dist && grad_out && grad_pred_dist, "cerb_bbox_decode_bwd: null argument");
+    return cerb_launch_status("cerb_bbox_decode_bwd",
+                              cerb_launch_bbox_decode_bwd(pred_dist, grad_out, n_rows, dtype, grad_pred_dist, (cudaStream_t)stream));
 }

@@ -327,30 +327,20 @@ extern "C" size_t cerb_bbox_loss_workspace_bytes(int B, int A) {
     return 16 + (size_t)fwd_ctas((long)B * A) * sizeof(float2);
 }
 
-#define BL_REQUIRE(cond, ...)            \
-    do {                                 \
-        if (!(cond)) {                   \
-            cerb_set_error(__VA_ARGS__); \
-            return CERB_EINVAL;          \
-        }                                \
-    } while (0)
-
-static bool bl_aligned(const void* p, size_t a) { return (reinterpret_cast<uintptr_t>(p) % a) == 0; }
-
 static int bl_params(const char* fn, const void* pred_dist, const void* pred_bboxes, const void* anchor_points,
                      const float* target_bboxes, const float* target_scores, const unsigned char* fg_mask,
                      const float* tss_dev, double tss_host, int B, int A, int C, int reg_max, int dtype, BboxLossParams& P) {
-    cerb_set_error("%s", "");
-    BL_REQUIRE(reg_max == CERB_REG_MAX, "%s: reg_max=%d bins, only %d is supported (loss.py:96, BboxLoss(m.reg_max - 1))", fn, reg_max, CERB_REG_MAX);
-    BL_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "%s: unsupported dtype %d", fn, dtype);
-    BL_REQUIRE(B >= 0 && A >= 0 && C >= 1, "%s: bad sizes B=%d A=%d C=%d", fn, B, A, C);
-    BL_REQUIRE((long long)B * A <= 0x7fffffffLL && (long long)B * A * C <= (1LL << 40), "%s: B*A overflows (B=%d A=%d C=%d)", fn, B, A, C);
+    cerb_clear_error();
+    CERB_REQUIRE(reg_max == CERB_REG_MAX, "%s: reg_max=%d bins, only %d is supported (loss.py:96, BboxLoss(m.reg_max - 1))", fn, reg_max, CERB_REG_MAX);
+    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "%s: unsupported dtype %d", fn, dtype);
+    CERB_REQUIRE(B >= 0 && A >= 0 && C >= 1, "%s: bad sizes B=%d A=%d C=%d", fn, B, A, C);
+    CERB_REQUIRE((long long)B * A <= 0x7fffffffLL && (long long)B * A * C <= (1LL << 40), "%s: B*A overflows (B=%d A=%d C=%d)", fn, B, A, C);
     if ((long long)B * A > 0) {
-        BL_REQUIRE(pred_dist && pred_bboxes && anchor_points && target_bboxes && target_scores && fg_mask, "%s: null argument", fn);
+        CERB_REQUIRE(pred_dist && pred_bboxes && anchor_points && target_bboxes && target_scores && fg_mask, "%s: null argument", fn);
         const size_t e = dtype == CERB_F16 ? 2 : 4;
-        BL_REQUIRE(bl_aligned(pred_dist, 32) && bl_aligned(pred_bboxes, 4 * e) && bl_aligned(anchor_points, e) &&
-                       bl_aligned(target_bboxes, 16) && bl_aligned(target_scores, 4),
-                   "%s: misaligned rows (pred_dist needs 32 bytes, box rows 4 elements)", fn);
+        CERB_REQUIRE(cerb_aligned(pred_dist, 32) && cerb_aligned(pred_bboxes, 4 * e) && cerb_aligned(anchor_points, e) &&
+                         cerb_aligned(target_bboxes, 16) && cerb_aligned(target_scores, 4),
+                     "%s: misaligned rows (pred_dist needs 32 bytes, box rows 4 elements)", fn);
     }
     P.pred_dist = pred_dist; P.pred_bboxes = pred_bboxes; P.anchor_points = anchor_points;
     P.target_bboxes = target_bboxes; P.target_scores = target_scores; P.fg_mask = fg_mask;
@@ -367,14 +357,11 @@ extern "C" int cerb_bbox_loss_fwd(const void* pred_dist, const void* pred_bboxes
     const int rc = bl_params("cerb_bbox_loss_fwd", pred_dist, pred_bboxes, anchor_points, target_bboxes, target_scores, fg_mask,
                              target_scores_sum, target_scores_sum_host, B, A, C, reg_max, dtype, P);
     if (rc) return rc;
-    BL_REQUIRE(loss_iou && loss_dfl, "cerb_bbox_loss_fwd: null argument");
-    BL_REQUIRE(per_anchor == nullptr || bl_aligned(per_anchor, 8), "cerb_bbox_loss_fwd: per_anchor must be 8-byte aligned");
+    CERB_REQUIRE(loss_iou && loss_dfl, "cerb_bbox_loss_fwd: null argument");
+    CERB_REQUIRE(per_anchor == nullptr || cerb_aligned(per_anchor, 8), "cerb_bbox_loss_fwd: per_anchor must be 8-byte aligned");
     const size_t need = cerb_bbox_loss_workspace_bytes(B, A);
-    if (workspace == nullptr || workspace_bytes < need) {
-        cerb_set_error("cerb_bbox_loss_fwd: workspace of %zu bytes required, got %zu", need, workspace_bytes);
-        return CERB_ENOSPC;
-    }
-    BL_REQUIRE(bl_aligned(workspace, 16), "cerb_bbox_loss_fwd: workspace must be 16-byte aligned");
+    if (const int ws_rc = cerb_require_workspace("cerb_bbox_loss_fwd", workspace, workspace_bytes, need)) return ws_rc;
+    CERB_REQUIRE(cerb_aligned(workspace, 16), "cerb_bbox_loss_fwd: workspace must be 16-byte aligned");
     unsigned* ticket = (unsigned*)workspace;
     float2* partials = (float2*)((char*)workspace + 16);
     const unsigned ctas = fwd_ctas(P.n_rows);
@@ -382,12 +369,7 @@ extern "C" int cerb_bbox_loss_fwd(const void* pred_dist, const void* pred_bboxes
         bbox_loss_fwd_kernel<__half><<<ctas, BL_THREADS, 0, (cudaStream_t)stream>>>(P, loss_iou, loss_dfl, per_anchor, partials, ticket);
     else
         bbox_loss_fwd_kernel<float><<<ctas, BL_THREADS, 0, (cudaStream_t)stream>>>(P, loss_iou, loss_dfl, per_anchor, partials, ticket);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_bbox_loss_fwd: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    return cerb_launch_status("cerb_bbox_loss_fwd", cudaGetLastError());
 }
 
 extern "C" int cerb_bbox_loss_bwd(const void* pred_dist, const void* pred_bboxes, const void* anchor_points, const float* target_bboxes,
@@ -399,18 +381,13 @@ extern "C" int cerb_bbox_loss_bwd(const void* pred_dist, const void* pred_bboxes
                              target_scores_sum, target_scores_sum_host, B, A, C, reg_max, dtype, P);
     if (rc) return rc;
     if (P.n_rows == 0) return 0;
-    BL_REQUIRE(grad_iou && grad_dfl && grad_pred_dist && grad_pred_bboxes, "cerb_bbox_loss_bwd: null argument");
-    BL_REQUIRE(bl_aligned(grad_pred_dist, 32) && bl_aligned(grad_pred_bboxes, dtype == CERB_F16 ? 8 : 16),
-               "cerb_bbox_loss_bwd: misaligned rows (grad_pred_dist needs 32 bytes, box rows 4 elements)");
+    CERB_REQUIRE(grad_iou && grad_dfl && grad_pred_dist && grad_pred_bboxes, "cerb_bbox_loss_bwd: null argument");
+    CERB_REQUIRE(cerb_aligned(grad_pred_dist, 32) && cerb_aligned(grad_pred_bboxes, dtype == CERB_F16 ? 8 : 16),
+                 "cerb_bbox_loss_bwd: misaligned rows (grad_pred_dist needs 32 bytes, box rows 4 elements)");
     const unsigned blocks = (unsigned)((P.n_rows * 4 + BL_THREADS - 1) / BL_THREADS);
     if (dtype == CERB_F16)
         bbox_loss_bwd_kernel<__half><<<blocks, BL_THREADS, 0, (cudaStream_t)stream>>>(P, grad_iou, grad_dfl, (__half*)grad_pred_dist, (__half*)grad_pred_bboxes);
     else
         bbox_loss_bwd_kernel<float><<<blocks, BL_THREADS, 0, (cudaStream_t)stream>>>(P, grad_iou, grad_dfl, (float*)grad_pred_dist, (float*)grad_pred_bboxes);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_bbox_loss_bwd: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    return cerb_launch_status("cerb_bbox_loss_bwd", cudaGetLastError());
 }

@@ -233,6 +233,20 @@ __device__ __forceinline__ void stg_stream16(void* p, uint4 v) {
 #endif
 }
 
-// host-side error plumbing (api.cu)
+// host-side error plumbing of the C ABI (api.cu): the message cerb_last_error() returns is thread-local
 void cerb_set_error(const char* fmt, ...);
+void cerb_clear_error();
+// 0, or CERB_ECUDA with "<fn>: launch failed: <msg>"
+int cerb_launch_status(const char* fn, cudaError_t e);
+// 0 when the call needs no workspace or gets enough, else CERB_ENOSPC with "<fn>: workspace of N bytes required, got M"
+int cerb_require_workspace(const char* fn, const void* ws, size_t have, size_t need);
+inline bool cerb_aligned(const void* p, size_t bytes) { return reinterpret_cast<uintptr_t>(p) % bytes == 0; }
+// argument check of an entry point: on failure set the message and return CERB_EINVAL
+#define CERB_REQUIRE(cond, ...)          \
+    do {                                 \
+        if (!(cond)) {                   \
+            cerb_set_error(__VA_ARGS__); \
+            return CERB_EINVAL;          \
+        }                                \
+    } while (0)
 bool cerb_debug_knob(const char* name, int* out);  // thread-local / environment test knob, false when unset

@@ -425,41 +425,33 @@ static int ht_stage_rows(int c) {
     return 0;
 }
 
-#define HT_REQUIRE(cond, ...)            \
-    do {                                 \
-        if (!(cond)) {                   \
-            cerb_set_error(__VA_ARGS__); \
-            return CERB_EINVAL;          \
-        }                                \
-    } while (0)
-
 extern "C" int cerb_head_tail(const void* const* box_feat, const void* const* cls_feat, const void* const* box_w,
                               const void* const* box_b, const void* const* cls_w, const void* const* cls_b, const int* c2,
                               const int* c3, const int* nc, int T, int L, int B, const int* H, const int* W,
                               const float* strides, int dtype, void* const* y, void* const* smax, int* summary_written,
                               void* stream) {
-    cerb_set_error("%s", "");
-    HT_REQUIRE(box_feat && cls_feat && box_w && box_b && cls_w && cls_b && c2 && c3 && nc && H && W && strides && y,
-               "cerb_head_tail: null argument");
-    HT_REQUIRE(dtype == CERB_F16, "cerb_head_tail: fp16 only (tcgen05 kind::f16); run the convolutions and cerb_decode for fp32");
-    HT_REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_head_tail: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
-    HT_REQUIRE(L >= 1 && L <= CERB_MAX_LEVELS, "cerb_head_tail: L=%d outside [1, %d]", L, CERB_MAX_LEVELS);
-    HT_REQUIRE(B >= 1, "cerb_head_tail: B=%d", B);
-    HT_REQUIRE(ht_encoder() != nullptr, "cerb_head_tail: cuTensorMapEncodeTiled is not available in this driver");
+    cerb_clear_error();
+    CERB_REQUIRE(box_feat && cls_feat && box_w && box_b && cls_w && cls_b && c2 && c3 && nc && H && W && strides && y,
+                 "cerb_head_tail: null argument");
+    CERB_REQUIRE(dtype == CERB_F16, "cerb_head_tail: fp16 only (tcgen05 kind::f16); run the convolutions and cerb_decode for fp32");
+    CERB_REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_head_tail: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
+    CERB_REQUIRE(L >= 1 && L <= CERB_MAX_LEVELS, "cerb_head_tail: L=%d outside [1, %d]", L, CERB_MAX_LEVELS);
+    CERB_REQUIRE(B >= 1, "cerb_head_tail: B=%d", B);
+    CERB_REQUIRE(ht_encoder() != nullptr, "cerb_head_tail: cuTensorMapEncodeTiled is not available in this driver");
     int A = 0, aoff[CERB_MAX_LEVELS];
     for (int l = 0; l < L; ++l) {
-        HT_REQUIRE(H[l] >= 1 && W[l] >= 1, "cerb_head_tail: level %d is %dx%d", l, H[l], W[l]);
-        HT_REQUIRE((H[l] * W[l]) % 8 == 0, "cerb_head_tail: H*W of level %d (%d) must be a multiple of 8 (16-byte rows for TMA)", l, H[l] * W[l]);
+        CERB_REQUIRE(H[l] >= 1 && W[l] >= 1, "cerb_head_tail: level %d is %dx%d", l, H[l], W[l]);
+        CERB_REQUIRE((H[l] * W[l]) % 8 == 0, "cerb_head_tail: H*W of level %d (%d) must be a multiple of 8 (16-byte rows for TMA)", l, H[l] * W[l]);
         aoff[l] = A;
         A += H[l] * W[l];
     }
     int max_ncp = 0;
     for (int t = 0; t < T; ++t) {
-        HT_REQUIRE(nc[t] >= 1 && ((nc[t] + 15) & ~15) <= HT_MAX_NCP, "cerb_head_tail: nc[%d]=%d outside [1, %d]", t, nc[t], HT_MAX_NCP);
-        HT_REQUIRE(c2[t] >= 16 && c2[t] % 16 == 0 && c3[t] >= 16 && c3[t] % 16 == 0,
-                   "cerb_head_tail: c2[%d]=%d / c3[%d]=%d must be multiples of 16", t, c2[t], t, c3[t]);
-        HT_REQUIRE((size_t)B * c2[t] < (1ull << 31) && (size_t)B * c3[t] < (1ull << 31), "cerb_head_tail: B * channels too large");
-        HT_REQUIRE(y[t] != nullptr, "cerb_head_tail: y[%d] is null", t);
+        CERB_REQUIRE(nc[t] >= 1 && ((nc[t] + 15) & ~15) <= HT_MAX_NCP, "cerb_head_tail: nc[%d]=%d outside [1, %d]", t, nc[t], HT_MAX_NCP);
+        CERB_REQUIRE(c2[t] >= 16 && c2[t] % 16 == 0 && c3[t] >= 16 && c3[t] % 16 == 0,
+                     "cerb_head_tail: c2[%d]=%d / c3[%d]=%d must be multiples of 16", t, c2[t], t, c3[t]);
+        CERB_REQUIRE((size_t)B * c2[t] < (1ull << 31) && (size_t)B * c3[t] < (1ull << 31), "cerb_head_tail: B * channels too large");
+        CERB_REQUIRE(y[t] != nullptr, "cerb_head_tail: y[%d] is null", t);
         max_ncp = max(max_ncp, (nc[t] + 15) & ~15);
     }
     bool want_summary = smax != nullptr;
@@ -482,9 +474,10 @@ extern "C" int cerb_head_tail(const void* const* box_feat, const void* const* cl
             for (int l = 0; l < L; ++l, ++r) {
                 HtRow& R = P.row[r];
                 const int i = t * L + l, hw = H[l] * W[l];
-                HT_REQUIRE(box_feat[i] && cls_feat[i] && box_w[i] && box_b[i] && cls_w[i] && cls_b[i], "cerb_head_tail: null tensor (task %d, level %d)", t, l);
-                HT_REQUIRE(((uintptr_t)box_feat[i] | (uintptr_t)cls_feat[i] | (uintptr_t)box_w[i] | (uintptr_t)cls_w[i]) % 16 == 0,
-                           "cerb_head_tail: tensors must be 16-byte aligned (task %d, level %d)", t, l);
+                CERB_REQUIRE(box_feat[i] && cls_feat[i] && box_w[i] && box_b[i] && cls_w[i] && cls_b[i], "cerb_head_tail: null tensor (task %d, level %d)", t, l);
+                CERB_REQUIRE(cerb_aligned(box_feat[i], 16) && cerb_aligned(cls_feat[i], 16) && cerb_aligned(box_w[i], 16) &&
+                                 cerb_aligned(cls_w[i], 16),
+                             "cerb_head_tail: tensors must be 16-byte aligned (task %d, level %d)", t, l);
                 R.b2 = (const __half*)box_b[i];
                 R.b3 = (const __half*)cls_b[i];
                 R.y = (__half*)y[t];
@@ -546,10 +539,7 @@ extern "C" int cerb_head_tail(const void* const* box_feat, const void* const* cl
             head_tail_kernel<<<min(tiles, sms), 64 + 32 * HT_EPI_WARPS * P.ngroups, smem, (cudaStream_t)stream>>>(P);
             e = cudaGetLastError();
         }
-        if (e != cudaSuccess) {
-            cerb_set_error("cerb_head_tail: launch failed: %s", cudaGetErrorString(e));
-            return CERB_ECUDA;
-        }
+        if (const int rc = cerb_launch_status("cerb_head_tail", e)) return rc;
     }
     return 0;
 }

@@ -266,28 +266,18 @@ extern "C" int cerb_tal_assign(const void* pd_scores, const float* pd_bboxes, co
                                double beta, double eps, int score_dtype, long long* target_labels, float* target_bboxes,
                                float* target_scores, unsigned char* fg_mask, long long* target_gt_idx, void* workspace,
                                size_t workspace_bytes, void* stream) {
-    cerb_set_error("%s", "");
-#define TAL_REQUIRE(cond, ...)           \
-    do {                                 \
-        if (!(cond)) {                   \
-            cerb_set_error(__VA_ARGS__); \
-            return CERB_EINVAL;          \
-        }                                \
-    } while (0)
-    TAL_REQUIRE(pd_scores && pd_bboxes && anc_points && gt_labels && gt_bboxes && mask_gt && target_labels && target_bboxes &&
-                    target_scores && fg_mask && target_gt_idx,
-                "cerb_tal_assign: null argument");
-    TAL_REQUIRE(B >= 1 && A >= 1 && C >= 1, "cerb_tal_assign: empty problem (B=%d A=%d C=%d)", B, A, C);
-    TAL_REQUIRE(G >= 1 && G <= TAL_MAX_GT, "cerb_tal_assign: G=%d outside [1, %d] (no boxes at all is the caller's early return, tal.py:89-93)", G, TAL_MAX_GT);
-    TAL_REQUIRE(topk >= 1 && topk <= TAL_MAX_TOPK && topk <= A, "cerb_tal_assign: topk=%d outside [1, min(%d, A)]", topk, TAL_MAX_TOPK);
-    TAL_REQUIRE(score_dtype == CERB_F16 || score_dtype == CERB_F32, "cerb_tal_assign: unsupported score dtype %d", score_dtype);
-    TAL_REQUIRE(((uintptr_t)pd_bboxes | (uintptr_t)gt_bboxes | (uintptr_t)target_bboxes) % 16 == 0 && (uintptr_t)anc_points % 8 == 0,
-                "cerb_tal_assign: box tensors must be 16-byte aligned, anchor points 8-byte aligned");
+    cerb_clear_error();
+    CERB_REQUIRE(pd_scores && pd_bboxes && anc_points && gt_labels && gt_bboxes && mask_gt && target_labels && target_bboxes &&
+                     target_scores && fg_mask && target_gt_idx,
+                 "cerb_tal_assign: null argument");
+    CERB_REQUIRE(B >= 1 && A >= 1 && C >= 1, "cerb_tal_assign: empty problem (B=%d A=%d C=%d)", B, A, C);
+    CERB_REQUIRE(G >= 1 && G <= TAL_MAX_GT, "cerb_tal_assign: G=%d outside [1, %d] (no boxes at all is the caller's early return, tal.py:89-93)", G, TAL_MAX_GT);
+    CERB_REQUIRE(topk >= 1 && topk <= TAL_MAX_TOPK && topk <= A, "cerb_tal_assign: topk=%d outside [1, min(%d, A)]", topk, TAL_MAX_TOPK);
+    CERB_REQUIRE(score_dtype == CERB_F16 || score_dtype == CERB_F32, "cerb_tal_assign: unsupported score dtype %d", score_dtype);
+    CERB_REQUIRE(cerb_aligned(pd_bboxes, 16) && cerb_aligned(gt_bboxes, 16) && cerb_aligned(target_bboxes, 16) && cerb_aligned(anc_points, 8),
+                 "cerb_tal_assign: box tensors must be 16-byte aligned, anchor points 8-byte aligned");
     const size_t need = cerb_tal_workspace_bytes_impl(B, A, G, topk);
-    if (workspace == nullptr || workspace_bytes < need) {
-        cerb_set_error("cerb_tal_assign: workspace of %zu bytes required, got %zu", need, workspace_bytes);
-        return CERB_ENOSPC;
-    }
+    if (const int rc = cerb_require_workspace("cerb_tal_assign", workspace, workspace_bytes, need)) return rc;
     TalParams P;
     P.scores = pd_scores; P.pd = pd_bboxes; P.anc = anc_points; P.gt_labels = gt_labels; P.gt_boxes = gt_bboxes; P.mask_gt = mask_gt;
     P.B = B; P.A = A; P.C = C; P.G = G; P.topk = topk; P.score_half = score_dtype == CERB_F16;
@@ -305,10 +295,5 @@ extern "C" int cerb_tal_assign(const void* pd_scores, const float* pd_bboxes, co
     const size_t n_out = (size_t)B * A * C;
     const int blocks = (int)((n_out + 255) / 256 < 148 * 16 ? (n_out + 255) / 256 : 148 * 16);
     tal_scores_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(P);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        cerb_set_error("cerb_tal_assign: launch failed: %s", cudaGetErrorString(e));
-        return CERB_ECUDA;
-    }
-    return 0;
+    return cerb_launch_status("cerb_tal_assign", cudaGetLastError());
 }

@@ -33,8 +33,17 @@ def _require_cuda(t: torch.Tensor, what: str) -> None:
         raise TypeError(f"{what} must be a CUDA tensor (cerberusdet_b200 has no CPU path), got device {t.device}")
 
 
-def _stream_ptr(device) -> int:
-    return torch.cuda.current_stream(device).cuda_stream
+def _launch(fn, device, *args) -> None:
+    """Call the C entry point ``fn(*args, stream)`` on ``device``'s current stream, under that device's guard; a non-zero
+    return code raises (``_lib.check``)."""
+    with torch.cuda.device(device):
+        _lib.check(fn(*args, torch.cuda.current_stream(device).cuda_stream))
+
+
+def _workspace(nbytes: int, device) -> torch.Tensor:
+    """Uninitialised device workspace for one call.  A 0-byte one has a null ``data_ptr()``, which the C ABI accepts from a
+    call that needs no workspace."""
+    return torch.empty((int(nbytes),), dtype=torch.uint8, device=device)
 
 
 def _dense16(x: torch.Tensor) -> torch.Tensor:
@@ -43,22 +52,22 @@ def _dense16(x: torch.Tensor) -> torch.Tensor:
     return x if x.data_ptr() % 16 == 0 else x.clone(memory_format=torch.contiguous_format)
 
 
-def _summary_len(level_sizes: Sequence[int], elt: int) -> int:
-    """Row length of the score summary (``cerb_summary_row_len``), or 0 when a level rules the 128-bit path out."""
+def _decode_shapes(B, nc: Sequence[int], level_sizes: Sequence, elt: int) -> list:
+    """Shapes of the decode outputs ``[y_0 .. y_{T-1}, smax_0 .. smax_{T-1}]``: ``y_t [B, 4+nc_t, A]`` and the score
+    summary ``smax_t [B, nc_t, R]``.  The summary exists exactly when every level allows 16-byte vectors (inputs and
+    outputs are 16-byte aligned by construction), so R (``cerb_summary_row_len``, 0 without a summary) is a function of
+    the shapes alone -- the fake kernels rely on that."""
     V = 16 // elt
-    if any(n % V for n in level_sizes):
-        return 0
-    n = sum(level_sizes) // V
-    return (n + V - 1) // V * V
+    A = sum(level_sizes)
+    R = 0 if any(n % V for n in level_sizes) else (A // V + V - 1) // V * V
+    return [(B, 4 + n, A) for n in nc] + [(B, n, R) for n in nc]
 
 
-def _decode_impl(levels: Sequence[torch.Tensor], nc: Sequence[int], strides: Sequence[float],
-                 cls_levels: Optional[Sequence[torch.Tensor]] = None,
-                 out: Optional[Sequence[torch.Tensor]] = None) -> List[torch.Tensor]:
-    """Returns ``[y_0 .. y_{T-1}, smax_0 .. smax_{T-1}]``; the score summaries ``smax_t`` are empty
-    tensors when the shapes do not allow them (see include/cerb_post.h).  With ``cls_levels`` the heads are split:
-    ``levels`` hold the 64 box channels, ``cls_levels`` the class channels (``cerb_decode_split``)."""
-    lib = _lib.load()
+def _dense_heads(levels: Sequence[torch.Tensor], nc: Sequence[int], strides: Sequence[float],
+                 cls_levels: Optional[Sequence[torch.Tensor]] = None):
+    """Check ``T*L`` raw head tensors (task-major) and return ``(code, B, H, W, lv, cl)``: the dtype code, the shapes and
+    the dense, 16-byte aligned tensors.  With ``cls_levels`` the heads are split: ``levels`` hold the 64 box channels,
+    ``cls_levels`` the class channels.  A device or dtype mismatch raises ``TypeError``, a shape mismatch ``ValueError``."""
     T = len(nc)
     if T == 0 or len(levels) % T:
         raise ValueError("levels must hold T*L tensors, task-major")
@@ -70,60 +79,62 @@ def _decode_impl(levels: Sequence[torch.Tensor], nc: Sequence[int], strides: Seq
     first = levels[0]
     _require_cuda(first, "head tensors")
     code = _dtype_code(first)
-    B = first.shape[0]
+    B = int(first.shape[0])
     H = [int(levels[l].shape[2]) for l in range(L)]
     W = [int(levels[l].shape[3]) for l in range(L)]
-    A = sum(h * w for h, w in zip(H, W))
-    lv = []
-    for t in range(T):
-        for l in range(L):
-            x = levels[t * L + l]
-            if x.device != first.device or x.dtype != first.dtype:
-                raise TypeError("all head tensors must share device and dtype")
-            cbox = 64 if cls_levels is not None else 64 + nc[t]
-            if tuple(x.shape) != (B, cbox, H[l], W[l]):
-                raise ValueError(f"task {t} level {l}: expected {(B, cbox, H[l], W[l])}, got {tuple(x.shape)}")
-            lv.append(_dense16(x))
-    cl = []
-    if cls_levels is not None:
+
+    def dense(tensors, channels, what):
+        out = []
         for t in range(T):
             for l in range(L):
-                c = cls_levels[t * L + l]
-                if c.device != first.device or c.dtype != first.dtype:
+                x, shape = tensors[t * L + l], (B, channels[t], H[l], W[l])
+                if x.device != first.device or x.dtype != first.dtype:
                     raise TypeError("all head tensors must share device and dtype")
-                if tuple(c.shape) != (B, nc[t], H[l], W[l]):
-                    raise ValueError(f"task {t} level {l}: expected class tensor {(B, nc[t], H[l], W[l])}, got {tuple(c.shape)}")
-                cl.append(_dense16(c))
-    # the score summary exists exactly when every level allows 16-byte vectors (inputs and outputs here are 16-byte
-    # aligned by construction), so its shape is a function of the shapes alone -- the fake kernel below relies on that
-    R = _summary_len([h * w for h, w in zip(H, W)], first.element_size())
+                if tuple(x.shape) != shape:
+                    raise ValueError(f"task {t} level {l}: expected {what}{shape}, got {tuple(x.shape)}")
+                out.append(_dense16(x))
+        return out
+
+    if cls_levels is None:
+        return code, B, H, W, dense(levels, [64 + n for n in nc], ""), []
+    return code, B, H, W, dense(levels, [64] * T, ""), dense(cls_levels, list(nc), "class tensor ")
+
+
+def _decode_impl(levels: Sequence[torch.Tensor], nc: Sequence[int], strides: Sequence[float],
+                 cls_levels: Optional[Sequence[torch.Tensor]] = None,
+                 out: Optional[Sequence[torch.Tensor]] = None) -> List[torch.Tensor]:
+    """Returns ``[y_0 .. y_{T-1}, smax_0 .. smax_{T-1}]``; the score summaries ``smax_t`` are empty
+    tensors when the shapes do not allow them (see include/cerb_post.h).  With ``cls_levels`` the heads are split:
+    ``levels`` hold the 64 box channels, ``cls_levels`` the class channels (``cerb_decode_split``)."""
+    lib = _lib.load()
+    code, B, H, W, lv, cl = _dense_heads(levels, nc, strides, cls_levels)
+    first, T, L = levels[0], len(nc), len(H)
+    shapes = _decode_shapes(B, nc, [h * w for h, w in zip(H, W)], first.element_size())
+    A, R = shapes[0][2], shapes[-1][2]
     assert R == 0 or R == int(lib.cerb_summary_row_len(A, code))
     if out is None:
-        ys = [torch.empty((B, 4 + nc[t], A), dtype=first.dtype, device=first.device) for t in range(T)]
-        sm = [torch.empty((B, nc[t], R), dtype=first.dtype, device=first.device) for t in range(T)]
+        out = [first.new_empty(s) for s in shapes]
     else:  # caller-provided static buffers [y_0 .. y_{T-1}, smax_0 .. smax_{T-1}] (CUDA graphs, pipelines)
         if len(out) != 2 * T:
             raise ValueError("out= must hold T prediction buffers followed by T score-summary buffers")
-        ys, sm = list(out[:T]), list(out[T:])
+        out = list(out)
         for t in range(T):
-            ok = (tuple(ys[t].shape) == (B, 4 + nc[t], A) and tuple(sm[t].shape) == (B, nc[t], R)
-                  and all(z.dtype == first.dtype and z.device == first.device and z.is_contiguous() and z.data_ptr() % 16 == 0
-                          for z in (ys[t], sm[t])))
+            ok = all(tuple(z.shape) == s and z.dtype == first.dtype and z.device == first.device and z.is_contiguous()
+                     and z.data_ptr() % 16 == 0 for z, s in ((out[t], shapes[t]), (out[T + t], shapes[T + t])))
             if not ok:
                 raise ValueError(f"out= buffers of task {t} must be contiguous, 16-byte aligned [B,4+nc,A] / [B,nc,{R}] {first.dtype} tensors")
     written = ctypes.c_int(0)
     tail = (_lib.int_array(list(nc)), T, L, B, _lib.int_array(H), _lib.int_array(W),
-            _lib.float_array([float(s) for s in strides]), code, _lib.ptr_array([y.data_ptr() for y in ys]),
-            _lib.ptr_array([x.data_ptr() for x in sm]), ctypes.byref(written), _stream_ptr(first.device))
-    with torch.cuda.device(first.device):
-        if cls_levels is None:
-            rc = lib.cerb_decode(_lib.ptr_array([x.data_ptr() for x in lv]), *tail)
-        else:
-            rc = lib.cerb_decode_split(_lib.ptr_array([x.data_ptr() for x in lv]), _lib.ptr_array([x.data_ptr() for x in cl]), *tail)
-    _lib.check(rc)
+            _lib.float_array([float(s) for s in strides]), code, _lib.ptr_array([y.data_ptr() for y in out[:T]]),
+            _lib.ptr_array([x.data_ptr() for x in out[T:]]), ctypes.byref(written))
+    lv_ptrs = _lib.ptr_array([x.data_ptr() for x in lv])
+    if cls_levels is None:
+        _launch(lib.cerb_decode, first.device, lv_ptrs, *tail)
+    else:
+        _launch(lib.cerb_decode_split, first.device, lv_ptrs, _lib.ptr_array([x.data_ptr() for x in cl]), *tail)
     if bool(written.value) != (R > 0 and B > 0):
         raise _lib.CerbLibraryError("cerb_decode: score summary state differs from what the shapes imply")
-    return ys + sm
+    return out
 
 
 @torch.library.custom_op("cerb::decode", mutates_args=())
@@ -152,14 +163,9 @@ def decode_split_op(box_levels: Sequence[torch.Tensor], cls_levels: Sequence[tor
 
 
 def _decode_fake(levels, nc, strides):
-    T = len(nc)
-    L = len(levels) // T
-    B = levels[0].shape[0]
+    L = len(levels) // len(nc)
     sizes = [levels[l].shape[2] * levels[l].shape[3] for l in range(L)]
-    A = sum(sizes)
-    R = _summary_len(sizes, levels[0].element_size())
-    return [levels[0].new_empty((B, 4 + nc[t], A)) for t in range(T)] + [
-        levels[0].new_empty((B, nc[t], R)) for t in range(T)]
+    return [levels[0].new_empty(s) for s in _decode_shapes(levels[0].shape[0], nc, sizes, levels[0].element_size())]
 
 
 @decode_op.register_fake
@@ -211,8 +217,7 @@ def _nms_impl(
     else:
         dets = torch.empty((T, B, max_det, 6), dtype=torch.float32, device=dev)  # the kernel writes every row
         counts = torch.empty((T, B), dtype=torch.int32, device=dev)
-    ws_bytes = lib.cerb_nms_workspace_bytes(T, B, max_det)
-    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
+    ws = _workspace(lib.cerb_nms_workspace_bytes(T, B, max_det), dev)
     cls_arr = _lib.int_array(list(classes)) if classes is not None else None
     sm_arr = None
     if len(smax) == T:
@@ -228,15 +233,13 @@ def _nms_impl(
             float(conf_thres), float(iou_thres), cls_arr, len(classes) if classes is not None else 0,
             int(bool(agnostic)), int(bool(multi_label)), int(max_det), int(max_nms), float(max_wh),
             sm_arr,
-            dets.data_ptr(), counts.data_ptr(), ws.data_ptr() if ws is not None else None, ws_bytes)
-    with torch.cuda.device(dev):
-        if deliver is not None:
-            if stats is not None or out is None:
-                raise ValueError("deliver= needs out= (the peer-mapped slot) and excludes stats=")
-            rc = lib.cerb_nms_deliver(*head, ctypes.byref(deliver), _stream_ptr(dev))
-        else:
-            rc = lib.cerb_nms_stats(*head, stats.data_ptr() if stats is not None else None, _stream_ptr(dev))
-    _lib.check(rc)
+            dets.data_ptr(), counts.data_ptr(), ws.data_ptr(), ws.numel())
+    if deliver is not None:
+        if stats is not None or out is None:
+            raise ValueError("deliver= needs out= (the peer-mapped slot) and excludes stats=")
+        _launch(lib.cerb_nms_deliver, dev, *head, ctypes.byref(deliver))
+    else:
+        _launch(lib.cerb_nms_stats, dev, *head, stats.data_ptr() if stats is not None else None)
     return dets, counts
 
 
@@ -343,16 +346,22 @@ def find_summary(y: torch.Tensor):
     return smax
 
 
+def _publish_summaries(ys: Sequence[torch.Tensor], sms: Sequence[torch.Tensor]) -> None:
+    """Remember ``sms[t]``, the score summary decode just wrote for ``ys[t]``, for ``nms_batched`` (where the shapes
+    allowed one)."""
+    for y, sm in zip(ys, sms):
+        if sm.shape[-1]:
+            _remember_summary(y, sm)
+
+
 # ----------------------------------------------------------------------------- friendly wrappers
 def decode_buffers(task_levels: Sequence[Sequence[torch.Tensor]]) -> List[torch.Tensor]:
     """Static output buffers for ``decode_heads(..., out=...)``: ``[y_0 .. y_{T-1}, smax_0 .. smax_{T-1}]``."""
     first = task_levels[0][0]
-    B = int(first.shape[0])
     sizes = [int(x.shape[2]) * int(x.shape[3]) for x in task_levels[0]]
-    A, R = sum(sizes), _summary_len(sizes, first.element_size())
     ncs = [int(lv[0].shape[1]) - 64 for lv in task_levels]
-    return ([torch.empty((B, 4 + n, A), dtype=first.dtype, device=first.device) for n in ncs]
-            + [torch.empty((B, n, R), dtype=first.dtype, device=first.device) for n in ncs])
+    return [torch.empty(s, dtype=first.dtype, device=first.device)
+            for s in _decode_shapes(int(first.shape[0]), ncs, sizes, first.element_size())]
 
 
 def decode_heads(task_levels: Sequence[Sequence[torch.Tensor]], strides: Sequence[float],
@@ -368,11 +377,8 @@ def decode_heads(task_levels: Sequence[Sequence[torch.Tensor]], strides: Sequenc
     else:
         out = decode_op(flat, nc, [float(s) for s in strides])
     T = len(nc)
-    ys, sms = out[:T], out[T:]
-    for y, sm in zip(ys, sms):
-        if sm.shape[-1]:
-            _remember_summary(y, sm)
-    return ys
+    _publish_summaries(out[:T], out[T:])
+    return out[:T]
 
 
 def decode_heads_split(task_box_levels: Sequence[Sequence[torch.Tensor]], task_cls_levels: Sequence[Sequence[torch.Tensor]],
@@ -384,11 +390,8 @@ def decode_heads_split(task_box_levels: Sequence[Sequence[torch.Tensor]], task_c
     out = decode_split_op([x for lv in task_box_levels for x in lv], [x for lv in task_cls_levels for x in lv], nc,
                           [float(s) for s in strides])
     T = len(nc)
-    ys, sms = out[:T], out[T:]
-    for y, sm in zip(ys, sms):
-        if sm.shape[-1]:
-            _remember_summary(y, sm)
-    return ys
+    _publish_summaries(out[:T], out[T:])
+    return out[:T]
 
 
 def _head_tail_impl(box_feats: Sequence[torch.Tensor], cls_feats: Sequence[torch.Tensor], box_w: Sequence[torch.Tensor],
@@ -409,7 +412,6 @@ def _head_tail_impl(box_feats: Sequence[torch.Tensor], cls_feats: Sequence[torch
     B = int(first.shape[0])
     H = [int(box_feats[l].shape[2]) for l in range(L)]
     W = [int(box_feats[l].shape[3]) for l in range(L)]
-    A = sum(h * w for h, w in zip(H, W))
     c2 = [int(box_feats[t * L].shape[1]) for t in range(T)]
     c3 = [int(cls_feats[t * L].shape[1]) for t in range(T)]
     nc = [int(cls_w[t * L].shape[0]) for t in range(T)]
@@ -435,20 +437,16 @@ def _head_tail_impl(box_feats: Sequence[torch.Tensor], cls_feats: Sequence[torch
             ptrs[3].append(dense(box_b[i], (64,), "box bias", t, l))
             ptrs[4].append(dense(cls_w[i], (nc[t], c3[t]), "class weight", t, l))
             ptrs[5].append(dense(cls_b[i], (nc[t],), "class bias", t, l))
-    R = _summary_len([h * w for h, w in zip(H, W)], 2)
-    ys = [torch.empty((B, 4 + nc[t], A), dtype=first.dtype, device=first.device) for t in range(T)]
-    sm = [torch.empty((B, nc[t], R), dtype=first.dtype, device=first.device) for t in range(T)]
+    out = [first.new_empty(s) for s in _decode_shapes(B, nc, [h * w for h, w in zip(H, W)], 2)]
+    R = out[-1].shape[-1]
     written = ctypes.c_int(0)
-    with torch.cuda.device(first.device):
-        rc = lib.cerb_head_tail(*[_lib.ptr_array(p) for p in ptrs], _lib.int_array(c2), _lib.int_array(c3), _lib.int_array(nc),
-                                T, L, B, _lib.int_array(H), _lib.int_array(W), _lib.float_array([float(s) for s in strides]),
-                                _lib.CERB_F16, _lib.ptr_array([y.data_ptr() for y in ys]),
-                                _lib.ptr_array([x.data_ptr() for x in sm]) if R else None, ctypes.byref(written),
-                                _stream_ptr(first.device))
-    _lib.check(rc)
+    _launch(lib.cerb_head_tail, first.device, *[_lib.ptr_array(p) for p in ptrs], _lib.int_array(c2), _lib.int_array(c3),
+            _lib.int_array(nc), T, L, B, _lib.int_array(H), _lib.int_array(W), _lib.float_array([float(s) for s in strides]),
+            _lib.CERB_F16, _lib.ptr_array([y.data_ptr() for y in out[:T]]),
+            _lib.ptr_array([x.data_ptr() for x in out[T:]]) if R else None, ctypes.byref(written))
     for x in keep:  # the kernel is only enqueued: keep temporaries alive on this stream
         x.record_stream(torch.cuda.current_stream(first.device))
-    return ys + sm
+    return out
 
 
 @torch.library.custom_op("cerb::head_tail", mutates_args=())
@@ -463,9 +461,8 @@ def _(box_feats, cls_feats, box_w, box_b, cls_w, cls_b, strides, T):
     L = len(box_feats) // T
     first = box_feats[0]
     sizes = [int(box_feats[l].shape[2]) * int(box_feats[l].shape[3]) for l in range(L)]
-    A, R = sum(sizes), _summary_len(sizes, 2)
     ncs = [int(cls_w[t * L].shape[0]) for t in range(T)]
-    return ([first.new_empty((first.shape[0], 4 + n, A)) for n in ncs] + [first.new_empty((first.shape[0], n, R)) for n in ncs])
+    return [first.new_empty(s) for s in _decode_shapes(first.shape[0], ncs, sizes, 2)]
 
 
 def head_tail(task_box_feats: Sequence[Sequence[torch.Tensor]], task_cls_feats: Sequence[Sequence[torch.Tensor]],
@@ -482,11 +479,23 @@ def head_tail(task_box_feats: Sequence[Sequence[torch.Tensor]], task_cls_feats: 
     T = len(task_box_feats)
     out = head_tail_op(flat(task_box_feats), flat(task_cls_feats), flat(task_box_w), flat(task_box_b), flat(task_cls_w),
                        flat(task_cls_b), [float(s) for s in strides], T)
-    ys, sms = out[:T], out[T:]
-    for y, sm in zip(ys, sms):
-        if sm.shape[-1]:
-            _remember_summary(y, sm)
-    return ys
+    _publish_summaries(out[:T], out[T:])
+    return out[:T]
+
+
+def _nms_params(conf_thres, iou_thres, classes, agnostic, multi_label, max_det, max_nms, max_wh) -> tuple:
+    """The NMS arguments as the ``cerb::nms`` schema takes them, after the reference's asserts (utils/general.py:399-400)
+    -- same exception type and wording."""
+    assert 0 <= conf_thres <= 1, f"Invalid Confidence threshold {conf_thres}, valid values are between 0.0 and 1.0"
+    assert 0 <= iou_thres <= 1, f"Invalid IoU {iou_thres}, valid values are between 0.0 and 1.0"
+    return (float(conf_thres), float(iou_thres), None if classes is None else [int(c) for c in classes], bool(agnostic),
+            bool(multi_label), int(max_det), int(max_nms), float(max_wh))
+
+
+def _summaries(preds: List[torch.Tensor], use_summary: bool) -> List[torch.Tensor]:
+    """The score summaries of ``preds`` when every one still has its summary, else none."""
+    found = [find_summary(p) for p in preds] if use_summary else []
+    return found if all(f is not None for f in found) else []
 
 
 def nms_batched(
@@ -507,17 +516,9 @@ def nms_batched(
     ``counts[T,B]`` (device tensors; no host sync).  Predictions that came out of ``decode_heads``
     unmodified bring their score summary along, which spares the kernel the full score scans.
     ``out=(dets, counts)`` writes into caller-provided buffers (e.g. ``shard.DetectionGatherer``'s)."""
-    # reference asserts (utils/general.py:399-400) -- same exception type and wording
-    assert 0 <= conf_thres <= 1, f"Invalid Confidence threshold {conf_thres}, valid values are between 0.0 and 1.0"
-    assert 0 <= iou_thres <= 1, f"Invalid IoU {iou_thres}, valid values are between 0.0 and 1.0"
+    params = _nms_params(conf_thres, iou_thres, classes, agnostic, multi_label, max_det, max_nms, max_wh)
     preds = list(preds)
-    smax = []
-    if use_summary:
-        found = [find_summary(p) for p in preds]
-        if all(f is not None for f in found):
-            smax = found
-    args = (preds, float(conf_thres), float(iou_thres), None if classes is None else [int(c) for c in classes],
-            bool(agnostic), bool(multi_label), int(max_det), int(max_nms), float(max_wh), smax)
+    args = (preds, *params, _summaries(preds, use_summary))
     if deliver is not None:  # multi-GPU: the launch also runs this rank's part of the delivery to rank dst
         return _nms_impl(*args, out=out, deliver=deliver)
     if out is not None:
@@ -526,19 +527,24 @@ def nms_batched(
     return nms_op(*args)
 
 
-def nms_statistics(preds: Sequence[torch.Tensor], **kw) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+def nms_statistics(
+    preds: Sequence[torch.Tensor],
+    conf_thres: float = 0.25,
+    iou_thres: float = 0.45,
+    classes: Optional[Sequence[int]] = None,
+    agnostic: bool = False,
+    multi_label: bool = False,
+    max_det: int = 300,
+    max_nms: int = MAX_NMS,
+    max_wh: float = MAX_WH,
+    use_summary: bool = True,
+) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
     """``nms_batched`` plus per-segment counters: returns ``(dets, counts, stats[T, B, 2])`` with the IoU tests made and
     the candidates consumed per (task, image) segment (``cerb_nms_stats``; bench.py's IoU pairs/s)."""
+    params = _nms_params(conf_thres, iou_thres, classes, agnostic, multi_label, max_det, max_nms, max_wh)
     preds = list(preds)
-    T, B = len(preds), int(preds[0].shape[0])
-    stats = torch.zeros((T, B, 2), dtype=torch.int64, device=preds[0].device)
-    use_summary = kw.pop("use_summary", True)
-    found = [find_summary(p) for p in preds] if use_summary else []
-    smax = found if found and all(f is not None for f in found) else []
-    dets, counts = _nms_impl(preds, float(kw.get("conf_thres", 0.25)), float(kw.get("iou_thres", 0.45)),
-                             None if kw.get("classes") is None else [int(c) for c in kw["classes"]], bool(kw.get("agnostic", False)),
-                             bool(kw.get("multi_label", False)), int(kw.get("max_det", 300)), int(kw.get("max_nms", MAX_NMS)),
-                             float(kw.get("max_wh", MAX_WH)), smax, None, stats)
+    stats = torch.zeros((len(preds), int(preds[0].shape[0]), 2), dtype=torch.int64, device=preds[0].device)
+    dets, counts = _nms_impl(preds, *params, _summaries(preds, use_summary), stats=stats)
     return dets, counts, stats
 
 
@@ -552,62 +558,36 @@ def cross_task_merge(dets: torch.Tensor, counts: torch.Tensor, class_offsets: Se
     _require_cuda(dets, "dets")
     T, B, max_det, _ = dets.shape
     dets, counts = dets.contiguous(), counts.contiguous()
-    ws_bytes = int(lib.cerb_cross_task_workspace_bytes(T, B, max_det))  # 0 while T*max_det <= 1024
-    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dets.device) if ws_bytes else None
+    ws = _workspace(lib.cerb_cross_task_workspace_bytes(T, B, max_det), dets.device)  # 0 bytes while T*max_det <= 1024
     out = torch.empty((B, T * max_det, 6), dtype=torch.float32, device=dets.device)
     out_counts = torch.empty((B,), dtype=torch.int32, device=dets.device)
     if scale is not None:
         scale = scale.to(device=dets.device, dtype=torch.float32).contiguous()
         if tuple(scale.shape) != (B, 5):
             raise ValueError("scale must be [B, 5]")
-    with torch.cuda.device(dets.device):
-        rc = lib.cerb_cross_task_ws(dets.data_ptr(), counts.data_ptr(), T, B, max_det, _lib.int_array([int(o) for o in class_offsets]),
-                                    float(iou_thres), scale.data_ptr() if scale is not None else None, out.data_ptr(),
-                                    out_counts.data_ptr(), ws.data_ptr() if ws is not None else None, ws_bytes,
-                                    _stream_ptr(dets.device))
-    _lib.check(rc)
+    _launch(lib.cerb_cross_task_ws, dets.device, dets.data_ptr(), counts.data_ptr(), T, B, max_det,
+            _lib.int_array([int(o) for o in class_offsets]), float(iou_thres), scale.data_ptr() if scale is not None else None,
+            out.data_ptr(), out_counts.data_ptr(), ws.data_ptr(), ws.numel())
     return out, out_counts
 
 
 def _decode_nms_impl(levels, nc, strides, conf_thres, iou_thres, classes, agnostic, multi_label, max_det, max_nms, max_wh):
     lib = _lib.load()
-    T = len(nc)
-    if T == 0 or len(levels) % T:
-        raise ValueError("levels must hold T*L tensors, task-major")
-    L = len(levels) // T
-    if len(strides) != L:
-        raise ValueError(f"expected {L} strides, got {len(strides)}")
-    first = levels[0]
-    _require_cuda(first, "head tensors")
-    code = _dtype_code(first)
-    B = int(first.shape[0])
-    H = [int(levels[l].shape[2]) for l in range(L)]
-    W = [int(levels[l].shape[3]) for l in range(L)]
-    A = sum(h * w for h, w in zip(H, W))
-    lv = []
-    for t in range(T):
-        for l in range(L):
-            x = levels[t * L + l]
-            if x.device != first.device or x.dtype != first.dtype or tuple(x.shape) != (B, 64 + nc[t], H[l], W[l]):
-                raise ValueError(f"task {t} level {l}: expected {(B, 64 + nc[t], H[l], W[l])} {first.dtype} on {first.device}")
-            lv.append(_dense16(x))
+    code, B, H, W, lv, _ = _dense_heads(levels, nc, strides)
+    first, T, L = levels[0], len(nc), len(H)
     dev = first.device
-    ys = [torch.empty((B, 4 + n, A), dtype=first.dtype, device=dev) for n in nc]
-    R = _summary_len([h * w for h, w in zip(H, W)], first.element_size())
-    sm = [torch.empty((B, n, max(R, 1)), dtype=first.dtype, device=dev) for n in nc]
+    out = [first.new_empty(s) for s in _decode_shapes(B, nc, [h * w for h, w in zip(H, W)], first.element_size())]
+    ys, sm = out[:T], out[T:]
     dets = torch.empty((T, B, max_det, 6), dtype=torch.float32, device=dev)
     counts = torch.empty((T, B), dtype=torch.int32, device=dev)
-    ws_bytes = lib.cerb_nms_workspace_bytes(T, B, max_det)
-    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
-    with torch.cuda.device(dev):
-        rc = lib.cerb_decode_nms(
+    ws = _workspace(lib.cerb_nms_workspace_bytes(T, B, max_det), dev)
+    _launch(lib.cerb_decode_nms, dev,
             _lib.ptr_array([x.data_ptr() for x in lv]), _lib.int_array(list(nc)), T, L, B, _lib.int_array(H), _lib.int_array(W),
             _lib.float_array([float(s) for s in strides]), code, _lib.ptr_array([y.data_ptr() for y in ys]),
-            _lib.ptr_array([x.data_ptr() for x in sm]) if R else None, float(conf_thres), float(iou_thres),
+            _lib.ptr_array([x.data_ptr() for x in sm]) if sm[0].shape[-1] else None, float(conf_thres), float(iou_thres),
             _lib.int_array(list(classes)) if classes is not None else None, len(classes) if classes is not None else 0,
             int(bool(agnostic)), int(bool(multi_label)), int(max_det), int(max_nms), float(max_wh), dets.data_ptr(),
-            counts.data_ptr(), ws.data_ptr() if ws is not None else None, ws_bytes, _stream_ptr(dev))
-    _lib.check(rc)
+            counts.data_ptr(), ws.data_ptr(), ws.numel())
     return [dets, counts] + ys
 
 
@@ -616,12 +596,9 @@ def decode_nms(task_levels: Sequence[Sequence[torch.Tensor]], strides: Sequence[
                multi_label: bool = False, max_det: int = 300, max_nms: int = MAX_NMS, max_wh: float = MAX_WH):
     """Raw head tensors -> padded detections in ONE library call (``cerb::decode_nms`` / ``cerb_decode_nms``: both kernels
     back to back on the current stream).  Returns ``(dets[T,B,max_det,6], counts[T,B], ys)``."""
-    assert 0 <= conf_thres <= 1, f"Invalid Confidence threshold {conf_thres}, valid values are between 0.0 and 1.0"
-    assert 0 <= iou_thres <= 1, f"Invalid IoU {iou_thres}, valid values are between 0.0 and 1.0"
+    params = _nms_params(conf_thres, iou_thres, classes, agnostic, multi_label, max_det, max_nms, max_wh)
     nc = [int(lv[0].shape[1]) - 64 for lv in task_levels]
-    out = decode_nms_op([x for row in task_levels for x in row], nc, [float(s) for s in strides], float(conf_thres),
-                        float(iou_thres), None if classes is None else [int(c) for c in classes], bool(agnostic),
-                        bool(multi_label), int(max_det), int(max_nms), float(max_wh))
+    out = decode_nms_op([x for row in task_levels for x in row], nc, [float(s) for s in strides], *params)
     return out[0], out[1], out[2:]
 
 
@@ -646,10 +623,8 @@ def match_batch(dets: torch.Tensor, counts: torch.Tensor, labels: torch.Tensor, 
     iou_host = list(iouv_host) if iouv_host is not None else [float(v) for v in iouv.detach().cpu().float().tolist()]
     K = len(iou_host)
     correct = torch.empty((B, max_det, K), dtype=torch.uint8, device=dev)
-    with torch.cuda.device(dev):
-        rc = lib.cerb_val_match(dets.data_ptr(), counts.data_ptr(), B, max_det, labels.data_ptr() if labels.numel() else None,
-                                offs_d.data_ptr(), mmax, _lib.float_array(iou_host), K, correct.data_ptr(), _stream_ptr(dev))
-    _lib.check(rc)
+    _launch(lib.cerb_val_match, dev, dets.data_ptr(), counts.data_ptr(), B, max_det, labels.data_ptr() if labels.numel() else None,
+            offs_d.data_ptr(), mmax, _lib.float_array(iou_host), K, correct.data_ptr())
     return correct.bool()
 
 
@@ -672,9 +647,7 @@ class _BboxDecode(torch.autograd.Function):
         x = pred_dist.contiguous()
         ap = anchor_points.to(pred_dist.dtype).contiguous()
         out = torch.empty((B, A, 4), dtype=pred_dist.dtype, device=pred_dist.device)
-        with torch.cuda.device(x.device):
-            rc = lib.cerb_bbox_decode_fwd(x.data_ptr(), ap.data_ptr(), B * A, A, 16, code, out.data_ptr(), _stream_ptr(x.device))
-        _lib.check(rc)
+        _launch(lib.cerb_bbox_decode_fwd, x.device, x.data_ptr(), ap.data_ptr(), B * A, A, 16, code, out.data_ptr())
         ctx.save_for_backward(x)
         ctx.code = code
         return out
@@ -685,10 +658,8 @@ class _BboxDecode(torch.autograd.Function):
         lib = _lib.load()
         g = grad_out.to(x.dtype).contiguous()
         grad_in = torch.empty_like(x)
-        with torch.cuda.device(x.device):
-            rc = lib.cerb_bbox_decode_bwd(x.data_ptr(), g.data_ptr(), x.shape[0] * x.shape[1], 16, ctx.code,
-                                          grad_in.data_ptr(), _stream_ptr(x.device))
-        _lib.check(rc)
+        _launch(lib.cerb_bbox_decode_bwd, x.device, x.data_ptr(), g.data_ptr(), x.shape[0] * x.shape[1], 16, ctx.code,
+                grad_in.data_ptr())
         return None, grad_in
 
 
@@ -726,13 +697,10 @@ def tal_assign(pd_scores: torch.Tensor, pd_bboxes: torch.Tensor, anc_points: tor
     scores = torch.empty((B, A, C), dtype=torch.float32, device=dev)
     fg = torch.empty((B, A), dtype=torch.bool, device=dev)
     gidx = torch.empty((B, A), dtype=torch.int64, device=dev)
-    ws_bytes = int(lib.cerb_tal_workspace_bytes(B, A, G, int(topk)))
-    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-    with torch.cuda.device(dev):
-        rc = lib.cerb_tal_assign(sc.data_ptr(), pb.data_ptr(), an.data_ptr(), gl.data_ptr(), gb.data_ptr(), mg.data_ptr(), B, A, C, G,
-                                 int(topk), float(alpha), float(beta), float(eps), code, labels.data_ptr(), bboxes.data_ptr(),
-                                 scores.data_ptr(), fg.data_ptr(), gidx.data_ptr(), ws.data_ptr(), ws_bytes, _stream_ptr(dev))
-    _lib.check(rc)
+    ws = _workspace(lib.cerb_tal_workspace_bytes(B, A, G, int(topk)), dev)
+    _launch(lib.cerb_tal_assign, dev, sc.data_ptr(), pb.data_ptr(), an.data_ptr(), gl.data_ptr(), gb.data_ptr(), mg.data_ptr(),
+            B, A, C, G, int(topk), float(alpha), float(beta), float(eps), code, labels.data_ptr(), bboxes.data_ptr(),
+            scores.data_ptr(), fg.data_ptr(), gidx.data_ptr(), ws.data_ptr(), ws.numel())
     for t in (sc, pb, an, gl, gb, mg, ws):
         t.record_stream(torch.cuda.current_stream(dev))
     return labels, bboxes, scores, fg, gidx
@@ -786,18 +754,14 @@ class _BboxLoss(torch.autograd.Function):
         tb, ts, fg = target_bboxes.contiguous(), target_scores.contiguous(), fg_mask.contiguous()
         loss_iou = torch.empty((), dtype=torch.float32, device=dev)
         loss_dfl = torch.empty((), dtype=torch.float32, device=dev)
-        ws_bytes = int(lib.cerb_bbox_loss_workspace_bytes(B, A))
-        ws = torch.zeros((ws_bytes,), dtype=torch.uint8, device=dev)
+        ws = torch.zeros((int(lib.cerb_bbox_loss_workspace_bytes(B, A)),), dtype=torch.uint8, device=dev)  # the ticket starts at 0
         if per_anchor is not None and (tuple(per_anchor.shape) != (B, A, 2) or per_anchor.dtype != torch.float32
                                        or not per_anchor.is_contiguous() or per_anchor.device != dev):
             raise ValueError(f"per_anchor must be a contiguous float32 [{B}, {A}, 2] tensor on {dev}")
         tss_ptr = tss_dev.data_ptr() if tss_dev is not None else None
-        with torch.cuda.device(dev):
-            rc = lib.cerb_bbox_loss_fwd(x.data_ptr(), pb.data_ptr(), ap.data_ptr(), tb.data_ptr(), ts.data_ptr(), fg.data_ptr(),
-                                        tss_ptr, tss_host, B, A, C, 16, code, loss_iou.data_ptr(), loss_dfl.data_ptr(),
-                                        per_anchor.data_ptr() if per_anchor is not None else None, ws.data_ptr(), ws_bytes,
-                                        _stream_ptr(dev))
-        _lib.check(rc)
+        _launch(lib.cerb_bbox_loss_fwd, dev, x.data_ptr(), pb.data_ptr(), ap.data_ptr(), tb.data_ptr(), ts.data_ptr(), fg.data_ptr(),
+                tss_ptr, tss_host, B, A, C, 16, code, loss_iou.data_ptr(), loss_dfl.data_ptr(),
+                per_anchor.data_ptr() if per_anchor is not None else None, ws.data_ptr(), ws.numel())
         ctx.save_for_backward(x, pb, ap, tb, ts, fg, tss_dev)
         ctx.meta = (B, A, C, code, tss_dev is not None, tss_host)
         return loss_iou, loss_dfl
@@ -812,11 +776,9 @@ class _BboxLoss(torch.autograd.Function):
         g_dfl = torch.zeros((), dtype=torch.float32, device=dev) if g_dfl is None else g_dfl.detach().reshape(()).float()
         grad_dist = torch.empty_like(x)
         grad_boxes = torch.empty_like(pb)
-        with torch.cuda.device(dev):
-            rc = lib.cerb_bbox_loss_bwd(x.data_ptr(), pb.data_ptr(), ap.data_ptr(), tb.data_ptr(), ts.data_ptr(), fg.data_ptr(),
-                                        tss.data_ptr() if has_tss else None, tss_host, B, A, C, 16, code, g_iou.data_ptr(),
-                                        g_dfl.data_ptr(), grad_dist.data_ptr(), grad_boxes.data_ptr(), _stream_ptr(dev))
-        _lib.check(rc)
+        _launch(lib.cerb_bbox_loss_bwd, dev, x.data_ptr(), pb.data_ptr(), ap.data_ptr(), tb.data_ptr(), ts.data_ptr(), fg.data_ptr(),
+                tss.data_ptr() if has_tss else None, tss_host, B, A, C, 16, code, g_iou.data_ptr(), g_dfl.data_ptr(),
+                grad_dist.data_ptr(), grad_boxes.data_ptr())
         return grad_dist, grad_boxes, None, None, None, None, None, None
 
 
@@ -871,13 +833,9 @@ def ap_per_class(tp: torch.Tensor, conf: torch.Tensor, pred_cls: torch.Tensor, t
     ap = torch.empty((nc, K), dtype=torch.float64, device=dev)
     p = torch.empty((nc, 1000), dtype=torch.float64, device=dev)
     r = torch.empty((nc, 1000), dtype=torch.float64, device=dev)
-    ws_bytes = int(lib.cerb_ap_workspace_bytes(n, K, nc))
-    ws = torch.empty((max(ws_bytes, 1),), dtype=torch.uint8, device=dev)
-    with torch.cuda.device(dev):
-        rc = lib.cerb_ap_per_class(tpc.data_ptr(), K, conf32.data_ptr(), cls32.data_ptr(), n, classes_h.data_ptr(),
-                                   nt_h.data_ptr(), nc, float(eps), ap.data_ptr(), p.data_ptr(), r.data_ptr(), ws.data_ptr(),
-                                   ws_bytes, _stream_ptr(dev))
-    _lib.check(rc)
+    ws = _workspace(lib.cerb_ap_workspace_bytes(n, K, nc), dev)
+    _launch(lib.cerb_ap_per_class, dev, tpc.data_ptr(), K, conf32.data_ptr(), cls32.data_ptr(), n, classes_h.data_ptr(),
+            nt_h.data_ptr(), nc, float(eps), ap.data_ptr(), p.data_ptr(), r.data_ptr(), ws.data_ptr(), ws.numel())
     for t in (tpc, conf32, cls32, ws):
         t.record_stream(torch.cuda.current_stream(dev))
     return ap, p, r, classes, nt

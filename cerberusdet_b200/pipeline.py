@@ -112,9 +112,7 @@ class PostHeadPipeline:
     def _nms(self, p, piggyback: bool = False):
         T = len(self.heads)
         ys = self.ybuf[p][:T]
-        for y, sm in zip(ys, self.ybuf[p][T:]):  # the summary of a static buffer describes whatever decode wrote last
-            if sm.shape[-1]:
-                ops._remember_summary(y, sm)
+        ops._publish_summaries(ys, self.ybuf[p][T:])  # the summary of a static buffer describes whatever decode wrote last
         deliver = self.delivery.nms_deliver_args(p, piggyback) if self.delivery is not None else None
         return ops.nms_batched(ys, out=self.outs[p], deliver=deliver, **self.kw)
 

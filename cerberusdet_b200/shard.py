@@ -284,25 +284,20 @@ class PeerDelivery:
         it.  A no-op on dst and in ``direct`` mode."""
         if self.rank == self.dst or self.direct:
             return
-        from . import _lib
+        from . import _lib, ops
 
-        dev = self.local.device
-        with torch.cuda.device(dev):
-            _lib.check(_lib.load().cerb_deliver_push(self._stage[slot].data_ptr(), self._remote[slot].data_ptr(), self.n,
-                                                     *self._words[slot], torch.cuda.current_stream(dev).cuda_stream))
+        ops._launch(_lib.load().cerb_deliver_push, self.local.device, self._stage[slot].data_ptr(), self._remote[slot].data_ptr(),
+                    self.n, *self._words[slot])
 
     def collect(self, slot: int) -> None:
         """dst: enqueue (current stream) the kernel that waits for every rank's batch in ``slot`` and acknowledges it.
         A no-op on the other ranks."""
         if self.rank != self.dst:
             return
-        from . import _lib
+        from . import _lib, ops
 
         flags, acks, collected = self._collect[slot]
-        dev = self.local.device
-        with torch.cuda.device(dev):
-            _lib.check(_lib.load().cerb_deliver_collect(flags, _lib.ptr_array(acks), collected, self.world, self.dst,
-                                                        torch.cuda.current_stream(dev).cuda_stream))
+        ops._launch(_lib.load().cerb_deliver_collect, self.local.device, flags, _lib.ptr_array(acks), collected, self.world, self.dst)
 
     # the hand-shake lives in kernels the pipeline enqueues: nothing to do around a write
     def before_write(self, slot: int) -> None:

@@ -126,6 +126,20 @@ def test_decode_rejects_cpu_and_bad_shapes(ops):
         ops.decode_heads(bad, STRIDES)
 
 
+def test_decode_nms_rejects_heads_as_decode_does(ops):
+    """decode_nms checks its raw heads as decode does: a dtype mismatch raises TypeError, a wrong shape ValueError."""
+    heads = synth_heads(range(1), [20], 64, torch.float32)
+    mixed = [[_dev(x) for x in heads[0]]]
+    mixed[0][1] = mixed[0][1].half()
+    bad = [[_dev(x) for x in heads[0]]]
+    bad[0][1] = bad[0][1][:, :80].contiguous()
+    for fn in (ops.decode_heads, ops.decode_nms):
+        with pytest.raises(TypeError):
+            fn(mixed, STRIDES)
+        with pytest.raises(ValueError):
+            fn(bad, STRIDES)
+
+
 # ------------------------------------------------------------------ NMS
 def _assert_rows_equal(got, want, ctx=""):
     assert len(got) == len(want)

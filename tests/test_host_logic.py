@@ -117,6 +117,20 @@ def test_ops_refuse_cpu_tensors():
         ops.bbox_decode(torch.zeros(4, 2), torch.zeros(1, 4, 64))
 
 
+def test_nms_statistics_takes_the_keywords_of_nms_batched():
+    import inspect
+
+    from cerberusdet_b200 import ops
+
+    defaults = lambda fn: {k: p.default for k, p in inspect.signature(fn).parameters.items() if k not in ("out", "deliver")}  # noqa: E731
+    assert defaults(ops.nms_statistics) == defaults(ops.nms_batched)
+    preds = [torch.zeros(1, 9, 8)]
+    with pytest.raises(TypeError, match="iou_thresh"):  # a misspelt keyword is an error, not the default threshold
+        ops.nms_statistics(preds, iou_thresh=0.5)
+    with pytest.raises(AssertionError, match="Invalid IoU"):  # the reference's assert, as in nms_batched
+        ops.nms_statistics(preds, iou_thres=1.5)
+
+
 def test_bench_reference_arm_prints_the_contract_line():
     """`bench.py --impl reference` (the arm the driver runs first) on the host cores: one bounded step, one JSON line."""
     import json
