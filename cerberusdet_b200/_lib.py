@@ -58,6 +58,7 @@ PROTOTYPES = {
     "cerb_bbox_loss_bwd": (_i, [_vp] * 7 + [_d] + [_i] * 5 + [_vp] * 5),
     "cerb_ap_workspace_bytes": (_sz, [_lg, _i, _i]),
     "cerb_ap_per_class": (_i, [_vp, _i, _vp, _vp, _lg, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "cerb_letterbox": (_i, [_vpp, _ip, _ip, ctypes.POINTER(_lg), _ip, _ip, _ip, _ip, _i, _i, _i, _i, _vp, _vp]),
     "cerb_debug_set": (_i, [ctypes.c_char_p, _i]),
     "cerb_debug_reset": (_i, []),
     "cerb_debug_set_chunking": (_i, [_i, _i]),

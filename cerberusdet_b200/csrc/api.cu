@@ -544,3 +544,41 @@ extern "C" int cerb_bbox_decode_bwd(const void* pred_dist, const void* grad_out,
     return cerb_launch_status("cerb_bbox_decode_bwd",
                               cerb_launch_bbox_decode_bwd(pred_dist, grad_out, n_rows, dtype, grad_pred_dist, (cudaStream_t)stream));
 }
+
+// ------------------------------------------------------------------ letterbox preprocessing (SURVEY row 10)
+extern "C" int cerb_letterbox(const void* const* src, const int* h, const int* w, const long* pitch, const int* unpad_h,
+                              const int* unpad_w, const int* top, const int* left, int B, int out_h, int out_w, int dtype,
+                              void* out, void* stream) {
+    cerb_clear_error();
+    CERB_REQUIRE(B >= 0, "cerb_letterbox: negative batch %d", B);
+    CERB_REQUIRE(out_h > 0 && out_w > 0 && out_h <= CERB_LB_MAX_SIDE && out_w <= CERB_LB_MAX_SIDE,
+                 "cerb_letterbox: output size %dx%d outside [1, %d]", out_h, out_w, CERB_LB_MAX_SIDE);
+    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_letterbox: unsupported dtype %d", dtype);
+    if (B == 0) return 0;
+    CERB_REQUIRE(src && h && w && pitch && unpad_h && unpad_w && top && left && out, "cerb_letterbox: null argument");
+    for (int i = 0; i < B; ++i) {
+        CERB_REQUIRE(src[i] != nullptr, "cerb_letterbox: image %d is null", i);
+        CERB_REQUIRE(h[i] > 0 && w[i] > 0 && h[i] <= CERB_LB_MAX_SIDE && w[i] <= CERB_LB_MAX_SIDE,
+                     "cerb_letterbox: image %d has size %dx%d outside [1, %d]", i, h[i], w[i], CERB_LB_MAX_SIDE);
+        CERB_REQUIRE(pitch[i] >= 3l * w[i], "cerb_letterbox: image %d has a row pitch of %ld bytes < 3 * width %d", i, pitch[i], w[i]);
+        CERB_REQUIRE(unpad_h[i] > 0 && unpad_w[i] > 0, "cerb_letterbox: image %d resizes to an empty %dx%d", i, unpad_h[i], unpad_w[i]);
+        CERB_REQUIRE(top[i] >= 0 && left[i] >= 0 && (long)top[i] + unpad_h[i] <= out_h && (long)left[i] + unpad_w[i] <= out_w,
+                     "cerb_letterbox: image %d: %dx%d at top %d, left %d does not fit the %dx%d output", i, unpad_h[i],
+                     unpad_w[i], top[i], left[i], out_h, out_w);
+    }
+    const size_t image_bytes = (size_t)3 * out_h * out_w * (dtype == CERB_F16 ? 2 : 4);
+    LetterboxParams P;
+    memset(&P, 0, sizeof(P));
+    P.out_h = out_h;
+    P.out_w = out_w;
+    for (int b0 = 0; b0 < B; b0 += CERB_LB_MAX_IMAGES) {  // one launch up to CERB_LB_MAX_IMAGES images
+        const int n = B - b0 < CERB_LB_MAX_IMAGES ? B - b0 : CERB_LB_MAX_IMAGES;
+        for (int k = 0; k < n; ++k) {
+            const int i = b0 + k;
+            P.img[k] = LbImage{(const unsigned char*)src[i], (long long)pitch[i], h[i], w[i], unpad_h[i], unpad_w[i], top[i], left[i]};
+        }
+        P.out = (char*)out + (size_t)b0 * image_bytes;
+        if (const int rc = cerb_launch_status("cerb_letterbox", cerb_launch_letterbox(P, n, dtype, (cudaStream_t)stream))) return rc;
+    }
+    return 0;
+}

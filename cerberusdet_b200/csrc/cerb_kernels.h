@@ -135,3 +135,21 @@ cudaError_t cerb_launch_bbox_decode_fwd(const void* pred, const void* anchor_poi
                                         cudaStream_t stream);
 cudaError_t cerb_launch_bbox_decode_bwd(const void* pred, const void* grad_out, long n_rows, int dtype, void* grad_in,
                                         cudaStream_t stream);
+
+// ------------------------------------------------------------------ letterbox preprocessing (SURVEY row 10)
+#define CERB_LB_MAX_IMAGES 256  // images per launch (the table travels in the kernel parameters: 40 B each)
+#define CERB_LB_MAX_SIDE 32768  // longest image or output side (keeps every offset of the kernel in 32 bits)
+struct LbImage {
+    const unsigned char* src;  // uint8 HWC BGR rows
+    long long pitch;           // bytes between rows, >= 3 * w
+    int h, w;                  // source size
+    int uh, uw;                // resized size (cv2.resize's dsize)
+    int top, left;             // border above / left of the resized image
+};
+struct LetterboxParams {
+    LbImage img[CERB_LB_MAX_IMAGES];
+    void* out;  // [n_images, 3, out_h, out_w] dtype: RGB planes, value / 255
+    int out_h, out_w;
+};
+// letterbox.cu; one CTA column per image of P.img[0 .. n_images)
+cudaError_t cerb_launch_letterbox(const LetterboxParams& P, int n_images, int dtype, cudaStream_t stream);

@@ -839,3 +839,59 @@ def ap_per_class(tp: torch.Tensor, conf: torch.Tensor, pred_cls: torch.Tensor, t
     for t in (tpc, conf32, cls32, ws):
         t.record_stream(torch.cuda.current_stream(dev))
     return ap, p, r, classes, nt
+
+
+# ----------------------------------------------------------------------------- letterbox preprocessing (SURVEY row 10)
+def _letterbox_impl(images: Sequence[torch.Tensor], geometry: Sequence[int], out_hw: Sequence[int], dtype: torch.dtype) -> torch.Tensor:
+    lib = _lib.load()
+    B = len(images)
+    if B == 0 or len(geometry) != 4 * B or len(out_hw) != 2:
+        raise ValueError("letterbox: one image and four geometry values (unpad_h, unpad_w, top, left) per image, out_hw = (H, W)")
+    code = _DTYPES.get(dtype)
+    if code is None:
+        raise TypeError(f"letterbox writes float16 or float32, got {dtype}")
+    dev = images[0].device
+    _require_cuda(images[0], "images")
+    ims = []
+    for i, im in enumerate(images):
+        if im.device != dev:
+            raise TypeError(f"image {i} is on {im.device}, image 0 on {dev}")
+        if im.dtype != torch.uint8 or im.dim() != 3 or im.shape[2] != 3:
+            raise TypeError(f"image {i}: expected a uint8 [h, w, 3] BGR tensor, got {im.dtype} {tuple(im.shape)}")
+        if im.stride(2) != 1 or im.stride(1) != 3 or im.stride(0) < 3 * im.shape[1]:  # rows may be strided (a crop), pixels packed
+            im = im.clone(memory_format=torch.contiguous_format)
+        ims.append(im)
+    out_h, out_w = int(out_hw[0]), int(out_hw[1])
+    out = torch.empty((B, 3, out_h, out_w), dtype=dtype, device=dev)
+    g = [int(v) for v in geometry]
+    _launch(lib.cerb_letterbox, dev, _lib.ptr_array([im.data_ptr() for im in ims]), _lib.int_array([int(im.shape[0]) for im in ims]),
+            _lib.int_array([int(im.shape[1]) for im in ims]), (ctypes.c_long * B)(*[im.stride(0) for im in ims]),
+            _lib.int_array(g[0::4]), _lib.int_array(g[1::4]), _lib.int_array(g[2::4]), _lib.int_array(g[3::4]), B, out_h, out_w,
+            code, out.data_ptr())
+    for im, orig in zip(ims, images):
+        if im is not orig:  # a packed copy made here: the kernel is only enqueued
+            im.record_stream(torch.cuda.current_stream(dev))
+    return out
+
+
+@torch.library.custom_op("cerb::letterbox", mutates_args=())
+def letterbox_op(images: Sequence[torch.Tensor], geometry: Sequence[int], out_hw: Sequence[int], dtype: torch.dtype) -> torch.Tensor:
+    """``[B, 3, H, W]`` letterboxed RGB / 255 from B uint8 HWC BGR images; ``geometry`` = ``(unpad_h, unpad_w, top, left)``
+    per image, flattened."""
+    return _letterbox_impl(images, geometry, out_hw, dtype)
+
+
+@letterbox_op.register_fake
+def _(images, geometry, out_hw, dtype):
+    return images[0].new_empty((len(images), 3, int(out_hw[0]), int(out_hw[1])), dtype=dtype)
+
+
+def letterbox(images: Sequence[torch.Tensor], geometry: Sequence[Sequence[int]], out_hw: Sequence[int],
+              dtype: torch.dtype = torch.float16) -> torch.Tensor:
+    """The reference's letterbox + BGR->RGB + HWC->CHW + stack + ``/255`` (cerberusdet_preprocessor.py:42-74,
+    data/augmentations.py:59-90) for B images in one ``cerb_letterbox`` launch.  ``images[i]``: a uint8 ``[h, w, 3]`` BGR
+    CUDA tensor (read in place; rows may be strided); ``geometry[i] = (unpad_h, unpad_w, top, left)``: the size it is
+    resized to and its border above and left (``preprocess.letterbox_geometry``); ``out_hw = (H, W)``.  Returns
+    ``[B, 3, H, W]`` in ``dtype`` (float16 | float32), the pad 114 outside the images; pixels equal cv2's."""
+    flat = [int(v) for g in geometry for v in g]
+    return letterbox_op(list(images), flat, [int(out_hw[0]), int(out_hw[1])], dtype)

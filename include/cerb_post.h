@@ -358,6 +358,26 @@ int cerb_ap_per_class(const unsigned char* tp, int K, const float* conf, const f
                       size_t workspace_bytes, void* stream);
 
 /*
+ * Letterbox preprocessing of B images of any sizes in one launch: the inference front end of
+ * CerberusPreprocessor.preprocess (cerberusdet/cerberusdet_preprocessor.py:42-74) -- letterbox
+ * (cerberusdet/data/augmentations.py:59-90: cv2.resize(INTER_LINEAR) + cv2.copyMakeBorder with 114), BGR -> RGB,
+ * HWC -> CHW, np.stack and the "/ 255" of the uploaded tensor.
+ *
+ *   src[i]        DEVICE uint8 HWC BGR pixels of image i (cv2.imread's layout), h[i] x w[i], rows pitch[i] bytes apart
+ *   unpad_h/w[i]  the size letterbox resizes image i to; top[i] / left[i] its border above / left of it (the caller
+ *                 computes them with the reference's arithmetic, cerberusdet_b200.preprocess.letterbox_geometry)
+ *   out           [B, 3, out_h, out_w] in dtype: RGB planes, value / 255 -- the pad (114) everywhere outside the image
+ * The resize reproduces cv2's uint8 fixed-point INTER_LINEAR (and its switch to INTER_AREA for an exact 2x downscale;
+ * a copy when unpad == h x w): the pixels equal cv2's bit for bit.  The / 255 is ATen's for a CUDA tensor and a Python
+ * scalar: a multiply by the fp32 reciprocal, rounded to dtype.  Images beyond 256 take one more launch per 256.
+ * CERB_EINVAL, before anything touches the device, for B < 0, an unknown dtype, a size outside 1..32768, a pitch below
+ * 3 * w, or an image that does not fit the output (top + unpad_h > out_h, left + unpad_w > out_w, negative border).
+ */
+int cerb_letterbox(const void* const* src, const int* h, const int* w, const long* pitch, const int* unpad_h,
+                   const int* unpad_w, const int* top, const int* left, int B, int out_h, int out_w, int dtype, void* out,
+                   void* stream);
+
+/*
  * Test / tools hooks.  cerb_debug_set(name, value) overrides one internal choice FOR THE CALLING THREAD (so the
  * library stays re-entrant); cerb_debug_reset() drops every override of the calling thread.  Results never depend
  * on a knob: the parity tests run the alternatives against each other.  Knobs: "decode_pipe" (0 = register-resident
