@@ -49,6 +49,7 @@ PROTOTYPES = {
     "cerb_cross_task_workspace_bytes": (_sz, [_i, _i, _i]),
     "cerb_cross_task_ws": (_i, [_vp, _vp, _i, _i, _i, _ip, _d, _vp, _vp, _vp, _vp, _sz, _vp]),
     "cerb_val_match": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _fp, _i, _vp, _vp]),
+    "cerb_confusion_matrix": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _vp]),
     "cerb_bbox_decode_fwd": (_i, [_vp, _vp, _lg, _i, _i, _i, _vp, _vp]),
     "cerb_bbox_decode_bwd": (_i, [_vp, _vp, _lg, _i, _i, _vp, _vp]),
     "cerb_tal_workspace_bytes": (_sz, [_i, _i, _i, _i]),

@@ -519,6 +519,29 @@ extern "C" int cerb_val_match(const float* dets, const int* counts, int B, int m
     return cerb_launch_status("cerb_val_match", cerb_launch_val_match(P, max_labels_per_image, (cudaStream_t)stream));
 }
 
+// ConfusionMatrix.process_batch (cerberusdet/utils/metrics.py:273-370) for a batch of images
+extern "C" int cerb_confusion_matrix(const float* dets, const int* counts, int B, int max_det, const float* labels,
+                                     const int* label_offsets, int n_labels, int nc, double conf, double iou_thres,
+                                     long long* matrix, int* cells, int* status, void* stream) {
+    cerb_clear_error();
+    CERB_REQUIRE(B >= 0 && n_labels >= 0, "cerb_confusion_matrix: negative size");
+    CERB_REQUIRE(max_det >= 0 && max_det <= CERB_CM_MAX_DETS, "cerb_confusion_matrix: max_det=%d outside [0, %d]", max_det, CERB_CM_MAX_DETS);
+    CERB_REQUIRE(nc >= 1 && nc <= CERB_CM_MAX_NC, "cerb_confusion_matrix: nc=%d outside [1, %d]", nc, CERB_CM_MAX_NC);
+    CERB_REQUIRE(iou_thres >= 0.0, "cerb_confusion_matrix: iou_thres=%g must be >= 0", iou_thres);
+    CERB_REQUIRE(label_offsets || (B <= 1 && n_labels <= CERB_CM_MAX_LABELS),
+                 "cerb_confusion_matrix: without label_offsets, one image of at most %d labels (B=%d, n_labels=%d)",
+                 CERB_CM_MAX_LABELS, B, n_labels);
+    if (B == 0) return 0;
+    CERB_REQUIRE(status && (dets || max_det == 0) && (labels || n_labels == 0), "cerb_confusion_matrix: null argument");
+    ConfusionParams P;
+    memset(&P, 0, sizeof(P));
+    P.dets = dets; P.counts = counts; P.labels = labels; P.label_offsets = label_offsets;
+    P.B = B; P.max_det = max_det; P.n_labels = n_labels; P.nc = nc;
+    P.conf = (float)conf; P.iou_thr = (float)iou_thres;
+    P.matrix = (unsigned long long*)matrix; P.cells = cells; P.status = status;
+    return cerb_launch_status("cerb_confusion_matrix", cerb_launch_confusion(P, (cudaStream_t)stream));
+}
+
 // ------------------------------------------------------------------ training-time sibling decode (SURVEY 8f-4)
 extern "C" int cerb_bbox_decode_fwd(const void* pred_dist, const void* anchor_points, long n_rows, int A, int reg_max,
                                     int dtype, void* out, void* stream) {

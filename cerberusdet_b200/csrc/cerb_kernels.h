@@ -129,6 +129,35 @@ struct ValMatchParams {
 };
 cudaError_t cerb_launch_val_match(const ValMatchParams& P, int max_labels_per_image, cudaStream_t stream);
 
+// box_iou (utils/metrics.py:415-433) of one label row q = (cls, x1, y1, x2, y2) and one detection (x1, y1, x2, y2) whose
+// area ad = (x2 - x1) * (y2 - y1) the caller computed: fp32, one rounding per operation, + 1e-7 in the denominator
+__device__ __forceinline__ float cerb_box_iou(const float* q, float x1, float y1, float x2, float y2, float ad) {
+    const float iw = fmaxf(__fsub_rn(fminf(q[3], x2), fmaxf(q[1], x1)), 0.f);
+    const float ih = fmaxf(__fsub_rn(fminf(q[4], y2), fmaxf(q[2], y1)), 0.f);
+    const float inter = __fmul_rn(iw, ih);
+    const float al = __fmul_rn(__fsub_rn(q[3], q[1]), __fsub_rn(q[4], q[2]));
+    return __fdiv_rn(inter, __fadd_rn(__fsub_rn(__fadd_rn(al, ad), inter), 1e-7f));
+}
+
+// ------------------------------------------------------------------ validation confusion matrix (confusion.cu)
+#define CERB_CM_MAX_LABELS 1024
+#define CERB_CM_MAX_DETS 30000
+#define CERB_CM_MAX_NC 32767         // (nc + 1)^2 cells index in 32 bits
+#define CERB_CM_CLASS_RANGE 1        // status: a label or conf-passing detection has a class outside [0, nc)
+#define CERB_CM_LABEL_COUNT 2        // status: the image's label rows are not within [0, 1024] / inside labels
+struct ConfusionParams {
+    const float* dets;           // [B, max_det, 6] (x1, y1, x2, y2, conf, cls)
+    const int* counts;           // [B], or null: every image has max_det detections
+    const float* labels;         // [n_labels, 5] (cls, x1, y1, x2, y2), images concatenated
+    const int* label_offsets;    // device [B + 1], or null (B == 1): all n_labels rows are image 0's
+    int B, max_det, n_labels, nc;
+    float conf, iou_thr;         // the Python floats rounded to fp32, as torch compares an fp32 tensor with them
+    unsigned long long* matrix;  // optional [nc + 1, nc + 1] int64, added to
+    int* cells;                  // optional [n_labels + B * max_det]: the cell each label / detection row adds to, or -1
+    int* status;                 // [B]
+};
+cudaError_t cerb_launch_confusion(const ConfusionParams& P, cudaStream_t stream);
+
 // ------------------------------------------------------------------ training-time sibling decode (SURVEY 8f-4)
 // Loss.bbox_decode forward / backward on pred_dist [n_rows = B * A, 64] (bins contiguous); train_decode.cu
 cudaError_t cerb_launch_bbox_decode_fwd(const void* pred, const void* anchor_points, long n_rows, int A, int dtype, void* out,

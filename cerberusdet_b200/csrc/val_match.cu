@@ -6,7 +6,7 @@
 // keeps its best label; per label the lowest detection index survives (val.py:48-51).  The best label of a
 // detection does not depend on t (it is the arg-max IoU over the class-matching labels; ties -> lowest label, the
 // canonical form of the reference's unstable sort), so one pass finds it and K atomicMin tables resolve the labels.
-// IoU as box_iou (utils/metrics.py:415-433): fp32, one rounding per operation, + 1e-7 in the denominator.
+// IoU: cerb_box_iou (cerb_kernels.h), box_iou's arithmetic.
 #include "cerb_kernels.h"
 
 #define VM_THREADS 256
@@ -35,11 +35,7 @@ __global__ void __launch_bounds__(VM_THREADS) val_match_kernel(const __grid_cons
             for (int l = 0; l < M; ++l) {
                 const float* q = P.labels + (size_t)(l0 + l) * 5;
                 if (q[0] != cls) continue;
-                const float iw = fmaxf(__fsub_rn(fminf(q[3], x2), fmaxf(q[1], x1)), 0.f);
-                const float ih = fmaxf(__fsub_rn(fminf(q[4], y2), fmaxf(q[2], y1)), 0.f);
-                const float inter = __fmul_rn(iw, ih);
-                const float al = __fmul_rn(__fsub_rn(q[3], q[1]), __fsub_rn(q[4], q[2]));
-                const float iou = __fdiv_rn(inter, __fadd_rn(__fsub_rn(__fadd_rn(al, ad), inter), 1e-7f));
+                const float iou = cerb_box_iou(q, x1, y1, x2, y2, ad);
                 if (iou > biou) { biou = iou; bl = l; }  // strict: the lowest label wins ties
             }
             if (bl >= 0)
@@ -62,11 +58,7 @@ __global__ void __launch_bounds__(VM_THREADS) val_match_kernel(const __grid_cons
         for (int l = 0; l < M; ++l) {
             const float* q = P.labels + (size_t)(l0 + l) * 5;
             if (q[0] != cls) continue;
-            const float iw = fmaxf(__fsub_rn(fminf(q[3], x2), fmaxf(q[1], x1)), 0.f);
-            const float ih = fmaxf(__fsub_rn(fminf(q[4], y2), fmaxf(q[2], y1)), 0.f);
-            const float inter = __fmul_rn(iw, ih);
-            const float al = __fmul_rn(__fsub_rn(q[3], q[1]), __fsub_rn(q[4], q[2]));
-            const float iou = __fdiv_rn(inter, __fadd_rn(__fsub_rn(__fadd_rn(al, ad), inter), 1e-7f));
+            const float iou = cerb_box_iou(q, x1, y1, x2, y2, ad);
             if (iou > biou) { biou = iou; bl = l; }
         }
         for (int i = 0; i < K; ++i)

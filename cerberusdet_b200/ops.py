@@ -628,6 +628,79 @@ def match_batch(dets: torch.Tensor, counts: torch.Tensor, labels: torch.Tensor, 
     return correct.bool()
 
 
+# ----------------------------------------------------------------------------- validation confusion matrix
+CM_MAX_LABELS, CM_MAX_DETS = 1024, 30000  # per image (include/cerb_post.h: cerb_confusion_matrix)
+
+
+@torch.library.custom_op("cerb::confusion_matrix", mutates_args=("matrix",))
+def confusion_matrix_op(dets: torch.Tensor, counts: torch.Tensor, labels: torch.Tensor, label_offsets: torch.Tensor, nc: int,
+                        conf: float, iou_thres: float, matrix: torch.Tensor) -> torch.Tensor:
+    """Adds the batch's ``ConfusionMatrix.process_batch`` counts into ``matrix`` and returns the per-image status ``[B]``
+    int32 (``cerb_confusion_matrix``)."""
+    lib = _lib.load()
+    _require_cuda(dets, "dets")
+    dev = dets.device
+    if dets.dim() != 3 or dets.shape[2] != 6 or dets.dtype != torch.float32:
+        raise ValueError(f"dets must be a float32 [B, max_det, 6] tensor, got {dets.dtype} {tuple(dets.shape)}")
+    B, max_det = int(dets.shape[0]), int(dets.shape[1])
+    for t, what, dtype, shape in ((counts, "counts", torch.int32, (B,)), (label_offsets, "label_offsets", torch.int32, (B + 1,)),
+                                  (matrix, "matrix", torch.int64, (nc + 1, nc + 1))):
+        if t.device != dev or t.dtype != dtype or tuple(t.shape) != shape:
+            raise ValueError(f"{what} must be a {dtype} {list(shape)} tensor on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    if labels.device != dev or labels.dtype != torch.float32 or labels.dim() != 2 or labels.shape[1] != 5:
+        raise ValueError(f"labels must be a float32 [n, 5] tensor on {dev}, got {labels.dtype} {tuple(labels.shape)}")
+    if not matrix.is_contiguous():
+        raise ValueError("matrix must be contiguous")
+    dets, counts, labels, offs = dets.contiguous(), counts.contiguous(), labels.contiguous(), label_offsets.contiguous()
+    status = torch.empty((B,), dtype=torch.int32, device=dev)
+    _launch(lib.cerb_confusion_matrix, dev, dets.data_ptr(), counts.data_ptr(), B, max_det, labels.data_ptr() if labels.numel() else None,
+            offs.data_ptr(), int(labels.shape[0]), int(nc), float(conf), float(iou_thres), matrix.data_ptr(), None, status.data_ptr())
+    return status
+
+
+@confusion_matrix_op.register_fake
+def _(dets, counts, labels, label_offsets, nc, conf, iou_thres, matrix):
+    return dets.new_empty((dets.shape[0],), dtype=torch.int32)
+
+
+def confusion_matrix_batch(dets: torch.Tensor, counts: torch.Tensor, labels: torch.Tensor, label_offsets, nc: int,
+                           conf: float = 0.25, iou_thres: float = 0.45,
+                           out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """``ConfusionMatrix(nc, conf, iou_thres).process_batch`` (utils/metrics.py:273-370) for every image of a batch in one
+    ``cerb_confusion_matrix`` launch: ``dets [B, max_det, 6]`` / ``counts [B]`` of one task in native image space (as
+    ``ops.nms_batched`` leaves them after rescaling), ``labels [sum M_b, 5]`` (cls, x1, y1, x2, y2) with ``label_offsets``
+    (a device tensor or ``B+1`` ints).  The counts are the sum of what the reference adds per image: an image with labels
+    and no detections adds ``[nc, cls]`` per label (its ``detections=None`` call), an image without labels nothing.
+
+    Returns ``(matrix, status)``: the ``int64 [nc+1, nc+1]`` device matrix ``[predicted, true]`` -- ``out`` added to, else a
+    new one -- and the per-image ``int32 [B]`` status, non-zero for an image that added nothing because a label or a
+    detection above ``conf`` has a class outside ``[0, nc)`` (1) or it has more than 1024 labels (2).  No host
+    synchronisation with device ``label_offsets`` and int32 ``counts``, so a CUDA graph can capture it.  Equal IoUs resolve
+    to the lowest label index, then the lowest detection index."""
+    _require_cuda(dets, "dets")
+    dev = dets.device
+    if not torch.is_tensor(label_offsets):
+        label_offsets = torch.tensor([int(o) for o in label_offsets], dtype=torch.int32, device=dev)
+    matrix = torch.zeros((int(nc) + 1, int(nc) + 1), dtype=torch.int64, device=dev) if out is None else out
+    status = confusion_matrix_op(dets.float(), counts.to(torch.int32), labels.to(device=dev, dtype=torch.float32),
+                                 label_offsets.to(device=dev, dtype=torch.int32), int(nc), float(conf), float(iou_thres), matrix)
+    return matrix, status
+
+
+def confusion_cells(detections: torch.Tensor, labels: torch.Tensor, nc: int, conf: float, iou_thres: float) -> torch.Tensor:
+    """One image's ``process_batch`` as cells: ``detections [N, 6]`` / ``labels [M, 5]`` float32 CUDA tensors
+    (N <= 30000, M <= 1024) -> one int32 device tensor ``[1 + M + N]``: the image's status, then the flat cell
+    (``row * (nc + 1) + col``) each label and each detection adds 1 to, or -1.  One launch, no host synchronisation."""
+    lib = _lib.load()
+    _require_cuda(detections, "detections")
+    n, m = int(detections.shape[0]), int(labels.shape[0])
+    det, lab = detections.contiguous(), labels.contiguous()
+    buf = torch.empty((1 + m + n,), dtype=torch.int32, device=det.device)
+    _launch(lib.cerb_confusion_matrix, det.device, det.data_ptr() if n else None, None, 1, n, lab.data_ptr() if m else None,
+            None, m, int(nc), float(conf), float(iou_thres), None, buf.data_ptr() + 4, buf.data_ptr())
+    return buf
+
+
 # ----------------------------------------------------------------------------- training-time sibling decode (SURVEY 8f-4)
 class _BboxDecode(torch.autograd.Function):
     """``Loss.bbox_decode`` (reference utils/loss.py:126-131) as one CUDA kernel per direction."""

@@ -26,7 +26,12 @@ What gets rebound (and restored by ``uninstall()``):
   -> ``val_stats.ap_per_class`` (``ops.ap_per_class`` for the per-class curves and APs, the host tail in numpy), in
   ``cerberusdet.utils.metrics`` and in every imported ``cerberusdet.*`` module that imported the name.  ``plot=True``,
   no CUDA device, non-bool ``tp``, more than 32 IoU columns, float64 inputs or NaN scores / classes keep the reference's
-  own function.
+  own function;
+* with ``confusion=True`` ``cerberusdet.utils.metrics.ConfusionMatrix.process_batch`` (utils/metrics.py:273-370, called per
+  image by the validation loop when ``plots`` is on) -> ``val_stats.make_confusion_process_batch``: one launch and one
+  device-to-host copy of the rows' cells per call, applied to the instance's numpy ``matrix`` (the class is kept).
+  ``detections=None``, CPU or non-fp32 tensors, more than 30000 detections or 1024 labels and classes outside
+  ``[0, nc)`` keep the reference's own method.
 
 CUDA fp16/fp32 tensors go to the kernels; anything else (CPU tensors, training mode, masks/labels
 arguments) is handed to the reference's own, saved implementation -- the patch never changes what a
@@ -52,14 +57,15 @@ def installed() -> bool:
 
 
 def install(import_all: bool = False, train: bool = False, val: bool = False, loss: bool = False,
-            metrics: bool = False) -> Dict[str, List[str]]:
+            metrics: bool = False, confusion: bool = False) -> Dict[str, List[str]]:
     """Patch the reference modules that are importable.  ``import_all`` also imports ``val`` /
     ``detect`` / ``cerberusdet_inference`` (they pull in the whole data pipeline); by default only
     modules already imported, plus ``models.yolo`` and ``utils.general``, are touched.  ``train`` also rebinds
     ``Loss.bbox_decode``, ``TaskAlignedAssigner.forward`` and the loss module's ``make_anchors`` (imports
     ``cerberusdet.utils.loss``), ``loss`` the box-regression term ``BboxLoss.forward`` (imports
     ``cerberusdet.utils.loss``), ``val`` the validation matching (imports ``cerberusdet.val``), ``metrics`` the mAP
-    statistics ``ap_per_class`` (imports ``cerberusdet.utils.metrics``).  Calling it again adds
+    statistics ``ap_per_class``, ``confusion`` the confusion matrix's ``ConfusionMatrix.process_batch`` (both import
+    ``cerberusdet.utils.metrics``).  Calling it again adds
     whatever is not patched yet (e.g. ``install()`` then ``install(train=True)``, then ``install(loss=True)``)."""
     import torch
 
@@ -218,6 +224,13 @@ def install(import_all: bool = False, train: bool = False, val: bool = False, lo
             if (modname == "cerberusdet" or modname.startswith("cerberusdet.")) and hasattr(mod, "ap_per_class") \
                     and mod.ap_per_class is ap_per_class._cerb_reference:
                 patch_once(mod, "ap_per_class", ap_per_class, f"{modname}.ap_per_class")
+    if confusion:
+        from . import val_stats as _val_stats
+
+        cm_cls = importlib.import_module("cerberusdet.utils.metrics").ConfusionMatrix
+        if not hasattr(cm_cls.process_batch, "_cerb_reference"):
+            patch_once(cm_cls, "process_batch", _val_stats.make_confusion_process_batch(cm_cls.process_batch),
+                       "cerberusdet.utils.metrics.ConfusionMatrix.process_batch")
     if not done["patched"]:
         return {"already": ["installed"]}
     return done

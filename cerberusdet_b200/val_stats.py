@@ -10,11 +10,14 @@ kernel) is "IoU descending, then label index ascending".
 
 After the loop: ``ap_per_class`` (cerberusdet/utils/metrics.py:56-120), the drop-in whose per-class curves and APs come
 from ``ops.ap_per_class`` and whose O(nc * 1000) tail runs here in numpy, and ``make_ap_per_class``, its guarded form for
-``patch.install(metrics=True)``.
+``patch.install(metrics=True)``.  With ``plots`` on, the loop also feeds ``ConfusionMatrix.process_batch``
+(utils/metrics.py:273-370) per image: ``make_confusion_process_batch`` is its drop-in for ``patch.install(confusion=True)``,
+and ``validation_batch_statistics(confusion=...)`` its batched form.
 """
 from __future__ import annotations
 
 from pathlib import Path
+from typing import Optional
 
 import numpy as np
 import torch
@@ -124,7 +127,8 @@ def _scale_boxes_batched(boxes, inv_gain, pad_x, pad_y, w0, h0):
     return out
 
 
-def validation_batch_statistics(dets: torch.Tensor, counts: torch.Tensor, batch: dict, iouv: torch.Tensor, single_cls: bool = False):
+def validation_batch_statistics(dets: torch.Tensor, counts: torch.Tensor, batch: dict, iouv: torch.Tensor, single_cls: bool = False,
+                                confusion: Optional[torch.Tensor] = None):
     """The "Statistics per image" block of the reference validation loop (cerberusdet/val.py:321-357) for a whole batch
     of ONE task: native-space predictions (``scale_boxes``), native-space labels (``xywh2xyxy`` * (w, h, w, h), then
     ``scale_boxes``), ``process_batch`` -- here: a handful of batched elementwise ops and ONE ``cerb_val_match`` launch, no
@@ -134,7 +138,12 @@ def validation_batch_statistics(dets: torch.Tensor, counts: torch.Tensor, batch:
     space); ``batch``: the reference's batch dict (``img``, ``batch_idx``, ``cls``, ``bboxes``, ``ori_shape``, ``ratio_pad``).
     Returns what the loop would have appended to ``stats``: a list of ``(correct [n, K] bool, conf [n], pcls [n], tcls [m])``
     device-tensor tuples in image order -- images with neither predictions nor labels contribute nothing, images without
-    predictions an empty first three (val.py:333-338)."""
+    predictions an empty first three (val.py:333-338).
+
+    ``confusion``: optional ``int64 [nc+1, nc+1]`` device matrix; the batch's ``ConfusionMatrix(nc).process_batch`` counts
+    (the calls the loop makes when ``plots`` is on, default ``conf`` 0.25 / ``iou_thres`` 0.45) are added to it with one
+    ``cerb_confusion_matrix`` launch on the same native-space predictions and labels.  A class outside ``[0, nc)`` raises
+    ``ValueError`` (the status is read with the counts, so no extra synchronisation)."""
     from . import ops
 
     dev = dets.device
@@ -165,7 +174,16 @@ def validation_batch_statistics(dets: torch.Tensor, counts: torch.Tensor, batch:
     tbox = _scale_boxes_batched(tbox, inv_gain[bidx], pad_x[bidx], pad_y[bidx], w0[bidx], h0[bidx])
     labelsn = torch.cat((cls, tbox), 1)
     correct = ops.match_batch(predn, counts, labelsn, offsets, iouv)  # [B, max_det, K] bool
-    n_host = counts.tolist()
+    if confusion is None:
+        n_host = counts.tolist()
+    else:
+        offsets_d = torch.cat((m_per.new_zeros(1), torch.cumsum(m_per, 0))).to(torch.int32)
+        _, status = ops.confusion_matrix_batch(predn, counts, labelsn, offsets_d, int(confusion.shape[0]) - 1, out=confusion)
+        host = torch.cat((counts.to(torch.int32).view(-1), status)).tolist()
+        n_host, bad = host[:B], [i for i, s in enumerate(host[B:]) if s]
+        if bad:
+            raise ValueError(f"confusion matrix: images {bad} have a class outside [0, {int(confusion.shape[0]) - 1}) or more than "
+                             f"{ops.CM_MAX_LABELS} labels; they were not counted")
     K = int(iouv.shape[0])
     stats = []
     for i in range(B):
@@ -246,3 +264,47 @@ def make_ap_per_class(reference_ap_per_class):
     ap_per_class_.__doc__ = ap_per_class.__doc__
     ap_per_class_._cerb_reference = reference_ap_per_class
     return ap_per_class_
+
+
+# ---------------------------------------------------------------------------------- confusion matrix (with plots on)
+def _confusion_on_path(cm, detections, labels) -> bool:
+    if not (getattr(detections, "is_cuda", False) and getattr(labels, "is_cuda", False)):  # (None: the reference's first case)
+        return False
+    if labels.device != detections.device or not detections.dtype == labels.dtype == torch.float32:
+        return False
+    if detections.dim() != 2 or detections.shape[1] != 6 or labels.dim() != 2 or labels.shape[1] != 5:
+        return False
+    from .ops import CM_MAX_DETS, CM_MAX_LABELS
+
+    if detections.shape[0] > CM_MAX_DETS or labels.shape[0] > CM_MAX_LABELS:
+        return False
+    nc, conf, iou = getattr(cm, "nc", None), getattr(cm, "conf", None), getattr(cm, "iou_thres", None)
+    if not (isinstance(nc, (int, np.integer)) and 1 <= nc <= 32767 and isinstance(getattr(cm, "matrix", None), np.ndarray)
+            and cm.matrix.shape == (nc + 1, nc + 1)):
+        return False
+    return isinstance(conf, (float, int, np.floating, np.integer)) and isinstance(iou, (float, int, np.floating, np.integer)) \
+        and float(iou) >= 0
+
+
+def make_confusion_process_batch(reference_process_batch):
+    """``ConfusionMatrix.process_batch(self, detections, labels)`` (utils/metrics.py:273-370) for
+    ``patch.install(confusion=True)``.  float32 CUDA tensors with at most 30000 detections and 1024 labels take ONE
+    ``cerb_confusion_matrix`` launch and ONE device-to-host copy of ``1 + M + N`` int32 (the status and the cell of every
+    row), applied to ``self.matrix`` with ``np.add.at`` -- the reference synchronises once per label and per detection.
+    The instance's ``nc``, ``conf`` and ``iou_thres`` are used.  Equal IoUs resolve to the lowest label index, then the
+    lowest detection index (the reference's unstable argsorts leave them undefined).  ``detections=None``, CPU tensors,
+    other dtypes, larger images, a negative ``iou_thres`` and a class outside ``[0, nc)`` (seen in the status, before
+    ``self.matrix`` is touched) run the reference's own method."""
+    from . import ops
+
+    def process_batch(self, detections, labels):
+        if not _confusion_on_path(self, detections, labels):
+            return reference_process_batch(self, detections, labels)
+        host = ops.confusion_cells(detections, labels, int(self.nc), float(self.conf), float(self.iou_thres)).cpu().numpy()
+        if host[0]:  # a class numpy would raise or wrap on
+            return reference_process_batch(self, detections, labels)
+        cells = host[1:][host[1:] >= 0]
+        np.add.at(self.matrix, (cells // (self.nc + 1), cells % (self.nc + 1)), 1)
+
+    process_batch._cerb_reference = reference_process_batch
+    return process_batch

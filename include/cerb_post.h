@@ -249,6 +249,31 @@ int cerb_val_match(const float* dets, const int* counts, int B, int max_det, con
                    unsigned char* correct, void* stream);
 
 /*
+ * The validation confusion matrix: ConfusionMatrix.process_batch (cerberusdet/utils/metrics.py:273-370) as the validation
+ * loop calls it per image (val.py:321-357), for a whole batch in one launch (one CTA per image).  Per image: detections
+ * with conf > (float)conf; IoU as box_iou (metrics.py:415-433); a detection's best label is the highest IoU >
+ * (float)iou_thres, ties -> lowest label index; a label keeps the highest-IoU detection that chose it, ties -> lowest
+ * detection index (the reference's unstable argsorts leave ties undefined).  Each label adds [cls(det), cls(label)] or
+ * [nc, cls(label)]; only if some pair survived, each unmatched conf-passing detection adds [cls(det), nc].  Classes are
+ * the values truncated to int.  An image with no labels adds nothing; one with no detections adds [nc, cls] per label.
+ *
+ *   dets, counts     [B, max_det, 6] fp32 (x1, y1, x2, y2, conf, cls) / device [B] int32, or counts NULL: all max_det rows
+ *   labels           device [n_labels, 5] fp32 rows (cls, x1, y1, x2, y2), images concatenated
+ *   label_offsets    device [B + 1] row offsets into labels, or NULL for one image (B == 1) owning all n_labels rows
+ *   matrix           optional in/out [nc + 1, nc + 1] int64 [predicted, true], added to with integer atomics
+ *   cells            optional out [n_labels + B * max_det] int32: the flat cell (row * (nc + 1) + col) each label row,
+ *                    then each detection row adds to, or -1 (filtered, matched, past counts[b], no pair in the image)
+ *   status           out [B] int32 per image: 0, or CERB_CM_CLASS_RANGE (1: a label or conf-passing detection has a class
+ *                    outside [0, nc)) | CERB_CM_LABEL_COUNT (2: more than 1024 labels, or offsets outside labels).  Such
+ *                    an image adds nothing and its cells are -1.
+ * CERB_EINVAL, before anything touches the device, for negative sizes, max_det > 30000, nc outside [1, 32767], iou_thres
+ * < 0 or NaN, or label_offsets NULL with B > 1 or n_labels > 1024.  No host synchronisation; capturable in a CUDA graph.
+ */
+int cerb_confusion_matrix(const float* dets, const int* counts, int B, int max_det, const float* labels,
+                          const int* label_offsets, int n_labels, int nc, double conf, double iou_thres, long long* matrix,
+                          int* cells, int* status, void* stream);
+
+/*
  * Training-time sibling of the decode (SURVEY 8f row 4): Loss.bbox_decode (cerberusdet/utils/loss.py:126-131) =
  * softmax over the reg_max bins of each side, expectation with proj = arange(reg_max), then
  * dist2bbox(xywh=False) (cerberusdet/utils/tal.py:196-205).
