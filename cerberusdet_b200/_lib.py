@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CERB_LIB") or os.path.join(_HERE, "libcerb_post.so")  # CERB_LIB: tools/ only
 
-CERB_F16, CERB_F32 = 0, 1
+CERB_F16, CERB_F32, CERB_BF16 = 0, 1, 2
 CERB_EINVAL, CERB_ECUDA, CERB_ENOSPC = -1, -2, -3
 
 _lib = None

@@ -126,8 +126,12 @@ extern "C" int cerb_debug_set_hist_sample(int stride) {
     return 0;
 }
 
+// bytes per element of a dtype code the post-head kernels take (fp16 / bf16 / fp32), 0 for any other
+static size_t post_elt(int dtype) { return dtype == CERB_F16 || dtype == CERB_BF16 ? 2 : dtype == CERB_F32 ? 4 : 0; }
+
 extern "C" size_t cerb_summary_row_len(int A, int dtype) {
-    const size_t V = dtype == CERB_F16 ? 8 : 4;
+    if (post_elt(dtype) == 0) return 0;
+    const size_t V = 16 / post_elt(dtype);
     if (A <= 0 || (size_t)A % V) return 0;
     return ((size_t)A / V + V - 1) / V * V;
 }
@@ -140,13 +144,13 @@ static int decode_common(const void* const* lvl, const void* const* cls_lvl, con
     CERB_REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_decode: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
     CERB_REQUIRE(L >= 1 && L <= CERB_MAX_LEVELS, "cerb_decode: L=%d outside [1, %d]", L, CERB_MAX_LEVELS);
     CERB_REQUIRE(B >= 0, "cerb_decode: negative batch");
-    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_decode: unsupported dtype %d", dtype);
+    CERB_REQUIRE(post_elt(dtype) != 0, "cerb_decode: unsupported dtype %d", dtype);
     DecodeParams P;
     memset(&P, 0, sizeof(P));
     P.T = T; P.L = L; P.B = B; P.nrows = T * L;
-    P.interleave_parts = dtype == CERB_F32 ? 1 : 2;  // measured best per dtype (profiles/r01_decode.md)
+    P.interleave_parts = dtype == CERB_F32 ? 1 : 2;  // measured best per dtype (profiles/r01_decode.md; bf16 takes fp16's)
     (void)knob(K_DECODE_ORDER, &P.interleave_parts);
-    const size_t elt = dtype == CERB_F16 ? 2 : 4;
+    const size_t elt = post_elt(dtype);
     int vec = (int)(16 / elt);
     long A = 0;
     if (summary_written) *summary_written = 0;
@@ -238,10 +242,12 @@ extern "C" size_t cerb_nms_workspace_bytes(int T, int B, int max_det) {
 }
 
 // torch compares a half tensor with a Python scalar after casting the scalar to half
-// (double -> float -> half), a float tensor after casting it to float (general.py:411).
+// (double -> float -> half), a bfloat16 tensor after casting it to bfloat16 (double -> float -> bf16, round to nearest
+// even, as c10::BFloat16 does: bf16(0.3) = 0.30078125), a float tensor after casting it to float (general.py:411).
 static float round_conf_to_dtype(double conf, int dtype) {
     float f = (float)conf;
     if (dtype == CERB_F16) f = __half2float(__float2half_rn(f));
+    if (dtype == CERB_BF16) f = __bfloat162float(__float2bfloat16_rn(f));
     return f;
 }
 // torchvision's CPU kernel widens the fp32 quotient and compares with the double threshold:
@@ -348,7 +354,7 @@ static int nms_impl(const void* const* pred, const int* nc, int T, int B, int A,
     CERB_REQUIRE(pred && nc, "cerb_nms: null argument");
     CERB_REQUIRE(T >= 1 && T <= CERB_MAX_TASKS, "cerb_nms: T=%d outside [1, %d]", T, CERB_MAX_TASKS);
     CERB_REQUIRE(B >= 0 && A >= 0, "cerb_nms: negative size");
-    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_nms: unsupported dtype %d", dtype);
+    CERB_REQUIRE(post_elt(dtype) != 0, "cerb_nms: unsupported dtype %d", dtype);
     CERB_REQUIRE(conf_thres >= 0.0 && conf_thres <= 1.0, "Invalid Confidence threshold %g, valid values are between 0.0 and 1.0", conf_thres);
     CERB_REQUIRE(iou_thres >= 0.0 && iou_thres <= 1.0, "Invalid IoU %g, valid values are between 0.0 and 1.0", iou_thres);
     CERB_REQUIRE(max_det >= 0 && max_nms >= 0, "cerb_nms: negative max_det/max_nms");
@@ -376,7 +382,7 @@ static int nms_impl(const void* const* pred, const int* nc, int T, int B, int A,
             CERB_REQUIRE(nc[t] <= 32 * CERB_MAX_CLASS_WORDS, "cerb_nms: class filter supports nc <= %d", 32 * CERB_MAX_CLASS_WORDS);
     }
     if (smax != nullptr) {
-        const int V = dtype == CERB_F16 ? 8 : 4;
+        const int V = (int)(16 / post_elt(dtype));
         CERB_REQUIRE(A % V == 0, "cerb_nms: a score summary needs A (%d) to be a multiple of %d", A, V);
         for (int t = 0; t < T; ++t) {
             CERB_REQUIRE(smax[t] != nullptr && cerb_aligned(smax[t], 16), "cerb_nms: smax[%d] is null or misaligned", t);
@@ -546,7 +552,7 @@ extern "C" int cerb_confusion_matrix(const float* dets, const int* counts, int B
 extern "C" int cerb_bbox_decode_fwd(const void* pred_dist, const void* anchor_points, long n_rows, int A, int reg_max,
                                     int dtype, void* out, void* stream) {
     cerb_clear_error();
-    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_bbox_decode_fwd: unsupported dtype %d", dtype);
+    CERB_REQUIRE(post_elt(dtype) != 0, "cerb_bbox_decode_fwd: unsupported dtype %d", dtype);
     CERB_REQUIRE(reg_max == CERB_REG_MAX, "cerb_bbox_decode_fwd: reg_max=%d, only %d is supported (models/yolo.py:75)", reg_max, CERB_REG_MAX);
     CERB_REQUIRE(n_rows >= 0 && n_rows < (1l << 40) && A >= 0, "cerb_bbox_decode_fwd: bad sizes n_rows=%ld A=%d", n_rows, A);
     if (n_rows == 0) return 0;
@@ -559,7 +565,7 @@ extern "C" int cerb_bbox_decode_fwd(const void* pred_dist, const void* anchor_po
 extern "C" int cerb_bbox_decode_bwd(const void* pred_dist, const void* grad_out, long n_rows, int reg_max, int dtype,
                                     void* grad_pred_dist, void* stream) {
     cerb_clear_error();
-    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "cerb_bbox_decode_bwd: unsupported dtype %d", dtype);
+    CERB_REQUIRE(post_elt(dtype) != 0, "cerb_bbox_decode_bwd: unsupported dtype %d", dtype);
     CERB_REQUIRE(reg_max == CERB_REG_MAX, "cerb_bbox_decode_bwd: reg_max=%d, only %d is supported (models/yolo.py:75)", reg_max, CERB_REG_MAX);
     CERB_REQUIRE(n_rows >= 0 && n_rows < (1l << 40), "cerb_bbox_decode_bwd: bad n_rows=%ld", n_rows);
     if (n_rows == 0) return 0;

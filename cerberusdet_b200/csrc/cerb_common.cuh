@@ -1,5 +1,6 @@
 // Shared definitions for the cerb_post kernels (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -9,6 +10,7 @@
 #define CERB_REG_MAX 16  // DFL bins per side, reference models/yolo.py:75
 #define CERB_DTYPE_F16 0
 #define CERB_DTYPE_F32 1
+#define CERB_DTYPE_BF16 2
 
 // ---- rounding helpers: the reference computes every elementwise op in the tensor
 // dtype, i.e. for half inputs each op is "compute in fp32, round to half".  rnd<T>()
@@ -17,6 +19,7 @@ template <typename T> __device__ __forceinline__ float rnd(float v);
 template <> __device__ __forceinline__ float rnd<float>(float v) { return v; }
 // (packed convert: F2FP runs on the ALU pipes, the scalar F2F.F16.F32 on the SFU pipe the exps already load)
 template <> __device__ __forceinline__ float rnd<__half>(float v) { return __low2float(__floats2half2_rn(v, 0.f)); }
+template <> __device__ __forceinline__ float rnd<__nv_bfloat16>(float v) { return __low2float(__floats2bfloat162_rn(v, 0.f)); }
 
 // two roundings at once: for half one F2FP.PACK_AB packs both values (the compiler does not pair scalar
 // conversions by itself), for float nothing happens
@@ -27,14 +30,23 @@ template <> __device__ __forceinline__ void rnd2<__half>(float a, float b, float
     ra = f.x;
     rb = f.y;
 }
+template <> __device__ __forceinline__ void rnd2<__nv_bfloat16>(float a, float b, float& ra, float& rb) {
+    const float2 f = __bfloat1622float2(__floats2bfloat162_rn(a, b));
+    ra = f.x;
+    rb = f.y;
+}
 
 template <typename T> __device__ __forceinline__ float to_f32(T v);
 template <> __device__ __forceinline__ float to_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ float to_f32<__half>(__half v) { return __half2float(v); }
+template <> __device__ __forceinline__ float to_f32<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }
 
 template <typename T> __device__ __forceinline__ T from_f32(float v);
 template <> __device__ __forceinline__ float from_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ __half from_f32<__half>(float v) { return __low2half(__floats2half2_rn(v, 0.f)); }
+template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) {
+    return __low2bfloat16(__floats2bfloat162_rn(v, 0.f));
+}
 
 __device__ __forceinline__ float fast_ex2(float x) {
 #ifdef CERB_EXPERIMENT_NO_MUFU  // tools/ only: where does the time go without the SFU?
@@ -55,8 +67,8 @@ __device__ __forceinline__ float fast_rcp(float x) {
 #endif
 }
 
-// ---- mixed-precision FMA (sm_100a, PTX fma.rn.f32.f16 -> SASS FHFMA): d = a.f16 * b.f16 + c.f32, a and b picked
-// from the low / high half of a packed register, one rounding in fp32
+// ---- mixed-precision FMA (sm_100a, PTX fma.rn.f32.f16 -> SASS FHFMA, fma.rn.f32.bf16 -> FHFMA.BF16): d = a * b + c.f32
+// with a and b 16-bit values picked from the low / high half of a packed register, one rounding in fp32
 __device__ __forceinline__ float fhfma_lo(uint32_t a2, uint32_t b2, float c) {
     float d;
     asm("{\n\t.reg .b16 al, ah, bl, bh;\n\tmov.b32 {al, ah}, %1;\n\tmov.b32 {bl, bh}, %2;\n\t"
@@ -71,8 +83,26 @@ __device__ __forceinline__ float fhfma_hi(uint32_t a2, uint32_t b2, float c) {
         : "=f"(d) : "r"(a2), "r"(b2), "f"(c));
     return d;
 }
+__device__ __forceinline__ float fbfma_lo(uint32_t a2, uint32_t b2, float c) {
+    float d;
+    asm("{\n\t.reg .b16 al, ah, bl, bh;\n\tmov.b32 {al, ah}, %1;\n\tmov.b32 {bl, bh}, %2;\n\t"
+        "fma.rn.f32.bf16 %0, al, bl, %3;\n\t}"
+        : "=f"(d) : "r"(a2), "r"(b2), "f"(c));
+    return d;
+}
+__device__ __forceinline__ float fbfma_hi(uint32_t a2, uint32_t b2, float c) {
+    float d;
+    asm("{\n\t.reg .b16 al, ah, bl, bh;\n\tmov.b32 {al, ah}, %1;\n\tmov.b32 {bl, bh}, %2;\n\t"
+        "fma.rn.f32.bf16 %0, ah, bh, %3;\n\t}"
+        : "=f"(d) : "r"(a2), "r"(b2), "f"(c));
+    return d;
+}
 __device__ __forceinline__ uint32_t pack_half2_rn(float lo, float hi) {
     const __half2 h = __floats2half2_rn(lo, hi);
+    return *reinterpret_cast<const uint32_t*>(&h);
+}
+__device__ __forceinline__ uint32_t pack_bf162_rn(float lo, float hi) {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<const uint32_t*>(&h);
 }
 // packed half2 bit pattern of two small non-negative integers (exact in half), a compile-time constant after unrolling
@@ -88,6 +118,41 @@ __host__ __device__ constexpr uint32_t half2_bits_of_ints(int lo, int hi) {
 }
 static_assert(half_bits_of_int(1) == 0x3C00 && half_bits_of_int(3) == 0x4200 && half_bits_of_int(9) == 0x4880 &&
               half_bits_of_int(15) == 0x4B80, "half encoding of the DFL bin weights");
+// the same for bfloat16 (k in [0, 256): exact with 8 significant bits): exponent 127 + floor(log2 k), 7 mantissa bits
+__host__ __device__ constexpr uint32_t bf16_bits_of_int(int k) {
+    if (k == 0) return 0u;
+    int e = 0;
+    for (int t = k; t > 1; t >>= 1) ++e;
+    return (uint32_t)((127 + e) << 7) | (((uint32_t)k << (7 - e)) & 0x7Fu);
+}
+__host__ __device__ constexpr uint32_t bf162_bits_of_ints(int lo, int hi) {
+    return bf16_bits_of_int(lo) | (bf16_bits_of_int(hi) << 16);
+}
+static_assert(bf16_bits_of_int(1) == 0x3F80 && bf16_bits_of_int(3) == 0x4040 && bf16_bits_of_int(9) == 0x4110 &&
+              bf16_bits_of_int(15) == 0x4170, "bfloat16 encoding of the DFL bin weights");
+
+// The packed forms of the two 16-bit tensor dtypes, for code that is written once for both: Pair<T>::type is the
+// two-lane vector type, pack2_rn rounds two floats into one, mixfma_lo / _hi is the mixed-precision FMA on a lane and
+// bits2_of_ints the packed pattern of two small integers.
+template <typename T> struct Pair;
+template <> struct Pair<__half> {
+    typedef __half2 type;
+    static __device__ __forceinline__ uint32_t pack2_rn(float lo, float hi) { return pack_half2_rn(lo, hi); }
+    static __device__ __forceinline__ __half2 splat(float v) { return __float2half2_rn(v); }
+    static __device__ __forceinline__ __half2 of_floats(float lo, float hi) { return __floats2half2_rn(lo, hi); }
+    static __device__ __forceinline__ float mixfma_lo(uint32_t a2, uint32_t b2, float c) { return fhfma_lo(a2, b2, c); }
+    static __device__ __forceinline__ float mixfma_hi(uint32_t a2, uint32_t b2, float c) { return fhfma_hi(a2, b2, c); }
+    static __host__ __device__ constexpr uint32_t bits2_of_ints(int lo, int hi) { return half2_bits_of_ints(lo, hi); }
+};
+template <> struct Pair<__nv_bfloat16> {
+    typedef __nv_bfloat162 type;
+    static __device__ __forceinline__ uint32_t pack2_rn(float lo, float hi) { return pack_bf162_rn(lo, hi); }
+    static __device__ __forceinline__ __nv_bfloat162 splat(float v) { return __float2bfloat162_rn(v); }
+    static __device__ __forceinline__ __nv_bfloat162 of_floats(float lo, float hi) { return __floats2bfloat162_rn(lo, hi); }
+    static __device__ __forceinline__ float mixfma_lo(uint32_t a2, uint32_t b2, float c) { return fbfma_lo(a2, b2, c); }
+    static __device__ __forceinline__ float mixfma_hi(uint32_t a2, uint32_t b2, float c) { return fbfma_hi(a2, b2, c); }
+    static __host__ __device__ constexpr uint32_t bits2_of_ints(int lo, int hi) { return bf162_bits_of_ints(lo, hi); }
+};
 
 // ---- packed fp32 pairs (sm_100a: PTX fma.rn.f32x2 / add.rn.f32x2 / mul.rn.f32x2 -> SASS FFMA2 / FADD2 / FMUL2): two
 // IEEE fp32 operations (each rounded exactly like the scalar instruction) for one issue slot.  The decode kernels are
@@ -135,6 +200,7 @@ __device__ __forceinline__ float2 fmul2(float2 a, float2 b) {
 // weighted sum are short trees / 4 partial sums (instruction-level parallelism instead of three 16-long
 // dependency chains); the scale-and-shift before the exponentials, the sum and the normalisation run on
 // packed fp32 pairs (bins k, k+1).  dfl_expectation_acc returns the fp32 accumulator BEFORE its final rounding.
+// bfloat16 follows the same rules with bf16 in place of half.
 #define CERB_LOG2E 1.4426950408889634f
 template <typename T> __device__ __forceinline__ float dfl_expectation_acc(float (&x)[CERB_REG_MAX]) {
 #ifdef CERB_EXPERIMENT_COPY_ONLY  // tools/ only: memory floor of this access pattern
@@ -162,17 +228,18 @@ template <typename T> __device__ __forceinline__ float dfl_expectation_acc(float
     float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
 #ifndef CERB_NO_FHFMA
     if constexpr (sizeof(T) == 2) {
-        // half: the rounded probabilities stay packed and feed the mixed-precision FMA (FHFMA: f16 x f16 + f32, one
-        // rounding) -- the same value as fmaf((float)k, (float)p, acc) without the two unpacking converts per pair
+        // half / bf16: the rounded probabilities stay packed and feed the mixed-precision FMA (FHFMA: f16 x f16 + f32,
+        // one rounding) -- the same value as fmaf((float)k, (float)p, acc) without the two unpacking converts per pair
+        typedef Pair<T> P2;
 #pragma unroll
         for (int k = 0; k < CERB_REG_MAX; k += 4) {
             const float2 q01 = fmul2(e[k / 2], inv2), q23 = fmul2(e[k / 2 + 1], inv2);
-            const uint32_t p01 = pack_half2_rn(q01.x, q01.y);
-            const uint32_t p23 = pack_half2_rn(q23.x, q23.y);
-            if (k != 0) a0 = fhfma_lo(p01, half2_bits_of_ints(k, k + 1), a0);  // 0 * p0 + 0 == +0
-            a1 = fhfma_hi(p01, half2_bits_of_ints(k, k + 1), a1);
-            a2 = fhfma_lo(p23, half2_bits_of_ints(k + 2, k + 3), a2);
-            a3 = fhfma_hi(p23, half2_bits_of_ints(k + 2, k + 3), a3);
+            const uint32_t p01 = P2::pack2_rn(q01.x, q01.y);
+            const uint32_t p23 = P2::pack2_rn(q23.x, q23.y);
+            if (k != 0) a0 = P2::mixfma_lo(p01, P2::bits2_of_ints(k, k + 1), a0);  // 0 * p0 + 0 == +0
+            a1 = P2::mixfma_hi(p01, P2::bits2_of_ints(k, k + 1), a1);
+            a2 = P2::mixfma_lo(p23, P2::bits2_of_ints(k + 2, k + 3), a2);
+            a3 = P2::mixfma_hi(p23, P2::bits2_of_ints(k + 2, k + 3), a3);
         }
         return (a0 + a1) + (a2 + a3);
     } else

@@ -141,6 +141,13 @@ cudaError_t cerb_launch_decode(DecodeParams& P, int dtype, int vec, cudaStream_t
             case 2: return launch_decode_t<__half, 2>(P, stream);
             default: return launch_decode_t<__half, 1>(P, stream);
         }
+    } else if (dtype == CERB_DTYPE_BF16) {
+        switch (vec) {
+            case 8: return launch_decode_t<__nv_bfloat16, 8>(P, stream);
+            case 4: return launch_decode_t<__nv_bfloat16, 4>(P, stream);
+            case 2: return launch_decode_t<__nv_bfloat16, 2>(P, stream);
+            default: return launch_decode_t<__nv_bfloat16, 1>(P, stream);
+        }
     } else {
         switch (vec) {
             case 4: return launch_decode_t<float, 4>(P, stream);

@@ -48,6 +48,11 @@ template <> __device__ __forceinline__ __half pack_max<__half, 8>(const Pack<__h
     const __half2 m = __hmax2(__hmax2(h[0], h[1]), __hmax2(h[2], h[3]));
     return __hmax(__low2half(m), __high2half(m));
 }
+template <> __device__ __forceinline__ __nv_bfloat16 pack_max<__nv_bfloat16, 8>(const Pack<__nv_bfloat16, 8>& v) {
+    const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&v.raw);
+    const __nv_bfloat162 m = __hmax2(__hmax2(h[0], h[1]), __hmax2(h[2], h[3]));
+    return __hmax(__low2bfloat16(m), __high2bfloat16(m));
+}
 template <> __device__ __forceinline__ float pack_max<float, 4>(const Pack<float, 4>& v) {
     return fmaxf(fmaxf(v.e[0], v.e[1]), fmaxf(v.e[2], v.e[3]));
 }
@@ -55,9 +60,9 @@ template <typename T, int VEC> __device__ __forceinline__ T pack_max(const Pack<
 
 // Expected DFL distances of one box side for VEC anchors: sum_k k * softmax(logits)_k (reference DFL.forward,
 // models/yolo.py:57-59).  Rounding points follow the reference for half tensors: probabilities are rounded to
-// half (softmax output), the 1x1 conv accumulates in fp32 and rounds once.
-// DVec holds the VEC rounded distances: as floats, or -- half tensors, even VEC -- as packed half2 pairs (anchors
-// i, i+1), so that the rounding of two anchors is ONE F2FP.PACK_AB and the box arithmetic after it runs on half2.
+// half (softmax output), the 1x1 conv accumulates in fp32 and rounds once; bfloat16 tensors likewise in bf16.
+// DVec holds the VEC rounded distances: as floats, or -- 16-bit tensors, even VEC -- as packed half2 / bfloat162 pairs
+// (anchors i, i+1), so that the rounding of two anchors is ONE F2FP.PACK_AB and the box arithmetic after it runs on pairs.
 #ifndef CERB_HALF2_EPILOGUE
 #define CERB_HALF2_EPILOGUE 1
 #endif
@@ -85,7 +90,7 @@ __device__ __forceinline__ void dfl_reduce(const Pack<T, VEC> (&v)[CERB_REG_MAX]
             }
             const float e0 = dfl_expectation_acc<T>(x0);
             const float e1 = dfl_expectation_acc<T>(x1);
-            d.h2[i / 2] = pack_half2_rn(e0, e1);
+            d.h2[i / 2] = Pair<T>::pack2_rn(e0, e1);
         }
     } else {
 #pragma unroll
@@ -111,24 +116,28 @@ __device__ __forceinline__ void dfl_side(const T* __restrict__ side_base, int hw
 // add/sub/mul IS "compute exactly, round once to half", and the operands here (|value| < 2^16, products by powers of
 // two or of two halves) never differ from the reference's "fp32 operation, then round to half" except on a tie that
 // only appears after the fp32 rounding -- which needs an operand below 2^-13 of the other AND an exact midpoint.
+// bfloat16 tensors run the same chain on bfloat162 pairs, with no exception: fp32 carries 24 >= 2 * 8 + 2 significant
+// bits, so rounding the fp32 result of an add/sub/mul to bf16 always equals the single rounding of the exact result.
+// The anchor centres round too: bf16(k) + 0.5 is exact only below 128 (128.5 -> 128, 129.5 -> 130), as in the reference.
 template <typename T, int VEC>
 __device__ __forceinline__ void axis_boxes(const DVec<T, VEC>& dlo, const DVec<T, VEC>& dhi, int a0, int W, bool x_axis, float st,
                                            Pack<T, VEC>& centre, Pack<T, VEC>& size) {
     int gx = a0 % W, gy = a0 / W;  // one division per thread; the VEC anchors then walk the grid row by row
     if constexpr (DVecTraits<T, VEC>::packed) {
-        const __half2 half = __float2half2_rn(0.5f), st2 = __float2half2_rn(st);
-        __half2* oc = reinterpret_cast<__half2*>(&centre.raw);
-        __half2* os = reinterpret_cast<__half2*>(&size.raw);
+        typedef typename Pair<T>::type T2;
+        const T2 half = Pair<T>::splat(0.5f), st2 = Pair<T>::splat(st);
+        T2* oc = reinterpret_cast<T2*>(&centre.raw);
+        T2* os = reinterpret_cast<T2*>(&size.raw);
 #pragma unroll
         for (int i = 0; i < VEC; i += 2) {
             const int g0 = x_axis ? gx : gy;
             if (++gx >= W) { gx = 0; ++gy; }
             const int g1 = x_axis ? gx : gy;
             if (++gx >= W) { gx = 0; ++gy; }
-            const __half2 ac = __hadd2(__floats2half2_rn((float)g0, (float)g1), half);
-            const __half2 lo = *reinterpret_cast<const __half2*>(&dlo.h2[i / 2]);
-            const __half2 hi = *reinterpret_cast<const __half2*>(&dhi.h2[i / 2]);
-            const __half2 p1 = __hsub2(ac, lo), p2 = __hadd2(ac, hi);
+            const T2 ac = __hadd2(Pair<T>::of_floats((float)g0, (float)g1), half);
+            const T2 lo = *reinterpret_cast<const T2*>(&dlo.h2[i / 2]);
+            const T2 hi = *reinterpret_cast<const T2*>(&dhi.h2[i / 2]);
+            const T2 p1 = __hsub2(ac, lo), p2 = __hadd2(ac, hi);
             oc[i / 2] = __hmul2(__hmul2(__hadd2(p1, p2), half), st2);
             os[i / 2] = __hmul2(__hsub2(p2, p1), st2);
         }
@@ -155,7 +164,7 @@ template <typename T, int VEC> __device__ __forceinline__ void sigmoid_pack(Pack
         for (int i = 0; i < VEC; i += 2) {
             const float2 s = sigmoid2(make_float2(to_f32<T>(v.e[i]), to_f32<T>(v.e[i + 1])));
             if constexpr (sizeof(T) == 2) {
-                reinterpret_cast<uint32_t*>(&v.raw)[i / 2] = pack_half2_rn(s.x, s.y);
+                reinterpret_cast<uint32_t*>(&v.raw)[i / 2] = Pair<T>::pack2_rn(s.x, s.y);
             } else {
                 v.e[i] = from_f32<T>(s.x);
                 v.e[i + 1] = from_f32<T>(s.y);

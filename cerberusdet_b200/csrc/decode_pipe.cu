@@ -268,7 +268,7 @@ template <typename T, int VEC, int IPT, int CIPT> static cudaError_t launch_pipe
 }
 
 // Items per thread (DFL rows, class rows) of the shipped instantiations: fp16 2 / PIPE_CIPT_F16, fp32 1 / 1
-// (profiles/r02_decode.md).  -DCERB_DECODE_VARIANTS also builds the other combinations for tools/ A/B runs
+// (profiles/r02_decode.md); bf16 takes fp16's (it moves the same bytes and runs the same packed arithmetic).  -DCERB_DECODE_VARIANTS also builds the other combinations for tools/ A/B runs
 // (ipt = 10 * IPT + CIPT selects one).
 #ifndef PIPE_IPT_F16
 #define PIPE_IPT_F16 2
@@ -291,6 +291,8 @@ cudaError_t cerb_launch_decode_pipe(const DecodeParams& P, int dtype, int ipt, c
             default: return launch_pipe_t<__half, 8, PIPE_IPT_F16, PIPE_CIPT_F16>(P, stream);
         }
     }
+    if (dtype == CERB_DTYPE_BF16) return ipt == 0 ? cudaErrorInvalidConfiguration
+                                                  : launch_pipe_t<__nv_bfloat16, 8, PIPE_IPT_F16, PIPE_CIPT_F16>(P, stream);
     switch (ipt) {
 #ifdef CERB_DECODE_VARIANTS
         case 21: return launch_pipe_t<float, 4, 2, 1>(P, stream);

@@ -10,7 +10,9 @@
 //    passes the threshold (multi-label, :444-446) or the best class of an anchor
 //    (:447-449).  Each gets a unique 64-bit key  score_bits << 32 | ~(a*nc + c), so that
 //    descending key order == "score descending, candidate index ascending", the
-//    canonical form of the reference's sort at :459 (ties there are unspecified).
+//    canonical form of the reference's sort at :459 (ties there are unspecified).  score_bits
+//    are the fp32 bits of the score: a half or bfloat16 score widens exactly (bf16: its own
+//    bits << 16), and the non-negative sigmoid outputs order as unsigned integers.
 //  * Greedy NMS is order-causal and stops at max_det (:465), so only a prefix of the
 //    sorted order is ever needed.  A 2048-bin histogram of the top 12 key bits locates
 //    successive chunks of <= CAP keys; each chunk is gathered, bitonic-sorted (registers +
@@ -220,6 +222,7 @@ template <typename T> __host__ __device__ __forceinline__ size_t summary_row_len
 template <typename T> struct RangeBounds;
 template <> struct RangeBounds<float> { unsigned lo, span; };
 template <> struct RangeBounds<__half> { __half2 lo2, hi2; };
+template <> struct RangeBounds<__nv_bfloat16> { __nv_bfloat162 lo2, hi2; };
 template <typename T> __device__ __forceinline__ RangeBounds<T> make_range_bounds(unsigned sb_lo, unsigned sb_hi);
 template <> __device__ __forceinline__ RangeBounds<float> make_range_bounds<float>(unsigned sb_lo, unsigned sb_hi) {
     RangeBounds<float> r;
@@ -232,6 +235,14 @@ template <> __device__ __forceinline__ RangeBounds<__half> make_range_bounds<__h
     RangeBounds<__half> r;
     r.lo2 = __half2half2(__float2half_ru(__uint_as_float(sb_lo)));
     r.hi2 = __half2half2(__float2half_rd(__uint_as_float(sb_hi)));
+    return r;
+}
+template <>
+__device__ __forceinline__ RangeBounds<__nv_bfloat16> make_range_bounds<__nv_bfloat16>(unsigned sb_lo, unsigned sb_hi) {
+    // smallest bf16 >= lo and largest bf16 <= hi, as for half
+    RangeBounds<__nv_bfloat16> r;
+    r.lo2 = __bfloat162bfloat162(__float2bfloat16_ru(__uint_as_float(sb_lo)));
+    r.hi2 = __bfloat162bfloat162(__float2bfloat16_rd(__uint_as_float(sb_hi)));
     return r;
 }
 // bit k set iff element k of the vector has its score bits in [sb_lo, sb_hi]
@@ -247,6 +258,19 @@ __device__ __forceinline__ unsigned range_hits<float>(const ScoreVec<float>& v, 
 template <>
 __device__ __forceinline__ unsigned range_hits<__half>(const ScoreVec<__half>& v, unsigned, unsigned, const RangeBounds<__half>& rb) {
     const __half2* h2 = reinterpret_cast<const __half2*>(&v.raw);
+    unsigned m[4], any = 0;
+#pragma unroll
+    for (int p = 0; p < 4; ++p) { m[p] = __hge2_mask(h2[p], rb.lo2) & __hle2_mask(h2[p], rb.hi2); any |= m[p]; }
+    if (!any) return 0u;
+    unsigned h = 0;
+#pragma unroll
+    for (int p = 0; p < 4; ++p) h |= ((m[p] & 1u) | ((m[p] >> 15) & 2u)) << (2 * p);
+    return h;
+}
+template <>
+__device__ __forceinline__ unsigned range_hits<__nv_bfloat16>(const ScoreVec<__nv_bfloat16>& v, unsigned, unsigned,
+                                                               const RangeBounds<__nv_bfloat16>& rb) {
+    const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&v.raw);
     unsigned m[4], any = 0;
 #pragma unroll
     for (int p = 0; p < 4; ++p) { m[p] = __hge2_mask(h2[p], rb.lo2) & __hle2_mask(h2[p], rb.hi2); any |= m[p]; }
@@ -1299,5 +1323,7 @@ cudaError_t cerb_launch_nms(const NmsParams& P, int dtype, cudaStream_t stream) 
     const bool multi = P.multi_label != 0;
     if (dtype == CERB_DTYPE_F16)
         return multi ? launch_nms_v<__half, true>(P, stream) : launch_nms_v<__half, false>(P, stream);
+    if (dtype == CERB_DTYPE_BF16)
+        return multi ? launch_nms_v<__nv_bfloat16, true>(P, stream) : launch_nms_v<__nv_bfloat16, false>(P, stream);
     return multi ? launch_nms_v<float, true>(P, stream) : launch_nms_v<float, false>(P, stream);
 }

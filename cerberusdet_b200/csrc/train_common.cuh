@@ -27,6 +27,12 @@ template <> struct Row16<__half> {
     __device__ __forceinline__ float get(int k) const { return __half2float(reinterpret_cast<const __half*>(v)[k]); }
     __device__ __forceinline__ void set(int k, float f) { reinterpret_cast<__half*>(v)[k] = from_f32<__half>(f); }
 };
+template <> struct Row16<__nv_bfloat16> {
+    static constexpr int NV = 1;
+    U8x32 v[1];
+    __device__ __forceinline__ float get(int k) const { return __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(v)[k]); }
+    __device__ __forceinline__ void set(int k, float f) { reinterpret_cast<__nv_bfloat16*>(v)[k] = from_f32<__nv_bfloat16>(f); }
+};
 template <> struct Row16<float> {
     static constexpr int NV = 2;
     U8x32 v[2];

@@ -7,7 +7,7 @@
 // (loss.py:139-146 permutes the raw heads), so a thread owns one (anchor, side): 16 contiguous values in
 // (1 or 2 256-bit loads, a warp reads 1 KB contiguous per instruction), one value out.  Same rounding points as the
 // inference kernel for half tensors (dfl_expectation<T>): probabilities rounded to half, fp32 accumulation
-// rounded once, the corner rounded once.
+// rounded once, the corner rounded once.  bfloat16 tensors round at the same points, in bf16.
 //
 // Backward (the autograd of the three reference ops, fused): with p = softmax(x), d = sum_k k p_k and g the
 // incoming gradient of this side's corner (negated for the l, t sides: x1y1 = anchor - lt),
@@ -87,7 +87,10 @@ cudaError_t cerb_launch_bbox_decode_fwd(const void* pred, const void* anchor_poi
     if (n_sides == 0) return cudaSuccess;
     const unsigned blocks = (unsigned)((n_sides + TD_THREADS - 1) / TD_THREADS);
     const bool al = td_aligned(pred);
-    if (dtype == CERB_DTYPE_F16) {
+    if (dtype == CERB_DTYPE_BF16) {
+        if (al) bbox_decode_fwd_kernel<__nv_bfloat16, true><<<blocks, TD_THREADS, 0, stream>>>((const __nv_bfloat16*)pred, (const __nv_bfloat16*)anchor_points, n_sides, A, (__nv_bfloat16*)out);
+        else bbox_decode_fwd_kernel<__nv_bfloat16, false><<<blocks, TD_THREADS, 0, stream>>>((const __nv_bfloat16*)pred, (const __nv_bfloat16*)anchor_points, n_sides, A, (__nv_bfloat16*)out);
+    } else if (dtype == CERB_DTYPE_F16) {
         if (al) bbox_decode_fwd_kernel<__half, true><<<blocks, TD_THREADS, 0, stream>>>((const __half*)pred, (const __half*)anchor_points, n_sides, A, (__half*)out);
         else bbox_decode_fwd_kernel<__half, false><<<blocks, TD_THREADS, 0, stream>>>((const __half*)pred, (const __half*)anchor_points, n_sides, A, (__half*)out);
     } else {
@@ -103,7 +106,10 @@ cudaError_t cerb_launch_bbox_decode_bwd(const void* pred, const void* grad_out, 
     if (n_sides == 0) return cudaSuccess;
     const unsigned blocks = (unsigned)((n_sides + TD_THREADS - 1) / TD_THREADS);
     const bool al = td_aligned(pred) && td_aligned(grad_in);
-    if (dtype == CERB_DTYPE_F16) {
+    if (dtype == CERB_DTYPE_BF16) {
+        if (al) bbox_decode_bwd_kernel<__nv_bfloat16, true><<<blocks, TD_THREADS, 0, stream>>>((const __nv_bfloat16*)pred, (const __nv_bfloat16*)grad_out, n_sides, (__nv_bfloat16*)grad_in);
+        else bbox_decode_bwd_kernel<__nv_bfloat16, false><<<blocks, TD_THREADS, 0, stream>>>((const __nv_bfloat16*)pred, (const __nv_bfloat16*)grad_out, n_sides, (__nv_bfloat16*)grad_in);
+    } else if (dtype == CERB_DTYPE_F16) {
         if (al) bbox_decode_bwd_kernel<__half, true><<<blocks, TD_THREADS, 0, stream>>>((const __half*)pred, (const __half*)grad_out, n_sides, (__half*)grad_in);
         else bbox_decode_bwd_kernel<__half, false><<<blocks, TD_THREADS, 0, stream>>>((const __half*)pred, (const __half*)grad_out, n_sides, (__half*)grad_in);
     } else {

@@ -97,7 +97,7 @@ def detect_forward(self, x):
     concatenations exactly like the reference does (yolo.py:89-90).
     """
     reference_forward = type(self)._cerb_reference_forward
-    if self.training or not x[0].is_cuda or x[0].dtype not in (torch.float16, torch.float32):
+    if self.training or not x[0].is_cuda or x[0].dtype not in (torch.float16, torch.bfloat16, torch.float32):
         return reference_forward(self, x)
     shape = x[0].shape  # BCHW before the convs: the reference's anchor-cache key (yolo.py:88,93)
     if getattr(self, _RAW_FLAG, False):

@@ -142,7 +142,7 @@ class CerberusDetInference:
             else:
                 preds = decode_heads(levels, self._head_strides(len(levels[0])))
         bsz = tensor.shape[0]
-        on_path = all(p.is_cuda and p.dtype in (torch.float16, torch.float32) for p in preds)
+        on_path = all(p.is_cuda and p.dtype in (torch.float16, torch.bfloat16, torch.float32) for p in preds)
         if on_path:
             # 2. one NMS launch over all (task, image) segments
             dets, counts = nms_batched(preds, conf_thres, iou_thres, agnostic=agnostic_nms, max_det=max_det)

@@ -19,13 +19,17 @@ MAX_WH = 7680.0  # reference utils/general.py:415
 MAX_NMS = 30000  # reference utils/general.py:416
 
 _DTYPES = {torch.float16: _lib.CERB_F16, torch.float32: _lib.CERB_F32}
+# the kernels that read head-dtype tensors (decode, NMS, the training-time box decode) also take bfloat16
+_HEAD_DTYPES = {**_DTYPES, torch.bfloat16: _lib.CERB_BF16}
 
 
-def _dtype_code(t: torch.Tensor) -> int:
+def _dtype_code(t: torch.Tensor, head: bool = False) -> int:
+    """The C ABI dtype code of ``t``: float16 / float32, and bfloat16 too with ``head=True``; else ``TypeError``."""
     try:
-        return _DTYPES[t.dtype]
+        return (_HEAD_DTYPES if head else _DTYPES)[t.dtype]
     except KeyError:
-        raise TypeError(f"cerberusdet_b200 supports float16 and float32 tensors, got {t.dtype}") from None
+        kinds = "float16, bfloat16 and float32" if head else "float16 and float32"
+        raise TypeError(f"cerberusdet_b200 supports {kinds} tensors, got {t.dtype}") from None
 
 
 def _require_cuda(t: torch.Tensor, what: str) -> None:
@@ -78,7 +82,7 @@ def _dense_heads(levels: Sequence[torch.Tensor], nc: Sequence[int], strides: Seq
         raise ValueError(f"expected {L} strides, got {len(strides)}")
     first = levels[0]
     _require_cuda(first, "head tensors")
-    code = _dtype_code(first)
+    code = _dtype_code(first, head=True)
     B = int(first.shape[0])
     H = [int(levels[l].shape[2]) for l in range(L)]
     W = [int(levels[l].shape[3]) for l in range(L)]
@@ -199,7 +203,7 @@ def _nms_impl(
     T = len(preds)
     first = preds[0]
     _require_cuda(first, "prediction")
-    code = _dtype_code(first)
+    code = _dtype_code(first, head=True)
     B, A = int(first.shape[0]), int(first.shape[2])
     ncs, ps = [], []
     for p in preds:
@@ -716,7 +720,7 @@ class _BboxDecode(torch.autograd.Function):
             raise ValueError(f"anchor_points must be [{A}, 2], got {tuple(anchor_points.shape)}")
         if anchor_points.device != pred_dist.device:
             raise TypeError("anchor_points and pred_dist must be on the same device")
-        code = _dtype_code(pred_dist)
+        code = _dtype_code(pred_dist, head=True)
         x = pred_dist.contiguous()
         ap = anchor_points.to(pred_dist.dtype).contiguous()
         out = torch.empty((B, A, 4), dtype=pred_dist.dtype, device=pred_dist.device)

@@ -13,8 +13,10 @@ What gets rebound (and restored by ``uninstall()``):
   computes the loss under ``amp.autocast`` (trainers/averaging.py:158): there ``softmax`` runs in fp32 on the fp16
   ``pred_dist``, autocast rounds its output to fp16 for the ``matmul`` with ``proj`` (fp32 accumulation, fp16 result) and
   ``dist2bbox`` stays in fp16 -- exactly the half path of the kernels (probabilities rounded to half, one rounding of
-  the expectation, one per corner), so fp16 ``pred_dist`` + fp16 anchors under autocast go to the kernels; any other
-  dtype mix (fp32 under autocast, anchors of another dtype) keeps the reference's own code;
+  the expectation, one per corner), so fp16 ``pred_dist`` + fp16 anchors under autocast go to the kernels.  bf16
+  autocast is the same with bf16 in place of fp16, so bf16 ``pred_dist`` + bf16 anchors go to the kernels' bf16 path,
+  with or without autocast; any other dtype mix (fp32 under autocast, a ``pred_dist`` dtype other than the autocast
+  dtype, anchors of another dtype) keeps the reference's own code;
 * with ``loss=True`` ``cerberusdet.utils.loss.BboxLoss.forward`` -> ``ops.bbox_loss`` (the box-regression term the loss
   computes right after the assigner, reference utils/loss.py:12-44: CIoU + DFL in one forward and one backward kernel, no
   host synchronisation).  On the path: ``use_dfl`` with 16 bins, CUDA tensors, and either everything fp32 without
@@ -33,9 +35,9 @@ What gets rebound (and restored by ``uninstall()``):
   ``detections=None``, CPU or non-fp32 tensors, more than 30000 detections or 1024 labels and classes outside
   ``[0, nc)`` keep the reference's own method.
 
-CUDA fp16/fp32 tensors go to the kernels; anything else (CPU tensors, training mode, masks/labels
-arguments) is handed to the reference's own, saved implementation -- the patch never changes what a
-non-CUDA run computes.
+CUDA fp16/fp32 tensors (and bf16 ones for the decode, the NMS and ``Loss.bbox_decode``) go to the kernels; anything
+else (CPU tensors, training mode, masks/labels arguments) is handed to the reference's own, saved implementation --
+the patch never changes what a non-CUDA run computes.
 """
 from __future__ import annotations
 
@@ -100,7 +102,8 @@ def install(import_all: bool = False, train: bool = False, val: bool = False, lo
         def non_max_suppression(prediction, conf_thres=0.25, iou_thres=0.45, classes=None, agnostic=False,
                                 multi_label=False, labels=(), max_det=300, nm=0):
             p = prediction[0] if isinstance(prediction, (list, tuple)) else prediction
-            on_path = p.is_cuda and p.dtype in (torch.float16, torch.float32) and not nm and not (labels is not None and len(labels))
+            on_path = (p.is_cuda and p.dtype in (torch.float16, torch.bfloat16, torch.float32) and not nm
+                       and not (labels is not None and len(labels)))
             if not on_path:
                 return reference_nms(prediction, conf_thres, iou_thres, classes, agnostic, multi_label, labels, max_det, nm)
             return _nms.non_max_suppression(prediction, conf_thres, iou_thres, classes, agnostic, multi_label, labels, max_det, nm)
@@ -131,10 +134,12 @@ def install(import_all: bool = False, train: bool = False, val: bool = False, lo
                 on_path = (self.use_dfl and pred_dist.is_cuda and pred_dist.dim() == 3 and pred_dist.shape[-1] == 64
                            and anchor_points.dtype == pred_dist.dtype)
                 if on_path and torch.is_autocast_enabled():
-                    # autocast: fp32 softmax -> fp16 probabilities -> fp16 matmul (fp32 accumulate): the kernels' half path
-                    on_path = pred_dist.dtype == torch.float16 and torch.get_autocast_dtype("cuda") == torch.float16
+                    # autocast: fp32 softmax -> fp16 (bf16) probabilities -> fp16 (bf16) matmul (fp32 accumulate): the
+                    # kernels' half (bf16) path, when pred_dist already has the autocast dtype
+                    on_path = (pred_dist.dtype in (torch.float16, torch.bfloat16)
+                               and torch.get_autocast_dtype("cuda") == pred_dist.dtype)
                 elif on_path:
-                    on_path = pred_dist.dtype in (torch.float16, torch.float32)
+                    on_path = pred_dist.dtype in (torch.float16, torch.bfloat16, torch.float32)
                 if not on_path:  # CPU tensors, reg_max != 16, mixed dtypes: the reference's own code
                     return reference_bbox_decode(self, anchor_points, pred_dist)
                 return _ops.bbox_decode(anchor_points, pred_dist)

@@ -17,7 +17,11 @@
  *    different streams: the only mutable state (last error, test knobs) is thread-local.
  *  - Return 0 on success, a negative CERB_E* code otherwise; cerb_last_error() gives the
  *    calling thread's message.  There is no CPU fallback.
- *  - dtype: CERB_F16 (IEEE half) or CERB_F32; tensors are contiguous.
+ *  - dtype: CERB_F16 (IEEE half) or CERB_F32; tensors are contiguous.  CERB_BF16 (bfloat16) is
+ *    accepted by the entry points that read head-dtype tensors: cerb_decode, cerb_decode_split,
+ *    cerb_nms (and its _stats / _deliver forms), cerb_decode_nms, cerb_summary_row_len,
+ *    cerb_bbox_decode_fwd and cerb_bbox_decode_bwd.  Every other entry point rejects it.
+ *    bf16 tensors round at the same points as half ones, in bf16 (see each prototype).
  */
 #ifndef CERB_POST_H
 #define CERB_POST_H
@@ -29,6 +33,7 @@ extern "C" {
 
 #define CERB_F16 0
 #define CERB_F32 1
+#define CERB_BF16 2
 
 #define CERB_MAX_TASKS_ABI 8
 #define CERB_MAX_LEVELS_ABI 4
@@ -54,6 +59,8 @@ const char* cerb_last_error(void);
  *   y[t]          output [B, 4 + nc[t], A], A = sum_l H[l]*W[l]; rows cx, cy, w, h (pixels),
  *                 then sigmoid class scores -- the layout Detect.forward returns.
  *   strides[l]    pixel stride of level l (8, 16, 32 for P3..P5).
+ * fp16 / bf16: every elementwise step rounds to the tensor dtype where the reference's does; for bf16 that includes
+ * the anchor centres, bf16(k) + 0.5, which are exact only below 128 (128.5 -> 128, 129.5 -> 130, ties to even).
  */
 int cerb_decode(const void* const* lvl, const int* nc, int T, int L, int B, const int* H, const int* W,
                 const float* strides, int dtype, void* const* y, void* const* smax, int* summary_written,
@@ -98,12 +105,13 @@ int cerb_head_tail(const void* const* box_feat, const void* const* cls_feat, con
  * Score summary (optional by-product of cerb_decode, optional input of cerb_nms).
  *   smax[t]   [B, nc[t], R] in the tensor dtype, R = cerb_summary_row_len(A, dtype): entry (b, c, i) is
  *             the maximum of the 16-byte score vector i of class c, i.e. of the scores of anchors
- *             [i*V, i*V+V), V = 8 (fp16) / 4 (fp32); rows are padded to a multiple of V entries.
+ *             [i*V, i*V+V), V = 8 (fp16, bf16) / 4 (fp32); rows are padded to a multiple of V entries.
  * cerb_decode fills it when `smax` is non-NULL and the tensors allow the 128-bit path (every
  * H[l]*W[l] a multiple of V, 16-byte aligned pointers) and then sets *summary_written = 1.
  * cerb_nms uses it only to skip score vectors that cannot hold a candidate; results are identical
  * with and without it.  It must describe exactly the `pred` passed.
  */
+/* R for A anchors; 0 when A is not a positive multiple of V or dtype is not CERB_F16 / CERB_BF16 / CERB_F32. */
 size_t cerb_summary_row_len(int A, int dtype);
 
 /* Bytes of device workspace cerb_nms / cerb_decode_nms need (0 unless max_det is large). */
@@ -120,7 +128,8 @@ size_t cerb_nms_workspace_bytes(int T, int B, int max_det);
  *
  *   pred[t]     [B, 4 + nc[t], A] prediction of task t (what Detect.forward returns)
  *   conf_thres, iou_thres   the Python floats; rounded inside exactly as torch does
- *               (conf to the tensor dtype; IoU quotient compared in double)
+ *               (conf to the tensor dtype -- for bf16 double -> float -> bf16, so 0.3 becomes
+ *               0.30078125; IoU quotient compared in double)
  *   classes     optional host list of class ids to keep (NULL / 0 = all)
  *   max_nms     30000 in the reference (:416); max_wh 7680 (:415)
  *   smax        optional score summaries from cerb_decode for exactly these predictions, or NULL
@@ -278,11 +287,11 @@ int cerb_confusion_matrix(const float* dets, const int* counts, int B, int max_d
  * softmax over the reg_max bins of each side, expectation with proj = arange(reg_max), then
  * dist2bbox(xywh=False) (cerberusdet/utils/tal.py:196-205).
  *
- *   pred_dist       [n_rows, 4 * reg_max], n_rows = B * A, the bins of a side contiguous (loss.py:139-146), fp16 | fp32
+ *   pred_dist       [n_rows, 4 * reg_max], n_rows = B * A, the bins of a side contiguous (loss.py:139-146), fp16 | bf16 | fp32
  *   anchor_points   [A, 2] (x, y) in grid units, same dtype (make_anchors, tal.py:181-193)
  *   out             [n_rows, 4] = (x1, y1, x2, y2) in grid units, same dtype
- * reg_max must be 16 (models/yolo.py:75).  Half tensors round where the reference's do (softmax output, the
- * expectation, the corner).
+ * reg_max must be 16 (models/yolo.py:75).  Half and bf16 tensors round where the reference's do (softmax output, the
+ * expectation, the corner), in their own dtype; bf16 autocast gives the same rounding points as a bf16 model.
  */
 int cerb_bbox_decode_fwd(const void* pred_dist, const void* anchor_points, long n_rows, int A, int reg_max, int dtype,
                          void* out, void* stream);
