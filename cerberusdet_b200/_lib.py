@@ -69,7 +69,12 @@ EXPORTS = tuple(PROTOTYPES)
 
 
 class CerbLibraryError(RuntimeError):
-    pass
+    """A library call failed; ``code`` is its C return code (``CERB_ECUDA``, ``CERB_ENOSPC``, ...) or None when the
+    error was raised on the Python side."""
+
+    def __init__(self, msg: str, code=None):
+        super().__init__(msg)
+        self.code = code
 
 
 def load() -> ctypes.CDLL:
@@ -113,7 +118,7 @@ def check(rc: int) -> None:
         raise AssertionError(msg)  # reference: `assert 0 <= conf_thres <= 1` (utils/general.py:399-400)
     if rc == CERB_EINVAL:
         raise ValueError(msg)
-    raise CerbLibraryError(f"libcerb_post error {rc}: {msg}")
+    raise CerbLibraryError(f"libcerb_post error {rc}: {msg}", code=rc)
 
 
 def int_array(values):

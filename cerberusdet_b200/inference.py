@@ -16,6 +16,7 @@ from typing import Dict, List, Optional, Sequence, Tuple, Union
 import torch
 
 from . import cross_task
+from ._lib import CERB_ENOSPC, CerbLibraryError
 from .detect import _FUSE_FLAG, _RAW_FLAG, FusedHeads, SplitHeads, head_strides
 from .ops import cross_task_merge, decode_heads, decode_heads_split, head_tail, nms_batched
 
@@ -131,11 +132,22 @@ class CerberusDetInference:
             levels = [all_out[t][1] for t in tasks]
             if any(isinstance(lv, FusedHeads) for lv in levels) and not all(isinstance(lv, FusedHeads) for lv in levels):
                 levels = [lv.to_split() if isinstance(lv, FusedHeads) else lv for lv in levels]
+            fused = None
             if all(isinstance(lv, FusedHeads) for lv in levels):  # last 1x1 convs + concat + decode in one kernel
                 strides = self._head_strides(len(levels[0].box_feat))
                 w = [lv.weights() for lv in levels]
-                preds = head_tail([lv.box_feat for lv in levels], [lv.cls_feat for lv in levels], [x[0] for x in w],
-                                  [x[1] for x in w], [x[2] for x in w], [x[3] for x in w], strides)
+                try:
+                    fused = head_tail([lv.box_feat for lv in levels], [lv.cls_feat for lv in levels], [x[0] for x in w],
+                                      [x[1] for x in w], [x[2] for x in w], [x[3] for x in w], strides)
+                except CerbLibraryError as exc:
+                    # the weights and two ring stages of the launch do not fit shared memory (wide c3 at large nc).
+                    # That depends on every head of the launch, so the kernel decides; these heads run unfused from now on
+                    if exc.code != CERB_ENOSPC:
+                        raise
+                    self.fuse_head_tail = False
+                    levels = [lv.to_split() for lv in levels]
+            if fused is not None:
+                preds = fused
             elif all(isinstance(lv, SplitHeads) for lv in levels):  # patched heads: no channel concat was made
                 strides = self._head_strides(len(levels[0].box))
                 preds = decode_heads_split([lv.box for lv in levels], [lv.cls for lv in levels], strides)
