@@ -17,6 +17,8 @@
 // rounds w1, h1 (twice), w1 * h1, w1 / h1 and atan(w1 / h1) to half, everything that meets a target coordinate is fp32,
 // and the cross-entropy's log_softmax keeps the half dtype (fp32 inside, output rounded to half) before nll_loss reads it
 // in fp32 -- what autocast does with F.cross_entropy on half logits, measured against the reference on the B200.
+// bf16 mode is the trainer's bf16 autocast case: autocast's op lists do not depend on the dtype, so the rounding points are
+// the half mode's with bf16 in place of half (checked against the loss run under bf16 autocast on the B200).
 // The backward follows autograd's conventions: alpha = v / (v - iou + 1 + eps) is a constant (computed under no_grad), minimum / maximum split
 // the gradient in half on exact ties, clamp(min=0) passes it at exactly 0, the gradient of a half intermediate is rounded
 // to half where autograd keeps it as a half tensor, and the cross-entropy gradient is (softmax - onehot) in fp32.
@@ -48,6 +50,14 @@ template <> struct BoxT<__half> {
         const uint2 u = reinterpret_cast<const uint2*>(p)[row];
         const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&u.x));
         const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+        return make_float4(a.x, a.y, b.x, b.y);
+    }
+};
+template <> struct BoxT<__nv_bfloat16> {
+    static __device__ __forceinline__ float4 load(const void* p, long row) {
+        const uint2 u = reinterpret_cast<const uint2*>(p)[row];
+        const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.x));
+        const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.y));
         return make_float4(a.x, a.y, b.x, b.y);
     }
 };
@@ -332,12 +342,12 @@ static int bl_params(const char* fn, const void* pred_dist, const void* pred_bbo
                      const float* tss_dev, double tss_host, int B, int A, int C, int reg_max, int dtype, BboxLossParams& P) {
     cerb_clear_error();
     CERB_REQUIRE(reg_max == CERB_REG_MAX, "%s: reg_max=%d bins, only %d is supported (loss.py:96, BboxLoss(m.reg_max - 1))", fn, reg_max, CERB_REG_MAX);
-    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_F32, "%s: unsupported dtype %d", fn, dtype);
+    CERB_REQUIRE(dtype == CERB_F16 || dtype == CERB_BF16 || dtype == CERB_F32, "%s: unsupported dtype %d", fn, dtype);
     CERB_REQUIRE(B >= 0 && A >= 0 && C >= 1, "%s: bad sizes B=%d A=%d C=%d", fn, B, A, C);
     CERB_REQUIRE((long long)B * A <= 0x7fffffffLL && (long long)B * A * C <= (1LL << 40), "%s: B*A overflows (B=%d A=%d C=%d)", fn, B, A, C);
     if ((long long)B * A > 0) {
         CERB_REQUIRE(pred_dist && pred_bboxes && anchor_points && target_bboxes && target_scores && fg_mask, "%s: null argument", fn);
-        const size_t e = dtype == CERB_F16 ? 2 : 4;
+        const size_t e = dtype == CERB_F32 ? 4 : 2;
         CERB_REQUIRE(cerb_aligned(pred_dist, 32) && cerb_aligned(pred_bboxes, 4 * e) && cerb_aligned(anchor_points, e) &&
                          cerb_aligned(target_bboxes, 16) && cerb_aligned(target_scores, 4),
                      "%s: misaligned rows (pred_dist needs 32 bytes, box rows 4 elements)", fn);
@@ -367,6 +377,8 @@ extern "C" int cerb_bbox_loss_fwd(const void* pred_dist, const void* pred_bboxes
     const unsigned ctas = fwd_ctas(P.n_rows);
     if (dtype == CERB_F16)
         bbox_loss_fwd_kernel<__half><<<ctas, BL_THREADS, 0, (cudaStream_t)stream>>>(P, loss_iou, loss_dfl, per_anchor, partials, ticket);
+    else if (dtype == CERB_BF16)
+        bbox_loss_fwd_kernel<__nv_bfloat16><<<ctas, BL_THREADS, 0, (cudaStream_t)stream>>>(P, loss_iou, loss_dfl, per_anchor, partials, ticket);
     else
         bbox_loss_fwd_kernel<float><<<ctas, BL_THREADS, 0, (cudaStream_t)stream>>>(P, loss_iou, loss_dfl, per_anchor, partials, ticket);
     return cerb_launch_status("cerb_bbox_loss_fwd", cudaGetLastError());
@@ -382,11 +394,14 @@ extern "C" int cerb_bbox_loss_bwd(const void* pred_dist, const void* pred_bboxes
     if (rc) return rc;
     if (P.n_rows == 0) return 0;
     CERB_REQUIRE(grad_iou && grad_dfl && grad_pred_dist && grad_pred_bboxes, "cerb_bbox_loss_bwd: null argument");
-    CERB_REQUIRE(cerb_aligned(grad_pred_dist, 32) && cerb_aligned(grad_pred_bboxes, dtype == CERB_F16 ? 8 : 16),
+    CERB_REQUIRE(cerb_aligned(grad_pred_dist, 32) && cerb_aligned(grad_pred_bboxes, dtype == CERB_F32 ? 16 : 8),
                  "cerb_bbox_loss_bwd: misaligned rows (grad_pred_dist needs 32 bytes, box rows 4 elements)");
     const unsigned blocks = (unsigned)((P.n_rows * 4 + BL_THREADS - 1) / BL_THREADS);
     if (dtype == CERB_F16)
         bbox_loss_bwd_kernel<__half><<<blocks, BL_THREADS, 0, (cudaStream_t)stream>>>(P, grad_iou, grad_dfl, (__half*)grad_pred_dist, (__half*)grad_pred_bboxes);
+    else if (dtype == CERB_BF16)
+        bbox_loss_bwd_kernel<__nv_bfloat16><<<blocks, BL_THREADS, 0, (cudaStream_t)stream>>>(P, grad_iou, grad_dfl, (__nv_bfloat16*)grad_pred_dist,
+                                                                                        (__nv_bfloat16*)grad_pred_bboxes);
     else
         bbox_loss_bwd_kernel<float><<<blocks, BL_THREADS, 0, (cudaStream_t)stream>>>(P, grad_iou, grad_dfl, (float*)grad_pred_dist, (float*)grad_pred_bboxes);
     return cerb_launch_status("cerb_bbox_loss_bwd", cudaGetLastError());

@@ -13,6 +13,8 @@
 //   tal_scores_kernel  the normalised one-hot scores [B, A, C], the one big output, written by the whole GPU.
 // Arithmetic: fp32, one rounding per reference op (no FMA contraction), libdevice atanf / powf / sqrtf like the ATen
 // kernels the reference runs, so indices and values match the reference on the same GPU bit for bit.
+// bf16 scores (the trainer under bf16 autocast) take tal_topk_bf16_kernel and tal_assign_bf16_kernel, built from the same
+// source as the fp16 / fp32 kernels (tal_stages.cuh) with a bf16 load and no rounding of the power (see align_metric).
 #include "../../include/cerb_post.h"
 #include "cerb_common.cuh"
 
@@ -22,7 +24,7 @@
 #define TAL_MAX_GT 1024
 
 struct TalParams {
-    const void* scores;      // [B, A, C] fp32 | fp16 (sigmoid scores)
+    const void* scores;      // [B, A, C] fp32 | fp16 | bf16 (sigmoid scores)
     const float* pd;         // [B, A, 4] xyxy, pixels
     const float* anc;        // [A, 2] anchor centres, pixels
     const float* gt_labels;  // [B, G]
@@ -80,161 +82,31 @@ __device__ __forceinline__ bool inside_gt(const float4 g, float ax, float ay, fl
     const float m = fminf(fminf(__fsub_rn(ax, g.x), __fsub_rn(ay, g.y)), fminf(__fsub_rn(g.z, ax), __fsub_rn(g.w, ay)));
     return m > eps;
 }
-__device__ __forceinline__ float load_score(const TalParams& P, int b, int a, int c) {
+// BF16 = false: fp16 or fp32 scores as P.score_half says; true: bf16 scores (the *_bf16 kernels)
+template <bool BF16> __device__ __forceinline__ float load_score(const TalParams& P, int b, int a, int c) {
     const size_t i = ((size_t)b * P.A + a) * P.C + c;
+    if constexpr (BF16) return __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(P.scores)[i]);
     return P.score_half ? __half2float(reinterpret_cast<const __half*>(P.scores)[i]) : reinterpret_cast<const float*>(P.scores)[i];
 }
 // align_metric of (box, anchor) BEFORE the inside mask: score^alpha * overlap^beta, with the reference's type promotion
-// (half scores: the power is rounded to half, then multiplied in fp32)
-__device__ __forceinline__ float align_metric(const TalParams& P, float score, float ov) {
+// (half scores: the power is rounded to half, then multiplied in fp32).  bf16 scores come from bf16 autocast, whose fp32
+// op list has pow: the power runs in fp32 on the widened score and is not rounded, so bf16 is the fp32 path after the load.
+template <bool BF16> __device__ __forceinline__ float align_metric(const TalParams& P, float score, float ov) {
     float sp = pow_like_torch(score, P.alpha);
-    if (P.score_half) sp = __half2float(__float2half_rn(sp));
+    if (!BF16 && P.score_half) sp = __half2float(__float2half_rn(sp));
     return __fmul_rn(sp, pow_like_torch(ov, P.beta));
 }
 
-__global__ void __launch_bounds__(TAL_THREADS_A) tal_topk_kernel(const __grid_constant__ TalParams P) {
-    __shared__ unsigned long long skeys[(TAL_THREADS_A / 32) * TAL_MAX_TOPK];
-    const int b = blockIdx.x / P.G, g = blockIdx.x - b * P.G, tid = threadIdx.x;
-    int* out = P.topk_idx + ((size_t)b * P.G + g) * P.topk;
-    if (!(P.mask_gt[(size_t)b * P.G + g] > 0.f)) {  // padded box: the reference zeroes its topk (tal.py:146-150)
-        if (tid < P.topk) out[tid] = -1;
-        return;
-    }
-    const float4 gt = reinterpret_cast<const float4*>(P.gt_boxes)[(size_t)b * P.G + g];
-    const int label = (int)P.gt_labels[(size_t)b * P.G + g];
-    // key = metric bits (metric >= 0: bit order = value order) in the high word, ~anchor in the low word:
-    // descending key = metric descending, then anchor ascending
-    unsigned long long best[TAL_MAX_TOPK];
-#pragma unroll
-    for (int i = 0; i < TAL_MAX_TOPK; ++i) best[i] = 0ull;  // (no real key is 0: ~anchor != 0)
-    const int K = P.topk;
-    for (int a = tid; a < P.A; a += TAL_THREADS_A) {
-        const float2 pt = reinterpret_cast<const float2*>(P.anc)[a];
-        float metric = 0.f;
-        if (inside_gt(gt, pt.x, pt.y, P.eps)) {
-            const float4 pb = reinterpret_cast<const float4*>(P.pd)[(size_t)b * P.A + a];
-            metric = align_metric(P, load_score(P, b, a, label), ciou_clamped(gt, pb));
-            if (!(metric >= 0.f)) metric = 0.f;  // NaN guard (scores are sigmoids, overlaps >= 0)
-        }
-        unsigned long long key = ((unsigned long long)__float_as_uint(metric) << 32) | (unsigned)(~a);
-        if (key > best[K - 1]) {  // insertion into the descending list (fully unrolled: registers)
-#pragma unroll
-            for (int i = 0; i < TAL_MAX_TOPK; ++i) {
-                if (i < K && key > best[i]) { const unsigned long long t = best[i]; best[i] = key; key = t; }
-            }
-        }
-    }
-    // merge without block-wide rounds: every warp pops the K largest heads of its 32 sorted lists with shuffles (keys are
-    // unique, so exactly one lane owns each maximum and shifts its list), then warp 0 does the same over the 8 * K survivors
-    const int lane = tid & 31, warp = tid >> 5;
-    unsigned long long mine = 0ull;  // lane r ends up with the warp's r-th largest key
-    for (int r = 0; r < K; ++r) {
-        unsigned long long m = best[0];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const unsigned long long t = __shfl_xor_sync(0xffffffffu, m, o);
-            m = t > m ? t : m;
-        }
-        if (best[0] == m && m != 0ull) {
-#pragma unroll
-            for (int i = 0; i + 1 < TAL_MAX_TOPK; ++i) best[i] = best[i + 1];
-            best[TAL_MAX_TOPK - 1] = 0ull;
-        }
-        if (lane == r) mine = m;
-    }
-    if (lane < K) skeys[warp * TAL_MAX_TOPK + lane] = mine;
-    __syncthreads();
-    if (warp == 0) {
-        constexpr int NW = TAL_THREADS_A / 32;
-        unsigned long long k[(NW * TAL_MAX_TOPK + 31) / 32];
-#pragma unroll
-        for (int j = 0; j < (NW * TAL_MAX_TOPK + 31) / 32; ++j) {
-            const int idx = lane + 32 * j, w = idx / TAL_MAX_TOPK, i = idx - w * TAL_MAX_TOPK;
-            k[j] = (w < NW && i < K) ? skeys[idx] : 0ull;
-        }
-        for (int r = 0; r < K; ++r) {
-            unsigned long long m = 0ull;
-#pragma unroll
-            for (int j = 0; j < (NW * TAL_MAX_TOPK + 31) / 32; ++j) m = k[j] > m ? k[j] : m;
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                const unsigned long long t = __shfl_xor_sync(0xffffffffu, m, o);
-                m = t > m ? t : m;
-            }
-#pragma unroll
-            for (int j = 0; j < (NW * TAL_MAX_TOPK + 31) / 32; ++j)
-                if (k[j] == m) k[j] = 0ull;
-            if (lane == 0) out[r] = m != 0ull ? (int)(~(unsigned)(m & 0xffffffffull)) : -1;
-        }
-    }
-}
-
-__global__ void __launch_bounds__(TAL_THREADS_B) tal_assign_kernel(const __grid_constant__ TalParams P) {
-    __shared__ float pos_align[TAL_MAX_GT], pos_ov[TAL_MAX_GT];
-    const int b = blockIdx.x, tid = threadIdx.x;
-    int* cnt = P.cnt + (size_t)b * P.A;
-    int* gsel = P.gsel + (size_t)b * P.A;
-    float* aval = P.aval + (size_t)b * P.A;
-    const float4* gts = reinterpret_cast<const float4*>(P.gt_boxes) + (size_t)b * P.G;
-    const float4* pds = reinterpret_cast<const float4*>(P.pd) + (size_t)b * P.A;
-    for (int a = tid; a < P.A; a += TAL_THREADS_B) { cnt[a] = 0; gsel[a] = 0; }
-    for (int g = tid; g < P.G; g += TAL_THREADS_B) { pos_align[g] = 0.f; pos_ov[g] = 0.f; }
-    __syncthreads();
-    // mask_pos = is_in_topk * mask_in_gts * mask_gt (tal.py:118): the (box, anchor) pairs of the topk lists that lie inside
-    for (int i = tid; i < P.G * P.topk; i += TAL_THREADS_B) {
-        const int g = i / P.topk;
-        const int a = P.topk_idx[((size_t)b * P.G + g) * P.topk + (i - g * P.topk)];
-        if (a < 0) continue;
-        const float2 pt = reinterpret_cast<const float2*>(P.anc)[a];
-        if (!inside_gt(gts[g], pt.x, pt.y, P.eps)) continue;
-        atomicAdd(&cnt[a], 1);
-        gsel[a] = g;  // unique writer when exactly one box claims the anchor; recomputed below otherwise
-    }
-    __syncthreads();
-    // select_highest_overlaps (tal.py:31-53): an anchor claimed by several boxes goes to argmax over ALL boxes of the
-    // overlap (first maximum), padded boxes included
-    for (int a = tid; a < P.A; a += TAL_THREADS_B) {
-        if (cnt[a] > 1) {
-            const float4 pb = pds[a];
-            float bestv = -1.f;
-            int bestg = 0;
-            for (int g = 0; g < P.G; ++g) {
-                const float ov = ciou_clamped(gts[g], pb);
-                if (ov > bestv) { bestv = ov; bestg = g; }
-            }
-            gsel[a] = bestg;
-        }
-    }
-    __syncthreads();
-    // per-box maxima of metric and overlap over the final positives (tal.py:103-106); values are >= 0, so the integer
-    // order of their bit patterns is their order
-    for (int a = tid; a < P.A; a += TAL_THREADS_B) {
-        if (cnt[a] > 0) {
-            const int g = gsel[a];
-            const float ov = ciou_clamped(gts[g], pds[a]);
-            float al = align_metric(P, load_score(P, b, a, (int)P.gt_labels[(size_t)b * P.G + g]), ov);
-            if (!(al >= 0.f)) al = 0.f;
-            aval[a] = al;
-            atomicMax(reinterpret_cast<int*>(&pos_align[g]), __float_as_int(al));
-            atomicMax(reinterpret_cast<int*>(&pos_ov[g]), __float_as_int(ov));
-        }
-    }
-    __syncthreads();
-    // get_targets (tal.py:153-178) + normalisation (:107-108); background anchors point at box 0 like the reference's argmax
-    for (int a = tid; a < P.A; a += TAL_THREADS_B) {
-        const bool fg = cnt[a] > 0;
-        const int g = fg ? gsel[a] : 0;
-        const size_t o = (size_t)b * P.A + a;
-        P.target_labels[o] = (long long)P.gt_labels[(size_t)b * P.G + g];
-        reinterpret_cast<float4*>(P.target_bboxes)[o] = gts[g];
-        P.fg_mask[o] = fg ? 1 : 0;
-        P.target_gt_idx[o] = g;
-    }
-    for (int g = tid; g < P.G; g += TAL_THREADS_B) {
-        P.pos[((size_t)b * P.G + g) * 2] = pos_align[g];
-        P.pos[((size_t)b * P.G + g) * 2 + 1] = pos_ov[g];
-    }
-}
+#define TAL_BF16 false
+#define TAL_KERNEL(stage) stage##_kernel
+#include "tal_stages.cuh"
+#undef TAL_BF16
+#undef TAL_KERNEL
+#define TAL_BF16 true
+#define TAL_KERNEL(stage) stage##_bf16_kernel
+#include "tal_stages.cuh"
+#undef TAL_BF16
+#undef TAL_KERNEL
 
 // target_scores [B, A, C] = one_hot(label) * fg * norm (tal.py:174-177, :107-108): the one big output (43 MB at B=64,
 // A=8400, C=20), written by the whole GPU with consecutive threads on consecutive elements
@@ -273,7 +145,8 @@ extern "C" int cerb_tal_assign(const void* pd_scores, const float* pd_bboxes, co
     CERB_REQUIRE(B >= 1 && A >= 1 && C >= 1, "cerb_tal_assign: empty problem (B=%d A=%d C=%d)", B, A, C);
     CERB_REQUIRE(G >= 1 && G <= TAL_MAX_GT, "cerb_tal_assign: G=%d outside [1, %d] (no boxes at all is the caller's early return, tal.py:89-93)", G, TAL_MAX_GT);
     CERB_REQUIRE(topk >= 1 && topk <= TAL_MAX_TOPK && topk <= A, "cerb_tal_assign: topk=%d outside [1, min(%d, A)]", topk, TAL_MAX_TOPK);
-    CERB_REQUIRE(score_dtype == CERB_F16 || score_dtype == CERB_F32, "cerb_tal_assign: unsupported score dtype %d", score_dtype);
+    CERB_REQUIRE(score_dtype == CERB_F16 || score_dtype == CERB_BF16 || score_dtype == CERB_F32,
+                 "cerb_tal_assign: unsupported score dtype %d", score_dtype);
     CERB_REQUIRE(cerb_aligned(pd_bboxes, 16) && cerb_aligned(gt_bboxes, 16) && cerb_aligned(target_bboxes, 16) && cerb_aligned(anc_points, 8),
                  "cerb_tal_assign: box tensors must be 16-byte aligned, anchor points 8-byte aligned");
     const size_t need = cerb_tal_workspace_bytes_impl(B, A, G, topk);
@@ -290,8 +163,13 @@ extern "C" int cerb_tal_assign(const void* pd_scores, const float* pd_bboxes, co
     P.pos = (float*)ws;
     P.target_labels = target_labels; P.target_bboxes = target_bboxes; P.target_scores = target_scores; P.fg_mask = fg_mask;
     P.target_gt_idx = target_gt_idx;
-    tal_topk_kernel<<<B * G, TAL_THREADS_A, 0, (cudaStream_t)stream>>>(P);
-    tal_assign_kernel<<<B, TAL_THREADS_B, 0, (cudaStream_t)stream>>>(P);
+    if (score_dtype == CERB_BF16) {
+        tal_topk_bf16_kernel<<<B * G, TAL_THREADS_A, 0, (cudaStream_t)stream>>>(P);
+        tal_assign_bf16_kernel<<<B, TAL_THREADS_B, 0, (cudaStream_t)stream>>>(P);
+    } else {
+        tal_topk_kernel<<<B * G, TAL_THREADS_A, 0, (cudaStream_t)stream>>>(P);
+        tal_assign_kernel<<<B, TAL_THREADS_B, 0, (cudaStream_t)stream>>>(P);
+    }
     const size_t n_out = (size_t)B * A * C;
     const int blocks = (int)((n_out + 255) / 256 < 148 * 16 ? (n_out + 255) / 256 : 148 * 16);
     tal_scores_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(P);

@@ -19,7 +19,8 @@ MAX_WH = 7680.0  # reference utils/general.py:415
 MAX_NMS = 30000  # reference utils/general.py:416
 
 _DTYPES = {torch.float16: _lib.CERB_F16, torch.float32: _lib.CERB_F32}
-# the kernels that read head-dtype tensors (decode, NMS, the training-time box decode) also take bfloat16
+# the kernels that read head-dtype tensors (decode, NMS, the training-time box decode, the assigner's scores and the
+# box-regression loss's predictions) also take bfloat16
 _HEAD_DTYPES = {**_DTYPES, torch.bfloat16: _lib.CERB_BF16}
 
 
@@ -751,10 +752,11 @@ def tal_assign(pd_scores: torch.Tensor, pd_bboxes: torch.Tensor, anc_points: tor
                gt_bboxes: torch.Tensor, mask_gt: torch.Tensor, topk: int = 10, num_classes: Optional[int] = None,
                alpha: float = 0.5, beta: float = 6.0, eps: float = 1e-9):
     """``TaskAlignedAssigner.forward`` (reference utils/tal.py:56-178) in three launches (``cerb_tal_assign``).
-    ``pd_scores [B, A, C]`` fp16 | fp32, ``pd_bboxes [B, A, 4]`` fp32 xyxy pixels, ``anc_points [A, 2]``, ``gt_labels [B, G, 1]``,
+    ``pd_scores [B, A, C]`` fp16 | bf16 | fp32, ``pd_bboxes [B, A, 4]`` fp32 xyxy pixels, ``anc_points [A, 2]``, ``gt_labels [B, G, 1]``,
     ``gt_bboxes [B, G, 4]``, ``mask_gt [B, G, 1]``.  Returns ``(target_labels [B, A] int64, target_bboxes [B, A, 4],
     target_scores [B, A, C] fp32, fg_mask [B, A] bool, target_gt_idx [B, A] int64)``.  ``G == 0`` is the caller's early
-    return in the reference (tal.py:89-93) and raises ``ValueError`` here."""
+    return in the reference (tal.py:89-93) and raises ``ValueError`` here.  bf16 scores are bf16 autocast's: its ``pow``
+    runs in fp32 on the widened scores, so they give exactly what the same scores in fp32 give."""
     lib = _lib.load()
     _require_cuda(pd_scores, "pd_scores")
     B, A, C = (int(v) for v in pd_scores.shape)
@@ -764,7 +766,7 @@ def tal_assign(pd_scores: torch.Tensor, pd_bboxes: torch.Tensor, anc_points: tor
     if G == 0:
         raise ValueError("tal_assign needs at least one (padded) ground-truth box per image; the reference returns early for none")
     dev = pd_scores.device
-    code = _dtype_code(pd_scores)
+    code = _dtype_code(pd_scores, head=True)
     f32 = lambda t, shape: t.to(device=dev, dtype=torch.float32).reshape(shape).contiguous()  # noqa: E731
     sc = pd_scores.contiguous()
     pb, an = f32(pd_bboxes, (B, A, 4)), f32(anc_points, (A, 2))
@@ -810,7 +812,7 @@ class _BboxLoss(torch.autograd.Function):
                 raise ValueError(f"{name} must be {list(shape)}, got {tuple(t.shape)}")
             if t.device != dev:
                 raise TypeError(f"{name} must be on {dev}, got {t.device}")
-        code = _dtype_code(pred_dist)
+        code = _dtype_code(pred_dist, head=True)
         if pred_bboxes.dtype != pred_dist.dtype or anchor_points.dtype != pred_dist.dtype:
             raise TypeError("pred_dist, pred_bboxes and anchor_points must share one dtype")
         if target_bboxes.dtype != torch.float32 or target_scores.dtype != torch.float32 or fg_mask.dtype != torch.bool:
@@ -867,8 +869,9 @@ def bbox_loss(pred_dist: torch.Tensor, pred_bboxes: torch.Tensor, anchor_points:
     ``pred_bboxes [B, A, 4]``.  No host synchronisation: the foreground mask is read by the kernels, and
     ``target_scores_sum`` (a 0-d CUDA tensor, or a number such as the call site's ``1``) is read on the device.
 
-    Two dtype combinations: everything float32; or the trainer's fp16-autocast case -- ``pred_dist``, ``pred_bboxes`` and
-    ``anchor_points`` float16, ``target_bboxes`` / ``target_scores`` float32 -- with the reference's half roundings.
+    Three dtype combinations: everything float32; or the trainer's fp16-autocast case -- ``pred_dist``, ``pred_bboxes`` and
+    ``anchor_points`` float16, ``target_bboxes`` / ``target_scores`` float32 -- with the reference's half roundings; or the
+    bf16-autocast case, the same with bfloat16 predictions and bf16 roundings.  The gradients have the predictions' dtype.
     ``per_anchor`` (float32 ``[B, A, 2]``, optional) receives the per-anchor terms ``(1 - CIoU) * weight`` and
     ``DFL * weight`` (zero at background anchors)."""
     return _BboxLoss.apply(pred_dist, pred_bboxes, anchor_points, target_bboxes, target_scores, target_scores_sum, fg_mask, per_anchor)

@@ -16,13 +16,17 @@ What gets rebound (and restored by ``uninstall()``):
   the expectation, one per corner), so fp16 ``pred_dist`` + fp16 anchors under autocast go to the kernels.  bf16
   autocast is the same with bf16 in place of fp16, so bf16 ``pred_dist`` + bf16 anchors go to the kernels' bf16 path,
   with or without autocast; any other dtype mix (fp32 under autocast, a ``pred_dist`` dtype other than the autocast
-  dtype, anchors of another dtype) keeps the reference's own code;
+  dtype, anchors of another dtype) keeps the reference's own code.  ``TaskAlignedAssigner.forward`` -> ``ops.tal_assign``
+  takes fp32 and fp16 scores, and bf16 scores under bf16 autocast only: autocast runs the assigner's ``pow`` in fp32 on
+  the widened scores, which is the kernels' bf16 rule, while bf16 scores outside autocast (a ``model.bfloat16()``
+  trainer) round the power to bf16 and keep the reference's code;
 * with ``loss=True`` ``cerberusdet.utils.loss.BboxLoss.forward`` -> ``ops.bbox_loss`` (the box-regression term the loss
   computes right after the assigner, reference utils/loss.py:12-44: CIoU + DFL in one forward and one backward kernel, no
   host synchronisation).  On the path: ``use_dfl`` with 16 bins, CUDA tensors, and either everything fp32 without
-  autocast or the trainer's fp16 autocast case (fp16 ``pred_dist`` / ``pred_bboxes`` / ``anchor_points``, fp32 targets);
-  anything else (CPU tensors, ``use_dfl=False``, another ``reg_max``, other dtype mixes, bf16 autocast) keeps the
-  reference's own code;
+  autocast, or the trainer's fp16 autocast case (fp16 ``pred_dist`` / ``pred_bboxes`` / ``anchor_points``, fp32 targets),
+  or its bf16 autocast case (the same with bf16 predictions); anything else (CPU tensors, ``use_dfl=False``, another
+  ``reg_max``, other dtype mixes, bf16 predictions outside autocast or under fp16 autocast, fp16 ones under bf16 autocast)
+  keeps the reference's own code;
 * with ``val=True`` the validation loop's per-image matching (val.py:32-54 ``process_batch``) -> ``ops.match_batch``;
 * with ``metrics=True`` ``ap_per_class`` (utils/metrics.py:56-120), which ``DetMetrics.process`` reads as a module global,
   -> ``val_stats.ap_per_class`` (``ops.ap_per_class`` for the per-class curves and APs, the host tail in numpy), in
@@ -35,9 +39,9 @@ What gets rebound (and restored by ``uninstall()``):
   ``detections=None``, CPU or non-fp32 tensors, more than 30000 detections or 1024 labels and classes outside
   ``[0, nc)`` keep the reference's own method.
 
-CUDA fp16/fp32 tensors (and bf16 ones for the decode, the NMS and ``Loss.bbox_decode``) go to the kernels; anything
-else (CPU tensors, training mode, masks/labels arguments) is handed to the reference's own, saved implementation --
-the patch never changes what a non-CUDA run computes.
+CUDA fp16/fp32 tensors (and bf16 ones for the decode, the NMS and ``Loss.bbox_decode``, and under bf16 autocast for the
+assigner and ``BboxLoss``) go to the kernels; anything else (CPU tensors, training mode, masks/labels arguments) is
+handed to the reference's own, saved implementation -- the patch never changes what a non-CUDA run computes.
 """
 from __future__ import annotations
 
@@ -153,7 +157,11 @@ def install(import_all: bool = False, train: bool = False, val: bool = False, lo
 
             @torch.no_grad()
             def forward(self, pd_scores, pd_bboxes, anc_points, gt_labels, gt_bboxes, mask_gt):
-                on_path = (pd_scores.is_cuda and pd_scores.dtype in (torch.float16, torch.float32) and pd_scores.dim() == 3
+                # bf16 scores only under bf16 autocast, where the reference's pow widens them to fp32 (the kernels' bf16
+                # rule); a bf16 model outside autocast rounds the power to bf16 and keeps the reference's code
+                bf16_ok = torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") == torch.bfloat16
+                on_path = (pd_scores.is_cuda and (pd_scores.dtype in (torch.float16, torch.float32)
+                                                  or (pd_scores.dtype == torch.bfloat16 and bf16_ok)) and pd_scores.dim() == 3
                            and pd_bboxes.dtype == torch.float32 and gt_bboxes.dtype == torch.float32 and gt_bboxes.dim() == 3
                            and 0 < gt_bboxes.size(1) <= 1024 and self.topk <= min(16, pd_scores.size(1))
                            and pd_scores.size(2) == self.num_classes)
@@ -200,8 +208,9 @@ def install(import_all: bool = False, train: bool = False, val: bool = False, lo
                            and target_bboxes.dtype == torch.float32 and target_scores.dtype == torch.float32
                            and pred_bboxes.dtype == pred_dist.dtype and anchor_points.dtype == pred_dist.dtype)
                 if on_path and torch.is_autocast_enabled("cuda"):
-                    # fp16 autocast: half predictions, fp32 targets -- the kernels' half mode
-                    on_path = pred_dist.dtype == torch.float16 and torch.get_autocast_dtype("cuda") == torch.float16
+                    # fp16 (bf16) autocast: fp16 (bf16) predictions, fp32 targets -- the kernels' half (bf16) mode
+                    on_path = (pred_dist.dtype in (torch.float16, torch.bfloat16)
+                               and torch.get_autocast_dtype("cuda") == pred_dist.dtype)
                 elif on_path:
                     on_path = pred_dist.dtype == torch.float32
                 if not on_path:  # CPU tensors, use_dfl=False, reg_max != 15, other dtype mixes: the reference's own code

@@ -20,8 +20,10 @@
  *  - dtype: CERB_F16 (IEEE half) or CERB_F32; tensors are contiguous.  CERB_BF16 (bfloat16) is
  *    accepted by the entry points that read head-dtype tensors: cerb_decode, cerb_decode_split,
  *    cerb_nms (and its _stats / _deliver forms), cerb_decode_nms, cerb_summary_row_len,
- *    cerb_bbox_decode_fwd and cerb_bbox_decode_bwd.  Every other entry point rejects it.
- *    bf16 tensors round at the same points as half ones, in bf16 (see each prototype).
+ *    cerb_bbox_decode_fwd and cerb_bbox_decode_bwd, and by the bf16-autocast training calls
+ *    cerb_tal_assign (score_dtype) and cerb_bbox_loss_fwd / _bwd.  Every other entry point rejects it.
+ *    bf16 tensors round at the same points as half ones, in bf16 (see each prototype); the
+ *    assigner's bf16 scores are the exception (see cerb_tal_assign).
  */
 #ifndef CERB_POST_H
 #define CERB_POST_H
@@ -309,7 +311,7 @@ int cerb_bbox_decode_bwd(const void* pred_dist, const void* grad_out, long n_row
  * select_candidates_in_gts :13-28, select_highest_overlaps :31-53 and bbox_iou(CIoU=True) of utils/metrics.py:373-408), as
  * called by the loss at cerberusdet/utils/loss.py:160-162, in three launches.
  *
- *   pd_scores     [B, A, C] sigmoid scores, fp16 | fp32 (score_dtype)      pd_bboxes   [B, A, 4] xyxy pixels, fp32
+ *   pd_scores     [B, A, C] sigmoid scores, fp16 | bf16 | fp32 (score_dtype)      pd_bboxes   [B, A, 4] xyxy pixels, fp32
  *   anc_points    [A, 2] anchor centres in pixels, fp32
  *   gt_labels     [B, G] class ids as floats, gt_bboxes [B, G, 4] xyxy pixels, mask_gt [B, G] 1 = real box, 0 = padding
  *   topk (<= 16), alpha, beta, eps: the assigner's attributes (10, 0.5, 6.0, 1e-9 in the reference, loss.py:100-105)
@@ -319,6 +321,8 @@ int cerb_bbox_decode_bwd(const void* pred_dist, const void* grad_out, long n_row
  * G >= 1 (the reference returns early for G == 0, tal.py:89-93: the caller keeps that branch), G <= 1024.
  * Equal metrics rank by anchor index ascending -- the reference's torch.topk (:140) leaves their order unspecified; it
  * only matters for boxes with fewer than topk positive-metric anchors AND anchors inside whose CIoU is <= 0.
+ * fp16 scores: score^alpha is rounded to half.  bf16 scores are bf16 autocast's, whose fp32 op list has pow: score^alpha
+ * is computed in fp32 on the widened score and not rounded, so bf16 scores give what the same values in fp32 give.
  */
 size_t cerb_tal_workspace_bytes(int B, int A, int G, int topk);
 int cerb_tal_assign(const void* pd_scores, const float* pd_bboxes, const float* anc_points, const float* gt_labels,
@@ -340,7 +344,8 @@ int cerb_tal_assign(const void* pd_scores, const float* pd_bboxes, const float* 
  *   target_scores_sum   device fp32 scalar, or NULL: target_scores_sum_host is used
  *   dtype          CERB_F32: every tensor above fp32.  CERB_F16: the trainer's fp16 autocast case -- half predictions and
  *                  anchors, fp32 targets; the reference's half roundings (w1, h1, w1*h1, w1/h1, atan(w1/h1), the
- *                  cross-entropy's log-probabilities) are kept
+ *                  cross-entropy's log-probabilities) are kept.  CERB_BF16: the bf16 autocast case, the same
+ *                  roundings in bf16
  *   loss_iou, loss_dfl   out: device fp32 scalars
  *   per_anchor     optional out [B, A, 2] fp32: (1 - CIoU) * weight and DFL * weight per anchor (0 at background), or NULL
  *   workspace      cerb_bbox_loss_workspace_bytes(B, A) bytes, 16-byte aligned, ZEROED before its first use (the

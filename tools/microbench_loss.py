@@ -106,22 +106,28 @@ def bwd_kernel(c, code):
     return run
 
 
+# mode: (prediction dtype, dtype code); "amp" and "bf16" run under autocast of that dtype
+MODES = {"fp32": (torch.float32, _lib.CERB_F32), "amp": (torch.float16, _lib.CERB_F16), "bf16": (torch.bfloat16, _lib.CERB_BF16)}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "bbox_loss.md"))
     ap.add_argument("--batch", type=int, default=64)
+    ap.add_argument("--modes", default="fp32,amp", help="comma-separated: fp32, amp (fp16 autocast), bf16 (bf16 autocast)")
     args = ap.parse_args()
     name, power = card()
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
     rows = []
     for C in (20, 80):
-        for mode, dtype in (("fp32", torch.float32), ("amp", torch.float16)):
+        for mode in args.modes.split(","):
+            dtype, code = MODES[mode]
             c = lp.loss_case(5, args.batch, LEVELS, STRIDES, C, 20, dtype=dtype, ops=ops)
-            amp = torch.autocast("cuda", dtype=torch.float16, enabled=mode == "amp")
+            amp = torch.autocast("cuda", dtype=dtype, enabled=mode != "fp32")
             with amp:
                 fused = time_events(lambda: fused_step(c), flush)
                 ref = time_host(lambda: reference_step(c), flush)
-            bwd = time_events(bwd_kernel(c, _lib.CERB_F16 if mode == "amp" else _lib.CERB_F32), flush)
+            bwd = time_events(bwd_kernel(c, code), flush)
             B, A = c["fg_mask"].shape
             npos = int(c["fg_mask"].sum())
             s = c["pred_dist"].element_size()
@@ -136,7 +142,7 @@ def main():
         "",
         f"Measured with `tools/microbench_loss.py` on **{name}** (power limit, max SM clock: {power}).  "
         f"B={args.batch}, 640x640 (8400 anchors), 20 ground truths per image through `ops.tal_assign`; \"fp32\" = every tensor "
-        "fp32, \"amp\" = the trainer's fp16 autocast case.",
+        "fp32, \"amp\" = the trainer's fp16 autocast case, \"bf16\" = its bf16 autocast case.",
         "",
         "- fused: `ops.bbox_loss` forward + backward (two kernels + the workspace memset), CUDA events, L2 overwritten between "
         "iterations, median of 50.",
