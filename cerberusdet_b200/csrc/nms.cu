@@ -85,10 +85,25 @@ extern "C" int cerb_debug_read_block_times(unsigned long long* out, int n) {
 // Optional phase timers (-DNMS_PROFILE, tools/ only): thread 0 of EVERY block accumulates clock64() deltas per phase in
 // registers/local memory (no global traffic at the stamps, so short phases are not inflated) and adds them to the global
 // totals once, at the end of the kernel.  g_nms_prof[0..9] phases, [10] blocks, [11] consumed, [12..14] collect sub-steps,
-// [15] fixpoint rounds.
+// [15] fixpoint rounds, [16] chunks collected, [17] tiles, [18] score vectors listed by summary pass 1, [19] chunks that
+// fell back to the plain scan, [20] exact-histogram rebuilds, [21] / [22] fixpoint settle-loop iterations / cycles summed
+// over the warps.  The collect sub-steps, [18], [21] and [22] are global atomics at the stamp (PROFX / PROF_GADD).
 #ifdef NMS_PROFILE
-__device__ unsigned long long g_nms_prof[16];
-#define PROF_DECL long long prof_t = clock64(), prof_x = 0; unsigned long long prof_acc[16] = {0};
+#define NMS_PROF_SLOTS 24
+__device__ unsigned long long g_nms_prof[NMS_PROF_SLOTS];
+__shared__ long long s_profx_t;
+#define PROF_DECL long long prof_t = clock64(); unsigned long long prof_acc[NMS_PROF_SLOTS] = {0};
+#define PROF_COUNT(slot, n) do { if (threadIdx.x == 0) prof_acc[slot] += (n); } while (0)
+#define PROF_GADD(slot, n) do { if (threadIdx.x == 0) atomicAdd(&g_nms_prof[slot], (unsigned long long)(n)); } while (0)
+#define PROFX_START do { if (threadIdx.x == 0) s_profx_t = clock64(); } while (0)
+#define PROFX(slot)                                                              \
+    do {                                                                         \
+        if (threadIdx.x == 0) {                                                  \
+            const long long now_ = clock64();                                    \
+            atomicAdd(&g_nms_prof[slot], (unsigned long long)(now_ - s_profx_t)); \
+            s_profx_t = now_;                                                    \
+        }                                                                        \
+    } while (0)
 #define PROF(slot)                                                        \
     do {                                                                  \
         if (threadIdx.x == 0) {                                           \
@@ -101,19 +116,22 @@ __device__ unsigned long long g_nms_prof[16];
     do {                                                                  \
         if (threadIdx.x == 0) {                                           \
             prof_acc[10] = 1; prof_acc[11] = (consumed_);                 \
-            for (int i_ = 0; i_ < 16; ++i_) if (prof_acc[i_]) atomicAdd(&g_nms_prof[i_], prof_acc[i_]); \
+            for (int i_ = 0; i_ < NMS_PROF_SLOTS; ++i_) if (prof_acc[i_]) atomicAdd(&g_nms_prof[i_], prof_acc[i_]); \
         }                                                                 \
     } while (0)
-extern "C" int cerb_debug_read_profile(unsigned long long* out16, int reset) {
+// out receives NMS_PROF_SLOTS (24) counters
+extern "C" int cerb_debug_read_profile(unsigned long long* out, int reset) {
     cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out16, g_nms_prof, sizeof(unsigned long long) * 16);
-    if (reset) { unsigned long long z[16] = {0}; cudaMemcpyToSymbol(g_nms_prof, z, sizeof(z)); }
+    cudaMemcpyFromSymbol(out, g_nms_prof, sizeof(unsigned long long) * NMS_PROF_SLOTS);
+    if (reset) { unsigned long long z[NMS_PROF_SLOTS] = {0}; cudaMemcpyToSymbol(g_nms_prof, z, sizeof(z)); }
     return 0;
 }
-#define PROFX(slot) do {} while (0)
 #else
 #define PROF_DECL
 #define PROF(slot) do {} while (0)
+#define PROF_COUNT(slot, n) do {} while (0)
+#define PROF_GADD(slot, n) do {} while (0)
+#define PROFX_START do {} while (0)
 #define PROFX(slot) do {} while (0)
 #define PROF_FLUSH(c) do {} while (0)
 #endif
@@ -431,6 +449,7 @@ __device__ __forceinline__ bool for_each_candidate_summary(const T* __restrict__
         __syncthreads();
         if (threadIdx.x == 0) *nhits = 0;
         __syncthreads();
+        PROFX_START;
     }
     // ---- pass 1: the summary (block-uniform trip count: warp_reserve needs whole warps)
     for (unsigned qb = 0; qb < nsv; qb += NMS_THREADS * SCAN_UNROLL) {
@@ -438,12 +457,11 @@ __device__ __forceinline__ bool for_each_candidate_summary(const T* __restrict__
         ScoreVec<T> m[SCAN_UNROLL];
 #pragma unroll
         for (int u = 0; u < SCAN_UNROLL; ++u) {
-            const unsigned q = q0 + u * NMS_THREADS;
-            if (q < nsv) {
-                const unsigned c = MULTI ? q / SV : 0u;
-                const unsigned j0 = (MULTI ? q - c * SV : q) * V;
-                m[u].raw = __ldg(reinterpret_cast<const uint4*>(smax + (size_t)c * SNV + j0));
-            }
+            // rows are SV vectors apart (SNV == SV * V), so summary vector q sits at smax + q * V.  The index is clamped
+            // rather than tested: behind a branch per load the compiler parks each loaded vector in local memory, which
+            // serialises the loads and, with 2 CTAs of 109 KB per SM, sends every reload to L2.
+            const unsigned q = min(q0 + u * NMS_THREADS, nsv - 1u);
+            m[u].raw = __ldg(reinterpret_cast<const uint4*>(smax) + q);
         }
         unsigned h[SCAN_UNROLL], ebase[SCAN_UNROLL], cnt = 0;
 #pragma unroll
@@ -475,12 +493,11 @@ __device__ __forceinline__ bool for_each_candidate_summary(const T* __restrict__
             unsigned pos = warp_reserve(nhits, cnt);
 #pragma unroll
             for (int u = 0; u < SCAN_UNROLL; ++u)
-#pragma unroll
-                for (int k = 0; k < V; ++k)
-                    if ((h[u] >> k) & 1u) {
-                        if (pos < NMS_BINS) hits[pos] = ebase[u] + k;
-                        ++pos;
-                    }
+                // set bits only: most summary vectors list nothing, and with 2 CTAs per SM this phase is bound by issue
+                for (unsigned hm = h[u]; hm; hm &= hm - 1u) {
+                    if (pos < NMS_BINS) hits[pos] = ebase[u] + (unsigned)(__ffs(hm) - 1);
+                    ++pos;
+                }
         } else {
 #pragma unroll
             for (int u = 0; u < SCAN_UNROLL; ++u)
@@ -498,6 +515,7 @@ __device__ __forceinline__ bool for_each_candidate_summary(const T* __restrict__
     const unsigned nh = *nhits;
     __syncthreads();
     PROFX(13);  // collect: wait for the block
+    PROF_GADD(18, nh);
     if (nh > NMS_BINS) return false;  // dense: not worth (and not possible) to list
     // ---- pass 2: the listed score vectors
     if (MULTI) {
@@ -507,13 +525,9 @@ __device__ __forceinline__ bool for_each_candidate_summary(const T* __restrict__
             unsigned e_[SCAN_UNROLL];
 #pragma unroll
             for (int u = 0; u < SCAN_UNROLL; ++u) {
-                const unsigned i = i0 + u * NMS_THREADS;
-                e_[u] = 0;
-                if (i < nh) {
-                    e_[u] = hits[i];
-                    const unsigned c = e_[u] / NV;
-                    v[u].raw = __ldg(reinterpret_cast<const uint4*>(sc + (size_t)c * A + (size_t)(e_[u] - c * NV) * V));
-                }
+                e_[u] = hits[min(i0 + u * NMS_THREADS, nh - 1u)];  // clamped: unconditional loads, as in pass 1
+                const unsigned c = e_[u] / NV;
+                v[u].raw = __ldg(reinterpret_cast<const uint4*>(sc + (size_t)c * A + (size_t)(e_[u] - c * NV) * V));
             }
             unsigned hv[SCAN_UNROLL], cnt = 0;
 #pragma unroll
@@ -887,6 +901,7 @@ __global__ void __launch_bounds__(NMS_THREADS, MINB) nms_kernel(const __grid_con
             int cls = 0, code = -1;
             bool dead = true;
             if (tid == 0) S.tile_wild = 0;
+            PROF_COUNT(17, 1);
             __syncthreads();
             if (tid < nt) {
                 const u64 key = S.keys[t0 + tid];
@@ -1007,13 +1022,26 @@ __global__ void __launch_bounds__(NMS_THREADS, MINB) nms_kernel(const __grid_con
                         if (w != myw) others |= mw[w] & (((u64)K[2 * w + 1] << 32) | (u64)K[2 * w]);
                     const unsigned sibling = K[wid ^ 1];
                     unsigned mine = K[wid];
+#ifdef NMS_PROFILE
+                    const long long settle_t0 = clock64();
+                    unsigned settle_it = 0;
+#endif
                     for (;;) {  // warp-local settle
                         const u64 own = upper ? (((u64)mine << 32) | (u64)sibling) : (((u64)sibling << 32) | (u64)mine);
                         const bool kj = !dead && (others | (mown & own)) == 0ull;
                         const unsigned nw = __ballot_sync(0xffffffffu, kj);
+#ifdef NMS_PROFILE
+                        ++settle_it;
+#endif
                         if (nw == mine) break;
                         mine = nw;
                     }
+#ifdef NMS_PROFILE
+                    if (lane == 0) {  // [21] settle iterations, [22] settle cycles: summed over the warps of the block
+                        atomicAdd(&g_nms_prof[21], (unsigned long long)settle_it);
+                        atomicAdd(&g_nms_prof[22], (unsigned long long)(clock64() - settle_t0));
+                    }
+#endif
                     int changed = 0;
                     if (lane == 0) { S.keep32[cur ^ 1][wid] = mine; changed = (mine != K[wid]); }
                     cur ^= 1;
@@ -1074,7 +1102,9 @@ __global__ void __launch_bounds__(NMS_THREADS, MINB) nms_kernel(const __grid_con
         if (smax && !summary_dense)
             done = for_each_candidate_summary<T, MULTI, true>(img, smax, nc, A, thr, P, put, sb_lo, sb_hi, S.g1, &S.nhits,
                                                               lo, hi, S.keys, &S.counter);
+        PROF_COUNT(16, 1);
         if (!done) {
+            PROF_COUNT(19, 1);
             summary_dense = true;  // candidates are dense in this segment: the plain scan is the better tool
             for_each_candidate<T, MULTI>(img, nc, A, thr, P, put, sb_lo, sb_hi);
         }
@@ -1165,6 +1195,7 @@ __global__ void __launch_bounds__(NMS_THREADS, MINB) nms_kernel(const __grid_con
         const unsigned n = collect((u64)lo0 << 52, (u64)hi0 << 52);
         if (n > cap) {
             // estimate was off (or ties piled up): count exactly what is left and retry
+            PROF_COUNT(20, 1);
             build_hist(1u, (unsigned)hi0);
             hstride = 1;
             exact = true;

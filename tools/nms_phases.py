@@ -9,7 +9,7 @@ from cerberusdet_b200.synth import STRIDES, synth_heads
 from kbench import CFG
 names = ["setup", "hist", "collect", "sort", "A gather", "B prev+kept", "C pairwise", "D fixpoint", "E append", "rest"]
 lib = _lib.load()
-buf = (ctypes.c_ulonglong * 16)()
+buf = (ctypes.c_ulonglong * 24)()
 for name in sys.argv[1:] or ["cfg2", "cfg3"]:
     c = CFG[name]
     heads = synth_heads(range(c["B"]), c["ncs"], c["imgsz"], c["dtype"], c.get("regime", "iid"), cfg=3)
@@ -22,3 +22,7 @@ for name in sys.argv[1:] or ["cfg2", "cfg3"]:
     for i, n in enumerate(names):
         print(f"   {n:14s} {buf[i]/runs:9.0f} cyc  {100*buf[i]/tot:5.1f}%")
     print("   fixpoint rounds per block:", buf[15] / runs)
+    print(f"   collect sub-steps (cycles per block): pass 1 {buf[12]/runs:.0f}, wait {buf[13]/runs:.0f}, pass 2 {buf[14]/runs:.0f}")
+    print(f"   chunks per block {buf[16]/runs:.3f}, tiles per block {buf[17]/runs:.3f}, vectors listed per block {buf[18]/runs:.0f}, "
+          f"plain-scan chunks {buf[19]}, exact-histogram rebuilds {buf[20]}")
+    print(f"   fixpoint: settle iterations per warp-round {buf[21]/max(buf[15]*16,1):.2f}, settle cycles per warp-round {buf[22]/max(buf[15]*16,1):.0f}")
